@@ -66,7 +66,16 @@ def parse_args():
     ap.add_argument("--skip-e2e", action="store_true")
     ap.add_argument("--skip-parity", action="store_true")
     ap.add_argument("--cpu-slices", type=int, default=0, help="slices per axis in the CPU sample (0: one per core)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the arrays the last step returned as DIR/<name>.npy (float32): "
+                         "whole volumes up to 4 Mi voxels, else a fixed seeded sample of 4 Mi voxels (dump_sample_index)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if a.dump_outputs is not None and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     cfg = dict(CONFIGS[a.config])
     a.customised = any(v is not None for v in (a.shape, a.sigma, a.levels, a.winsize, a.dtype)) or \
         (a.no_of and not cfg["no_of"]) or a.recompute_flow
@@ -318,6 +327,45 @@ def slab_digests(t):
     return out
 
 
+DUMP_VOXELS = 1 << 22      # per array: 16 MiB of float32, so the two results of a step stay well under 64 MB
+
+
+def dump_sample_index(nvox):
+    """Flat (C-order) indices of the voxels --dump-outputs writes: all of them up to DUMP_VOXELS, else one voxel
+    drawn with a fixed seed from each of DUMP_VOXELS equal runs of the volume, so the sample covers all of it."""
+    if nvox <= DUMP_VOXELS:
+        return np.arange(nvox, dtype=np.int64)
+    run = nvox // DUMP_VOXELS
+    return np.arange(DUMP_VOXELS, dtype=np.int64) * run + np.random.default_rng(0).integers(0, run, DUMP_VOXELS)
+
+
+def dump_outputs(path, arrays, shape, z_range, rank, world):
+    """arrays: name -> this rank's Z-slab [z1 - z0][Y][X] of a result (device tensor). Every rank takes its part of
+    the voxels at dump_sample_index(); rank 0 writes path/<name>.npy in index order, shaped [Z][Y][X] when the
+    whole volume fits the budget."""
+    import torch
+    import torch.distributed as dist
+    Z, Y, X = shape
+    idx = dump_sample_index(Z * Y * X)
+    lo, hi = z_range[0] * Y * X, z_range[1] * Y * X
+    mine = np.nonzero((idx >= lo) & (idx < hi))[0]
+    if rank == 0:
+        os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        local = torch.from_numpy(idx[mine] - lo).to(t.device)
+        part = (mine, torch.take(t, local).cpu().numpy())
+        parts = [None] * world
+        if world > 1:
+            dist.gather_object(part, parts if rank == 0 else None, dst=0)
+        else:
+            parts[0] = part
+        if rank == 0:
+            out = np.empty(idx.size, np.float32)
+            for pos, vals in parts:
+                out[pos] = vals
+            np.save(os.path.join(path, f"{name}.npy"), out.reshape(shape) if idx.size == Z * Y * X else out)
+
+
 # ----------------------------------------------------------------------------------------------------------------
 def main():
     args = parse_args()
@@ -496,6 +544,10 @@ def main():
     identity = {"result_sha256": result_sha, "what": "sha256 over the sha256 of every Z slice of the Z+Y+X result",
                 "expected_n1_sha256": expected,
                 "equals_n1": (result_sha == expected) if expected else None}
+    if args.dump_outputs:
+        # what a caller of the timed path receives: (zy, zyx) at N = 1; at N > 1 the result slabs (no zy is asked for)
+        dump_outputs(args.dump_outputs, {name: t for name, t in zip(("zy", "zyx"), res) if t is not None}, shape,
+                     (0, Z) if world == 1 else dd.z_range, rank, world)
 
     del res, zyx
     eng.release_workspace()

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -75,3 +76,58 @@ def test_reference_arm_prints_the_contract_line():
     cb = line["cpu_baseline"]
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == line["value"] and cb["sample"]
     assert line["config"]["shape"] == [18, 48, 64] and line["vs_baseline"] is None
+
+
+def test_steps_and_dump_outputs_arguments():
+    assert _args(["--steps", "7"]).steps == 7 and _args([]).dump_outputs is None
+    assert _args(["--dump-outputs", "out"]).dump_outputs == "out"
+    for bad in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "out"]):
+        with pytest.raises(SystemExit):
+            _args(bad)
+
+
+def test_dump_sample_is_fixed_and_spans_the_volume():
+    import bench
+    assert np.array_equal(bench.dump_sample_index(1000), np.arange(1000))
+    nvox = 512 * 1024 * 1024
+    idx = bench.dump_sample_index(nvox)
+    assert idx.size == bench.DUMP_VOXELS and 2 * idx.size * 4 <= 64 << 20     # zy + zyx in float32
+    assert np.all(np.diff(idx) > 0) and idx[0] >= 0 and idx[-1] < nvox
+    assert idx[-1] >= nvox - 2 * (nvox // idx.size)                          # reaches the end of the volume
+    assert np.array_equal(idx, bench.dump_sample_index(nvox))
+
+
+def _dump_worker(rank, world, port, shape, budget, out_dir):
+    import torch
+    import torch.distributed as dist
+    import bench
+    from flowdenoising_b200.dist import split_range
+    os.environ["MASTER_ADDR"] = "127.0.0.1"
+    os.environ["MASTER_PORT"] = str(port)
+    dist.init_process_group("gloo", rank=rank, world_size=world)
+    try:
+        bench.DUMP_VOXELS = budget
+        vol = np.arange(np.prod(shape), dtype=np.float32).reshape(shape)
+        z0, z1 = split_range(shape[0], world, rank)
+        bench.dump_outputs(out_dir, {"zyx": torch.from_numpy(vol[z0:z1].copy())}, shape, (z0, z1), rank, world)
+    finally:
+        dist.destroy_process_group()
+
+
+@pytest.mark.parametrize("world,budget", [(1, 10_000), (1, 500), (3, 10_000), (3, 500)])
+def test_dump_outputs_assembles_rank_slabs(tmp_path, monkeypatch, world, budget):
+    """Whole volume within the budget (shaped [Z][Y][X]), else the seeded sample in index order; uneven Z-slabs."""
+    import socket
+    pytest.importorskip("torch")
+    import torch.multiprocessing as mp
+    import bench
+    shape = (11, 13, 10)
+    with socket.socket() as s:
+        s.bind(("127.0.0.1", 0))
+        port = s.getsockname()[1]
+    mp.spawn(_dump_worker, args=(world, port, shape, budget, str(tmp_path)), nprocs=world, join=True)
+    got = np.load(tmp_path / "zyx.npy")
+    vol = np.arange(np.prod(shape), dtype=np.float32).reshape(shape)
+    monkeypatch.setattr(bench, "DUMP_VOXELS", budget)
+    want = vol if vol.size <= budget else vol.ravel()[bench.dump_sample_index(vol.size)]
+    assert got.dtype == np.float32 and got.shape == want.shape and np.array_equal(got, want)
