@@ -19,7 +19,10 @@ c_i64 = C.c_int64
 class OfParams(C.Structure):
     """struct fdn_of_params (reference constants: src/flowdenoising.py:47-53)."""
     _fields_ = [("levels", C.c_int), ("winsize", C.c_int), ("iterations", C.c_int), ("poly_n", C.c_int),
-                ("poly_sigma", C.c_double), ("use_prev_flow", C.c_int)]
+                ("poly_sigma", C.c_double), ("use_prev_flow", C.c_int), ("flags", C.c_int)]
+
+
+FARNEBACK_GAUSSIAN = 256   # FDN_OF_FARNEBACK_GAUSSIAN (= cv2.OPTFLOW_FARNEBACK_GAUSSIAN)
 
 
 class View(C.Structure):
@@ -75,6 +78,8 @@ SIGNATURES = {
                                      C.c_void_p, C.c_size_t, C.c_void_p]),
     "fdn_flow_iterations": (C.c_int, [c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, C.c_int,
                                       C.c_int, C.c_void_p, C.c_size_t, C.c_void_p, C.POINTER(C.c_void_p)]),
+    "fdn_flow_iterations_gaussian": (C.c_int, [c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, C.c_int, C.c_int, C.c_int,
+                                               C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_void_p)]),
     "fdn_set_flow_iter_variant": (None, [C.c_int]),
     "fdn_flow_area_down": (C.c_int, [c_f32p, C.c_int, C.c_int, C.c_int, c_f32p, C.c_int, C.c_int, C.c_float,
                                      C.c_void_p]),

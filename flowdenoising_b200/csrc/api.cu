@@ -53,7 +53,8 @@ static std::vector<cudaEvent_t> g_event_pool;
 static std::mutex g_prof_mutex;   // the record list is shared by every host thread that launches with profiling on
 static const char* const g_kernel_names[K_COUNT] = {
     "k_blur_rows", "k_blur_cols", "k_resize_linear_img", "k_polyexp", "k_flow_iter", "k_flow_area_down",
-    "k_flow_upsample", "k_warp_acc", "k_gauss_axis", "k_gauss_rows", "k_transpose", "k_copy3d"};
+    "k_flow_upsample", "k_warp_acc", "k_gauss_axis", "k_gauss_rows", "k_transpose", "k_copy3d",
+    "k_flow_gauss_iter"};
 
 static cudaEvent_t get_event()
 {
@@ -132,6 +133,8 @@ static int check_of(const fdn_of_params* of)
     FDN_CHECK_ARG(of->iterations >= 1, "iterations must be >= 1");
     FDN_CHECK_ARG(of->poly_n >= 1 && of->poly_n <= 7, "poly_n %d unsupported (1..7)", of->poly_n);
     FDN_CHECK_ARG(of->levels >= 0, "levels must be >= 0");
+    FDN_CHECK_ARG((of->flags & ~FDN_OF_FARNEBACK_GAUSSIAN) == 0, "unsupported flags 0x%x (only FDN_OF_FARNEBACK_GAUSSIAN)",
+                  (unsigned)of->flags);
     return FDN_OK;
 }
 
@@ -215,9 +218,13 @@ static int farneback_batch(const float* R, const Geometry& g, SlotMap map0, Slot
         const bool want_P = (k == 0);
         if ((slot == 1 && (a == P) != want_P) || (slot == 2 && (b == P) != want_P)) { float* t = a; a = b; b = t; }
         float* res = nullptr;
-        if ((rc = launch_flow_level(R + g.R_off[k], (int64_t)g.R_slot, map0, map1, cur, a, b, n, h, w, of.winsize, iters,
-                                    fs, st, &res)))
-            return rc;
+        if (of.flags & FDN_OF_FARNEBACK_GAUSSIAN)
+            rc = launch_flow_level_gauss(R + g.R_off[k], (int64_t)g.R_slot, map0, map1, cur, a, b, n, h, w, of.winsize,
+                                         iters, st, &res);
+        else
+            rc = launch_flow_level(R + g.R_off[k], (int64_t)g.R_slot, map0, map1, cur, a, b, n, h, w, of.winsize, iters,
+                                   fs, st, &res);
+        if (rc) return rc;
         cur = res;
         ch = h; cw = w;
     }
@@ -347,7 +354,7 @@ using namespace fdn;
 #pragma GCC visibility push(default)
 extern "C" {
 
-int fdn_version(void) { return 100; }
+int fdn_version(void) { return 101; }
 const char* fdn_last_error(void) { return g_err; }
 int64_t fdn_launch_count(void) { return g_launches.load(); }
 int64_t fdn_progress_milli(void) { return (int64_t)g_progress_milli.load(); }
@@ -615,6 +622,17 @@ int fdn_flow_iterations(const float* d_R0, const float* d_R1, float* d_flow, flo
     FDN_CHECK_ARG(delta % stride == 0, "R1 - R0 must be a multiple of one image (fdn_polyexp_floats(h, w))");
     return launch_flow_level(d_R0, stride, SlotMap{0, 0}, SlotMap{(int)(delta / stride), 0}, d_flow, d_tmp1, d_tmp2, n, h,
                              w, winsize, iterations, fs, st, d_result);
+}
+
+int fdn_flow_iterations_gaussian(const float* d_R0, const float* d_R1, float* d_flow, float* d_tmp1, float* d_tmp2, int n,
+                                 int h, int w, int winsize, int iterations, void* stream, float** d_result)
+{
+    FDN_CHECK_ARG(d_R0 && d_R1 && d_flow && d_tmp1 && d_tmp2 && n >= 1 && iterations >= 1 && d_result, "bad argument");
+    const int64_t stride = (int64_t)R_image_floats(h, w);
+    const ptrdiff_t delta = d_R1 - d_R0;
+    FDN_CHECK_ARG(delta % stride == 0, "R1 - R0 must be a multiple of one image (fdn_polyexp_floats(h, w))");
+    return launch_flow_level_gauss(d_R0, stride, SlotMap{0, 0}, SlotMap{(int)(delta / stride), 0}, d_flow, d_tmp1, d_tmp2,
+                                   n, h, w, winsize, iterations, static_cast<cudaStream_t>(stream), d_result);
 }
 
 int fdn_flow_iteration(const float* d_R0, const float* d_R1, const float* d_flow_in, float* d_flow_out, int n, int h,

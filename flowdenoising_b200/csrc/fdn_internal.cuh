@@ -52,7 +52,7 @@ static inline int64_t cdiv(int64_t a, int64_t b) { return (a + b - 1) / b; }
 // ---- optional per-kernel timing with CUDA events on the launching stream (bench.py roofline) ----
 enum KernelId {
     K_BLUR_ROWS = 0, K_BLUR_COLS, K_RESIZE_IMG, K_POLYEXP, K_FLOW_ITER, K_FLOW_AREA, K_FLOW_UP, K_WARP_ACC,
-    K_GAUSS_AXIS, K_GAUSS_ROWS, K_TRANSPOSE, K_COPY3D, K_COUNT
+    K_GAUSS_AXIS, K_GAUSS_ROWS, K_TRANSPOSE, K_COPY3D, K_FLOW_GAUSS, K_COUNT
 };
 extern bool g_prof_on;
 int prof_begin(int id, double algorithmic_bytes, cudaStream_t st, int n = 0, int h = 0, int w = 0);   // -> record index
@@ -131,7 +131,11 @@ int flow_iter_scratch_init(const FlowScratch& fs, cudaStream_t st);             
 int launch_flow_level(const float* R, int64_t R_stride, SlotMap map0, SlotMap map1, float* cur, float* a, float* b,
                       int n, int h, int w, int winsize, int iters, const FlowScratch& fs, cudaStream_t st,
                       float** result);
-// 0: strip kernel k_flow_iter everywhere, 1 (default): warp-specialised k_flow_iter_ws where it applies
+// The same with the Gaussian window (OPTFLOW_FARNEBACK_GAUSSIAN): one launch per iteration, no scratch.
+int launch_flow_level_gauss(const float* R, int64_t R_stride, SlotMap map0, SlotMap map1, float* cur, float* a,
+                            float* b, int n, int h, int w, int winsize, int iters, cudaStream_t st, float** result);
+// 0: strip kernel k_flow_iter everywhere, 1 (default): warp-specialised k_flow_iter_ws where it applies; with the
+// Gaussian window 0 selects the shared-memory-ring kernel for every winsize
 void set_flow_iter_variant(int v);
 int launch_flow_area_down(const float* flow, int n, int H, int W, float* out, int h, int w, float scale,
                           cudaStream_t st);

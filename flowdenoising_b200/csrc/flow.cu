@@ -21,6 +21,7 @@
 //   Every R0 / flow row is read once (no vertical halo), R1 gathers mostly hit L1/L2.
 //   Algorithmic HBM bytes per pixel: R0 20 + R1 20 + flow in 8 + flow out 8 = 56 (SURVEY.md §8d).
 // Compiled with -fmad=false: OpenCV's scalar code has no fused multiply-adds here.
+#include <math.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -1162,6 +1163,253 @@ int launch_flow_level(const float* R, int64_t R_stride, SlotMap map0, SlotMap ma
         int rc = m == 2 ? launch_ws<2>(wa, blocks, st) : launch_ws<4>(wa, blocks, st);
         if (rc) return rc;
         FDN_LAUNCHED("k_flow_iter_ws");
+    }
+    *result = bufs[iters % 3];
+    return FDN_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Gaussian window (OPTFLOW_FARNEBACK_GAUSSIAN, FarnebackUpdateFlow_GaussianBlur): M is smoothed by a separable
+// Gaussian of 2m+1 float32 taps (sigma = 0.3 m) instead of the box mean, then the same regularised solve without the
+// 1/winsize^2 scale. OpenCV's order, no FMA:
+//   vertical   v(y, x)  = M[y]*k0 + sum_{i=1..m} (M[min(y+i, h-1)] + M[max(y-i, 0)]) * k[i]     (float32)
+//   horizontal g(y, x)  = v[x]*k0 + sum_{i=1..m} (v[min(x+i, w-1)] + v[max(x-i, 0)]) * k[i]     (float32)
+// Nothing runs along a row or a column, so the filter is tile local and still bit exact: a block owns a strip of CW
+// output columns of one image pair plus an m-column halo on each side (128 threads, thread t <-> image column
+// x0 - m + t, clamped: the replicated border), and marches down the rows. Per row a thread computes M of the new row
+// y + m from R0, flow_in and the R1 gather (update_matrices_px, the arithmetic of phase V of k_flow_iter), keeps the
+// last 2m+1 rows of M in a ring, and writes the vertical sums of its column to a shared-memory tile; after a barrier
+// the CW core threads run the horizontal sums and the solve of the tile's rows. No carries, no tickets, no scratch:
+// blocks are independent. Rows past the bottom are recomputed at row h-1 and the m rows above the top hold M of
+// row 0, so every step of the march is the same. Algorithmic HBM bytes per pixel: 56, as for the box kernels.
+//   k_flow_gauss_iter       (MT = 2, 4: winsize 4/5, 8/9): the ring lives in registers, a tile is one ring period
+//                           (2m+1 rows) so every ring slot is a compile-time constant of the unrolled row loop;
+//   k_flow_gauss_iter_smem  (any m <= 15): the ring lives in shared memory, tiles of GW_TR rows.
+// ------------------------------------------------------------------------------------------------
+#define GW_NT 128
+#define GW_TR 8
+#define GW_MAX_M 15
+
+struct GaussIterArgs {
+    const float* R;      // level base inside slot 0 (layout as FlowIterArgs)
+    int64_t R_stride;
+    SlotMap map0, map1;
+    const float* flow_in;
+    float* flow_out;
+    int h, w, m;
+    int CW, strips;      // core columns per strip (GW_NT - 2m), strips per image
+    float k[GW_MAX_M + 1];
+};
+
+// taps as OpenCV builds them (float, normalised through a double sum)
+static void gauss_window_taps(int m, float* k)
+{
+    const double sigma = m * 0.3;
+    double s = 1;
+    k[0] = (float)s;
+    for (int i = 1; i <= m; i++) {
+        const float t = (float)exp(-i * i / (2 * sigma * sigma));
+        k[i] = t;
+        s += t * 2;
+    }
+    s = 1. / s;
+    for (int i = 0; i <= m; i++) k[i] = (float)(k[i] * s);
+}
+
+template <int MT>
+__global__ void __launch_bounds__(GW_NT, 4)
+k_flow_gauss_iter(GaussIterArgs a)
+{
+    constexpr bool kReg = MT > 0;
+    extern __shared__ __align__(16) float gw_smem[];
+    const int m = kReg ? MT : a.m;
+    const int RR = 2 * m + 1;
+    const int TR = kReg ? 2 * MT + 1 : GW_TR;
+    const int h = a.h, w = a.w;
+    float* tile = gw_smem;                       // [TR][5][GW_NT] vertical sums
+    float* ring = gw_smem + TR * 5 * GW_NT + threadIdx.x;   // [RR][5][GW_NT] rows of M (shared-memory variant)
+
+    const int t = threadIdx.x;
+    const int b = blockIdx.x / a.strips, k = blockIdx.x - b * a.strips;
+    const int x0 = k * a.CW;
+    const int xcol = x0 - m + t;
+    const bool active = xcol <= w - 1 + m;       // columns past the right halo of a narrow image are not needed
+    const int xcl = min(max(xcol, 0), w - 1);
+    const bool core = t < a.CW && x0 + t < w;
+
+    const float* R0 = a.R + (int64_t)a.map0.slot(b) * a.R_stride;
+    const float* R1 = a.R + (int64_t)a.map1.slot(b) * a.R_stride;
+    const float4* R0a = reinterpret_cast<const float4*>(R0);
+    const float4* R1a = reinterpret_cast<const float4*>(R1);
+    const float* R0b = R0 + (int64_t)4 * h * w;
+    const float* R1b = R1 + (int64_t)4 * h * w;
+    const float2* fin = reinterpret_cast<const float2*>(a.flow_in) + (int64_t)b * h * w;
+    float2* fout = reinterpret_cast<float2*>(a.flow_out) + (int64_t)b * h * w;
+
+    auto matrices = [&](int row, float M[5]) {
+        update_matrices_px(R0a, R0b, R1a, R1b, __ldg(fin + row * w + xcl), xcl, row, h, w, M);
+    };
+    // horizontal sums + solve of tile row r (image row y), core threads
+    auto solve_row = [&](int r, int y) {
+        const float* tl = tile + r * 5 * GW_NT + t + m;
+        double g[5];
+#pragma unroll
+        for (int c = 0; c < 5; c++) {
+            const float* v = tl + c * GW_NT;
+            float s = __fmul_rn(v[0], a.k[0]);
+            if (kReg) {
+#pragma unroll
+                for (int i = 1; i <= MT; i++) s = __fadd_rn(s, __fmul_rn(__fadd_rn(v[i], v[-i]), a.k[i]));
+            } else {
+                for (int i = 1; i <= m; i++) s = __fadd_rn(s, __fmul_rn(__fadd_rn(v[i], v[-i]), a.k[i]));
+            }
+            g[c] = (double)s;
+        }
+        const double det = __dadd_rn(__dsub_rn(__dmul_rn(g[0], g[2]), __dmul_rn(g[1], g[1])), 1e-3);
+        const double idet = __drcp_rn(det);   // == 1./det correctly rounded
+        float2 o;
+        o.x = (float)__dmul_rn(__dsub_rn(__dmul_rn(g[0], g[4]), __dmul_rn(g[1], g[3])), idet);
+        o.y = (float)__dmul_rn(__dsub_rn(__dmul_rn(g[2], g[3]), __dmul_rn(g[1], g[4])), idet);
+        fout[y * w + x0 + t] = o;
+    };
+
+    if constexpr (kReg) {
+        constexpr int RRc = 2 * MT + 1;
+        float rg[RRc][5];   // row j of M in slot j mod RR (rows -m..-1 hold row 0)
+        if (active) {
+            float M0[5];
+            matrices(0, M0);
+#pragma unroll
+            for (int j = -MT; j <= 0; j++)
+#pragma unroll
+                for (int c = 0; c < 5; c++) rg[(j + RRc) % RRc][c] = M0[c];
+#pragma unroll
+            for (int j = 1; j < MT; j++) matrices(min(j, h - 1), rg[j]);
+        }
+        for (int y0 = 0; y0 < h; y0 += RRc) {   // y0 = 0 mod RR: row y0 + r + i sits in slot (r + i) mod RR
+            if (active) {
+#pragma unroll
+                for (int r = 0; r < RRc; r++) {
+                    const int y = y0 + r;
+                    if (y < h) {
+                        matrices(min(y + MT, h - 1), rg[(r + MT) % RRc]);
+#pragma unroll
+                        for (int c = 0; c < 5; c++) {
+                            float s = __fmul_rn(rg[r][c], a.k[0]);
+#pragma unroll
+                            for (int i = 1; i <= MT; i++)
+                                s = __fadd_rn(s, __fmul_rn(__fadd_rn(rg[(r + i) % RRc][c], rg[(r - i + RRc) % RRc][c]),
+                                                          a.k[i]));
+                            tile[(r * 5 + c) * GW_NT + t] = s;
+                        }
+                    }
+                }
+            }
+            __syncthreads();
+            if (core) {
+#pragma unroll
+                for (int r = 0; r < RRc; r++)
+                    if (y0 + r < h) solve_row(r, y0 + r);
+            }
+            __syncthreads();
+        }
+    } else {
+        // ring slot of row j: (j + m) mod RR, kept as a running index (rows -m..-1 hold row 0)
+        if (active) {
+            float M0[5];
+            matrices(0, M0);
+            for (int j = -m; j <= 0; j++)
+#pragma unroll
+                for (int c = 0; c < 5; c++) ring[((j + m) * 5 + c) * GW_NT] = M0[c];
+            for (int j = 1; j < m; j++) {
+                float Mv[5];
+                matrices(min(j, h - 1), Mv);
+#pragma unroll
+                for (int c = 0; c < 5; c++) ring[((j + m) * 5 + c) * GW_NT] = Mv[c];
+            }
+        }
+        int sy = m;   // slot of row y
+        for (int y0 = 0; y0 < h; y0 += GW_TR) {
+            if (active) {
+                for (int r = 0; r < GW_TR && y0 + r < h; r++) {
+                    const int y = y0 + r;
+                    int sn = sy + m;   // slot of the new row y + m
+                    if (sn >= RR) sn -= RR;
+                    float Mv[5];
+                    matrices(min(y + m, h - 1), Mv);
+#pragma unroll
+                    for (int c = 0; c < 5; c++) ring[(sn * 5 + c) * GW_NT] = Mv[c];
+#pragma unroll
+                    for (int c = 0; c < 5; c++) {
+                        const float* rc = ring + c * GW_NT;
+                        float s = __fmul_rn(rc[sy * 5 * GW_NT], a.k[0]);
+                        int sd = sy, su = sy;
+                        for (int i = 1; i <= m; i++) {
+                            if (++sd == RR) sd = 0;
+                            if (--su < 0) su = RR - 1;
+                            s = __fadd_rn(s, __fmul_rn(__fadd_rn(rc[sd * 5 * GW_NT], rc[su * 5 * GW_NT]), a.k[i]));
+                        }
+                        tile[(r * 5 + c) * GW_NT + t] = s;
+                    }
+                    if (++sy == RR) sy = 0;
+                }
+            }
+            __syncthreads();
+            if (core) {
+                for (int r = 0; r < GW_TR && y0 + r < h; r++) solve_row(r, y0 + r);
+            }
+            __syncthreads();
+        }
+    }
+}
+
+static size_t gauss_smem_bytes(int MT, int m)
+{
+    const int TR = MT > 0 ? 2 * MT + 1 : GW_TR;
+    return sizeof(float) * 5 * GW_NT * (size_t)(TR + (MT > 0 ? 0 : 2 * m + 1));
+}
+
+template <int MT>
+static int launch_gauss_variant(const GaussIterArgs& a, unsigned blocks, cudaStream_t st)
+{
+    static std::atomic<bool> seen[64];
+    if (first_use_on_device(seen))
+        FDN_CUDA(cudaFuncSetAttribute(k_flow_gauss_iter<MT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)gauss_smem_bytes(MT, GW_MAX_M)));
+    k_flow_gauss_iter<MT><<<blocks, GW_NT, gauss_smem_bytes(MT, a.m), st>>>(a);
+    return FDN_OK;
+}
+
+int launch_flow_level_gauss(const float* R, int64_t R_stride, SlotMap map0, SlotMap map1, float* cur, float* bufa,
+                            float* bufb, int n, int h, int w, int winsize, int iters, cudaStream_t st, float** result)
+{
+    FDN_CHECK_ARG(winsize >= 1 && winsize <= 31, "winsize %d unsupported (1..31)", winsize);
+    FDN_CHECK_ARG(cur != bufa && cur != bufb && bufa != bufb, "the three flow buffers must be distinct");
+    FDN_CHECK_ARG((int64_t)h * w < (1ll << 28), "level image too large");
+    GaussIterArgs a;
+    a.R = R; a.R_stride = R_stride;
+    a.map0 = map0; a.map1 = map1;
+    a.h = h; a.w = w; a.m = winsize / 2;
+    a.CW = GW_NT - 2 * a.m;
+    a.strips = (int)cdiv(w, a.CW);
+    FDN_CHECK_ARG((int64_t)n * a.strips < (1ll << 31), "too many image pairs in one launch");
+    gauss_window_taps(a.m, a.k);
+    const unsigned blocks = (unsigned)n * (unsigned)a.strips;
+    const bool reg = g_flow_variant.load() == 1 && (a.m == 2 || a.m == 4);
+    float* bufs[3] = {cur, bufa, bufb};
+    for (int i = 0; i < iters; i++) {
+        a.flow_in = bufs[i % 3];
+        a.flow_out = bufs[(i + 1) % 3];
+        ProfScope ps(K_FLOW_GAUSS, 56.0 * n * h * w, st, n, h, w);
+        int rc;
+        if (reg) {
+            rc = a.m == 2 ? launch_gauss_variant<2>(a, blocks, st) : launch_gauss_variant<4>(a, blocks, st);
+            if (rc) return rc;
+            FDN_LAUNCHED("k_flow_gauss_iter");
+        } else {
+            if ((rc = launch_gauss_variant<0>(a, blocks, st))) return rc;
+            FDN_LAUNCHED("k_flow_gauss_iter_smem");
+        }
     }
     *result = bufs[iters % 3];
     return FDN_OK;

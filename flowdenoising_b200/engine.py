@@ -15,7 +15,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 from . import _lib
-from ._lib import OfParams, View
+from ._lib import FARNEBACK_GAUSSIAN, OfParams, View
 
 # reference defaults, src/flowdenoising.py:47-53
 OF_LEVELS = 3
@@ -34,10 +34,13 @@ class FlowParams:
     poly_n: int = OF_POLY_N
     poly_sigma: float = OF_POLY_SIGMA
     use_prev_flow: bool = True
+    # OPTFLOW_FARNEBACK_GAUSSIAN: Gaussian window instead of the box mean (a different flow estimate)
+    gaussian_window: bool = False
 
     def c_struct(self) -> OfParams:
         return OfParams(int(self.levels), int(self.winsize), int(self.iterations), int(self.poly_n),
-                        float(self.poly_sigma), int(bool(self.use_prev_flow)))
+                        float(self.poly_sigma), int(bool(self.use_prev_flow)),
+                        FARNEBACK_GAUSSIAN if self.gaussian_window else 0)
 
 
 def gaussian_kernel(sigma: float) -> np.ndarray:

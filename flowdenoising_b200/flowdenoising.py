@@ -391,7 +391,7 @@ def warp_slice(reference, flow):
     return acc[0].cpu().numpy()
 
 
-def _get_flow(reference, target, l, w, prev_flow, use_prev, iterations, poly_n, poly_sigma):
+def _get_flow(reference, target, l, w, prev_flow, use_prev, iterations, poly_n, poly_sigma, gaussian_window):
     eng = _get_engine()
     torch = eng.torch
     ref = _to_dev(reference, torch, eng.device)[None]
@@ -402,7 +402,8 @@ def _get_flow(reference, target, l, w, prev_flow, use_prev, iterations, poly_n, 
         fl = _to_dev(prev_flow, torch, eng.device)[None].contiguous()
     else:
         fl = torch.zeros(ref.shape + (2,), dtype=torch.float32, device=eng.device)
-    p = FlowParams(int(l), int(w), int(iterations), int(poly_n), float(poly_sigma), bool(use_prev))
+    p = FlowParams(int(l), int(w), int(iterations), int(poly_n), float(poly_sigma), bool(use_prev),
+                   bool(gaussian_window))
     # cv2.calcOpticalFlowFarneback(prev=target, next=reference, ...)
     eng.farneback(tgt, ref, fl, p)
     out = fl[0].cpu().numpy()
@@ -414,15 +415,15 @@ def _get_flow(reference, target, l, w, prev_flow, use_prev, iterations, poly_n, 
 
 
 def get_flow_with_prev_flow(reference, target, l=OF_LEVELS, w=OF_WINDOW_SIZE, prev_flow=None,
-                            iterations=OF_ITERS, poly_n=OF_POLY_N, poly_sigma=OF_POLY_SIGMA):
-    '''src/flowdenoising.py:65-87 (OPTFLOW_USE_INITIAL_FLOW).'''
-    return _get_flow(reference, target, l, w, prev_flow, True, iterations, poly_n, poly_sigma)
+                            iterations=OF_ITERS, poly_n=OF_POLY_N, poly_sigma=OF_POLY_SIGMA, gaussian_window=False):
+    '''src/flowdenoising.py:65-87 (OPTFLOW_USE_INITIAL_FLOW); gaussian_window adds OPTFLOW_FARNEBACK_GAUSSIAN.'''
+    return _get_flow(reference, target, l, w, prev_flow, True, iterations, poly_n, poly_sigma, gaussian_window)
 
 
 def get_flow_without_prev_flow(reference, target, l=OF_LEVELS, w=OF_WINDOW_SIZE, prev_flow=None,
-                               iterations=OF_ITERS, poly_n=OF_POLY_N, poly_sigma=OF_POLY_SIGMA):
-    '''src/flowdenoising.py:89-114 (--recompute_flow).'''
-    return _get_flow(reference, target, l, w, None, False, iterations, poly_n, poly_sigma)
+                               iterations=OF_ITERS, poly_n=OF_POLY_N, poly_sigma=OF_POLY_SIGMA, gaussian_window=False):
+    '''src/flowdenoising.py:89-114 (--recompute_flow); gaussian_window adds OPTFLOW_FARNEBACK_GAUSSIAN.'''
+    return _get_flow(reference, target, l, w, None, False, iterations, poly_n, poly_sigma, gaussian_window)
 
 
 class GaussianDenoising():
@@ -752,14 +753,15 @@ class FlowDenoising(GaussianDenoising):
     ``warp_slice`` is accepted for signature compatibility (the remap is fused into the accumulation kernel).'''
 
     def __init__(self, number_of_processes, vol, l=OF_LEVELS, w=OF_WINDOW_SIZE, get_flow=None, warp_slice=None,
-                 iterations=OF_ITERS, poly_n=OF_POLY_N, poly_sigma=OF_POLY_SIGMA):
+                 iterations=OF_ITERS, poly_n=OF_POLY_N, poly_sigma=OF_POLY_SIGMA, gaussian_window=False):
         super().__init__(number_of_processes, vol)
         self.l = l
         self.w = w
         self.get_flow = get_flow if get_flow is not None else get_flow_with_prev_flow
         self.warp_slice = warp_slice
         use_prev = self.get_flow is not get_flow_without_prev_flow
-        self._flow_params = FlowParams(int(l), int(w), int(iterations), int(poly_n), float(poly_sigma), use_prev)
+        self._flow_params = FlowParams(int(l), int(w), int(iterations), int(poly_n), float(poly_sigma), use_prev,
+                                       bool(gaussian_window))
 
 
 def int_or_str(text):
@@ -775,7 +777,8 @@ number_of_PUs = multiprocessing.cpu_count()
 
 def build_parser():
     '''Same flags and defaults as src/flowdenoising.py:382-415, plus --iterations/--poly_n/--poly_sigma
-    (fixed constants in the reference, :50-52) and --compat_zy_output (reproduces quirk Q1).'''
+    (fixed constants in the reference, :50-52), --gaussian_window (OpenCV's OPTFLOW_FARNEBACK_GAUSSIAN) and
+    --compat_zy_output (reproduces quirk Q1).'''
     parser = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.ArgumentDefaultsHelpFormatter)
     parser.add_argument("-i", "--input", type=int_or_str, help="Input a MRC-file or a multi-image TIFF-file",
                         default="./volume.mrc")
@@ -809,6 +812,10 @@ def build_parser():
     parser.add_argument("--iterations", type=int, default=OF_ITERS, help="Farneback iterations per pyramid level")
     parser.add_argument("--poly_n", type=int, default=OF_POLY_N, help="Farneback polynomial-expansion neighbourhood")
     parser.add_argument("--poly_sigma", type=float, default=OF_POLY_SIGMA, help="Farneback polynomial-expansion sigma")
+    parser.add_argument("--gaussian_window", action="store_true",
+                        help="Farneback with a Gaussian window instead of the box window (cv2.OPTFLOW_FARNEBACK_GAUSSIAN): "
+                             "changes the flow estimate, usually more accurate; it is not a speed switch. Wants a larger "
+                             "--winsize for the same robustness; winsize 2m and 2m+1 give the same window")
     parser.add_argument("--compat_zy_output", action="store_true",
                         help="Write the Z+Y intermediate like the reference CLI does (flowdenoising.py:520) "
                              "instead of the full Z+Y+X result")
@@ -877,7 +884,8 @@ def main(argv=None):
         fd = GaussianDenoising(args.number_of_processes, vol)
     else:
         fd = FlowDenoising(args.number_of_processes, vol, args.levels, args.winsize, get_flow, warp_slice,
-                           iterations=args.iterations, poly_n=args.poly_n, poly_sigma=args.poly_sigma)
+                           iterations=args.iterations, poly_n=args.poly_n, poly_sigma=args.poly_sigma,
+                           gaussian_window=args.gaussian_window)
     fd.border = args.border
     fd.slab_slices = args.slab_slices
     if args.gpus > 1:

@@ -45,6 +45,12 @@ extern "C" {
 
 #define FDN_MAX_LEVELS 16
 
+/* fdn_of_params.flags: OpenCV's OPTFLOW_FARNEBACK_GAUSSIAN (same value). The matrices of the displacement update are
+ * smoothed by a separable Gaussian window (2m+1 taps, m = winsize/2, sigma = 0.3 m) instead of the winsize x winsize
+ * box mean: a different, usually more accurate flow estimate, not a speed switch. winsize 2m and 2m+1 are the same
+ * window in this mode. */
+#define FDN_OF_FARNEBACK_GAUSSIAN 256
+
 /* Farneback parameters (reference constants src/flowdenoising.py:47-53; pyr_scale is fixed at 0.5 like :73) */
 typedef struct fdn_of_params {
     int levels;          /* -l  (OF_LEVELS = 3): EXTRA pyramid levels, cropped while min(W,H)*0.5^k >= 32 */
@@ -53,6 +59,7 @@ typedef struct fdn_of_params {
     int poly_n;          /* OF_POLY_N = 5 (5 or 7 as in OpenCV) */
     double poly_sigma;   /* OF_POLY_SIGMA = 1.2 */
     int use_prev_flow;   /* 1: chain flows (get_flow_with_prev_flow), 0: --recompute_flow */
+    int flags;           /* 0 (box window) or FDN_OF_FARNEBACK_GAUSSIAN; any other bit is rejected */
 } fdn_of_params;
 
 /* Geometry of one volume view of a pass. The view holds n_in slices of (H, W). Output slice s (0..n_out-1)
@@ -168,8 +175,14 @@ int fdn_flow_iteration(const float* d_R0, const float* d_R1, const float* d_flow
 int fdn_flow_iterations(const float* d_R0, const float* d_R1, float* d_flow, float* d_tmp1, float* d_tmp2, int n,
                         int h, int w, int winsize, int iterations, void* d_scratch, size_t scratch_bytes,
                         void* stream, float** d_result);
+/* The same iterations with the Gaussian window (FDN_OF_FARNEBACK_GAUSSIAN): one launch per iteration, blocks without
+ * dependencies on each other, so no scratch. winsize 1..31. */
+int fdn_flow_iterations_gaussian(const float* d_R0, const float* d_R1, float* d_flow, float* d_tmp1, float* d_tmp2,
+                                 int n, int h, int w, int winsize, int iterations, void* stream, float** d_result);
 /* Development / test switch: 1 (default) = warp-specialised k_flow_iter_ws where it applies, 0 = the strip kernel
- * k_flow_iter everywhere (the two are compared bit for bit by tests/test_gpu_stages.py). Process-wide. */
+ * k_flow_iter everywhere (the two are compared bit for bit by tests/test_gpu_stages.py). With the Gaussian window,
+ * 1 = the register-ring kernel for winsize 4, 5, 8, 9 and 0 = the shared-memory-ring kernel everywhere (compared bit for
+ * bit by tests/test_gpu_gaussian_window.py). Process-wide. */
 void fdn_set_flow_iter_variant(int variant);
 /* Flow resampling between levels: INTER_AREA down-scale * scale (initial flow, coarsest level) and
  * INTER_LINEAR up-scale * 2 (next finer level). */
