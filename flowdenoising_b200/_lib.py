@@ -24,6 +24,9 @@ class OfParams(C.Structure):
 
 FARNEBACK_GAUSSIAN = 256   # FDN_OF_FARNEBACK_GAUSSIAN (= cv2.OPTFLOW_FARNEBACK_GAUSSIAN)
 
+# FDN_DTYPE_*: element types of typed volumes (the reference's integer semantics, opt-in)
+DTYPE_F32, DTYPE_U8, DTYPE_I8, DTYPE_U16, DTYPE_I16 = 0, 1, 2, 3, 4
+
 
 class View(C.Structure):
     """struct fdn_view."""
@@ -87,6 +90,15 @@ SIGNATURES = {
     "fdn_farneback_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.POINTER(OfParams)]),
     "fdn_farneback": (C.c_int, [c_f32p, c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, C.POINTER(OfParams), C.c_void_p,
                                 C.c_size_t, C.c_void_p]),
+    "fdn_workspace_bytes_typed": (C.c_size_t, [C.POINTER(View), C.c_int, C.POINTER(OfParams), C.c_int, C.c_int]),
+    "fdn_filter_axis_typed": (C.c_int, [c_f32p, c_f32p, C.c_int, C.POINTER(View), C.POINTER(C.c_double), C.c_int,
+                                        C.POINTER(OfParams), C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "fdn_gauss_axis_typed": (C.c_int, [c_f32p, c_f32p, C.c_int, C.POINTER(View), C.POINTER(C.c_double), C.c_int,
+                                       C.c_int, C.c_void_p]),
+    "fdn_gauss_rows_typed": (C.c_int, [c_f32p, c_f32p, C.c_int, c_i64, C.c_int, C.POINTER(C.c_double), C.c_int,
+                                       C.c_int, C.c_void_p]),
+    "fdn_transpose_yx_typed": (C.c_int, [c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "fdn_remap_typed": (C.c_int, [c_f32p, c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "fdn_warp_accumulate": (C.c_int, [c_f32p, c_i64, c_i64, c_f32p, C.c_double, c_f32p, c_i64, c_i64, C.c_int,
                                       C.c_int, C.c_int, C.c_void_p]),
 }

@@ -139,8 +139,9 @@ static int check_of(const fdn_of_params* of)
 }
 
 // Pyramid + polynomial expansion of `n` images (view-strided input, image b = input slice in_map.slot(b)) into
-// R slots R_map.slot(b). tmpA/tmpB/img: scratch of n*H*W floats each.
-static int build_R(const float* in, int64_t in_ss, int64_t in_rs, SlotMap in_map, int n, int H, int W,
+// R slots R_map.slot(b). tmpA/tmpB/img: scratch of n*H*W floats each. T: element type of the input view.
+template <typename T>
+static int build_R(const T* in, int64_t in_ss, int64_t in_rs, SlotMap in_map, int n, int H, int W,
                    const Geometry& g, const PolyConsts& pc, float* R, SlotMap R_map, float* tmpA, float* tmpB,
                    float* img, cudaStream_t st)
 {
@@ -235,10 +236,12 @@ static int farneback_batch(const float* R, const Geometry& g, SlotMap map0, Slot
 struct PassPlan {
     int chunk, r, slots, full_wrap;
     Geometry g;
-    size_t off_R, off_P, off_S1, off_S2, off_stash, off_scratch, scratch_bytes, total;
+    size_t off_R, off_P, off_S1, off_S2, off_stash, off_scratch, scratch_bytes, off_acc, total;
 };
 
-static int make_plan(const fdn_view& v, int klen, const fdn_of_params& of, int chunk, PassPlan* p)
+// esize: bytes per element of the volume (4: float32, whose accumulator is the output itself; 1 or 2: a typed volume,
+// whose stash holds T and whose float32 accumulator for one chunk follows the other buffers)
+static int make_plan(const fdn_view& v, int klen, const fdn_of_params& of, int chunk, size_t esize, PassPlan* p)
 {
     int rc;
     FDN_CHECK_ARG(klen >= 1 && (klen & 1), "kernel length must be odd (src/flowdenoising.py:309)");
@@ -267,19 +270,25 @@ static int make_plan(const fdn_view& v, int klen, const fdn_of_params& of, int c
     p->off_P = off;  off += align_up(fl, 256);
     p->off_S1 = off; off += align_up(fl, 256);
     p->off_S2 = off; off += align_up(fl, 256);
-    p->off_stash = off; off += align_up(sizeof(float) * px * (size_t)p->r, 256);   // remapped forward neighbours
+    p->off_stash = off; off += align_up(esize * px * (size_t)p->r, 256);   // remapped forward neighbours
     p->scratch_bytes = flow_iter_scratch_bytes(2 * chunk, v.H, v.W);  // level 0 is the largest
     p->off_scratch = off; off += align_up(p->scratch_bytes, 256);
+    p->off_acc = off;
+    if (esize != sizeof(float)) off += align_up(sizeof(float) * px, 256);
     p->total = off;
     return FDN_OK;
 }
 
-static int filter_axis_of(const float* d_in, float* d_out, const fdn_view& v, const double* kernel, int klen,
+// T = float: the accumulator is d_out itself. Integer T: a float32 accumulator of one chunk in the workspace; the last
+// tap truncates it into d_out (the reference's `filtered_vol[z] = tmp_slice` into an integer volume).
+template <typename T>
+static int filter_axis_of(const T* d_in, T* d_out, const fdn_view& v, const double* kernel, int klen,
                           const fdn_of_params& of, int chunk, void* ws, size_t ws_bytes, cudaStream_t st)
 {
+    constexpr bool typed = !std::is_same<T, float>::value;
     int rc;
     PassPlan p;
-    if ((rc = make_plan(v, klen, of, chunk, &p))) return rc;
+    if ((rc = make_plan(v, klen, of, chunk, sizeof(T), &p))) return rc;
     if (ws_bytes < p.total || ws == nullptr) {
         set_error("workspace too small: need %zu bytes, got %zu", p.total, ws_bytes);
         return FDN_ERR_WORKSPACE;
@@ -290,7 +299,7 @@ static int filter_axis_of(const float* d_in, float* d_out, const fdn_view& v, co
     float* P = reinterpret_cast<float*>(base + p.off_P);
     float* S1 = reinterpret_cast<float*>(base + p.off_S1);
     float* S2 = reinterpret_cast<float*>(base + p.off_S2);
-    float* stash = reinterpret_cast<float*>(base + p.off_stash);
+    T* stash = reinterpret_cast<T*>(base + p.off_stash);
     FlowScratch fs;
     if ((rc = flow_scratch_make(base + p.off_scratch, p.scratch_bytes, 2 * p.chunk, H, W, &fs))) return rc;
     if ((rc = flow_iter_scratch_init(fs, st))) return rc;
@@ -323,7 +332,9 @@ static int filter_axis_of(const float* d_in, float* d_out, const fdn_view& v, co
         const int cbase = p.full_wrap ? c0 + v.halo : r;             // R slot of the chunk's first centre slice
         const int swrap = p.full_wrap ? v.n_in : 0;
         SlotMap map0{cbase, swrap, C, cbase};
-        float* acc = d_out + (int64_t)c0 * v.out_slice_stride;
+        T* out = d_out + (int64_t)c0 * v.out_slice_stride;
+        float* acc = typed ? reinterpret_cast<float*>(base + p.off_acc) : reinterpret_cast<float*>(out);
+        const int64_t a_ss = typed ? (int64_t)H * W : v.out_slice_stride, a_rs = typed ? (int64_t)W : v.out_row_stride;
         const size_t fbytes = sizeof(float) * 2 * 2 * (size_t)C * H * W;
         if (r > 0) FDN_CUDA(cudaMemsetAsync(P, 0, fbytes, st));  // prev_flow = zeros (:310, :318)
         for (int d = 1; d <= r; d++) {
@@ -332,18 +343,36 @@ static int filter_axis_of(const float* d_in, float* d_out, const fdn_view& v, co
             // backward neighbour: tap r-d accumulated now (reference order -1, -2, ..., -r); forward neighbour:
             // remapped now, applied by launch_acc_finish after the centre tap (order 0, +1, ..., +r)
             SlotMap nmap{c0 + v.halo - d, wrap_in, C, c0 + v.halo + d};
-            if ((rc = launch_warp_pair(d_in, v.in_slice_stride, v.in_row_stride, nmap, P, kernel[r - d], acc,
-                                       v.out_slice_stride, v.out_row_stride, stash + (size_t)(d - 1) * C * H * W, C, H, W,
-                                       d == 1 ? 1 : 0, st)))
+            if ((rc = launch_warp_pair(d_in, v.in_slice_stride, v.in_row_stride, nmap, P, kernel[r - d], acc, a_ss, a_rs,
+                                       stash + (size_t)(d - 1) * C * H * W, C, H, W, d == 1 ? 1 : 0, st)))
                 return rc;
             progress_add(st, 1000ll * C / (r + 1));
         }
         SlotMap cmap{c0 + v.halo, wrap_in};
-        if ((rc = launch_acc_finish(d_in, v.in_slice_stride, v.in_row_stride, cmap, stash, r, kernel + r, acc,
-                                    v.out_slice_stride, v.out_row_stride, C, H, W, r > 0 ? 1 : 0, st)))
+        if ((rc = launch_acc_finish(d_in, v.in_slice_stride, v.in_row_stride, cmap, stash, r, kernel + r, acc, a_ss, a_rs,
+                                    out, v.out_slice_stride, v.out_row_stride, C, H, W, r > 0 ? 1 : 0, st)))
             return rc;
         progress_add(st, 1000ll * C - (long long)r * (1000ll * C / (r + 1)));
     }
+    return FDN_OK;
+}
+
+// ---- typed volumes (FDN_DTYPE_*) ----
+static size_t dtype_size(int dtype)
+{
+    switch (dtype) {
+        case FDN_DTYPE_F32: return 4;
+        case FDN_DTYPE_U8: case FDN_DTYPE_I8: return 1;
+        case FDN_DTYPE_U16: case FDN_DTYPE_I16: return 2;
+        default: return 0;
+    }
+}
+
+static int check_dtype(int dtype, bool with_of)
+{
+    FDN_CHECK_ARG(dtype_size(dtype) != 0, "unknown dtype %d (FDN_DTYPE_F32, _U8, _I8, _U16 or _I16)", dtype);
+    FDN_CHECK_ARG(!(with_of && dtype == FDN_DTYPE_I8),
+                  "int8 volumes are supported without optical flow only (cv2.remap rejects int8 images)");
     return FDN_OK;
 }
 
@@ -504,7 +533,7 @@ size_t fdn_workspace_bytes(const fdn_view* view, int klen, const fdn_of_params* 
     if (!view) { set_error("null view"); return 0; }
     if (!of) return 0;  // the no-OF path needs no workspace
     PassPlan p;
-    if (make_plan(*view, klen, *of, chunk, &p)) return 0;
+    if (make_plan(*view, klen, *of, chunk, sizeof(float), &p)) return 0;
     return p.total;
 }
 
@@ -515,6 +544,137 @@ int fdn_filter_axis(const float* d_in, float* d_out, const fdn_view* view, const
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (!of) return fdn_gauss_axis(d_in, d_out, view, kernel, klen, 1, stream);
     return filter_axis_of(d_in, d_out, *view, kernel, klen, *of, chunk, d_workspace, workspace_bytes, st);
+}
+
+size_t fdn_workspace_bytes_typed(const fdn_view* view, int klen, const fdn_of_params* of, int chunk, int dtype)
+{
+    if (!view) { set_error("null view"); return 0; }
+    if (check_dtype(dtype, of != nullptr)) return 0;
+    if (!of) return 0;
+    PassPlan p;
+    if (make_plan(*view, klen, *of, chunk, dtype_size(dtype), &p)) return 0;
+    return p.total;
+}
+
+int fdn_filter_axis_typed(const void* d_in, void* d_out, int dtype, const fdn_view* view, const double* kernel, int klen,
+                          const fdn_of_params* of, int chunk, void* d_workspace, size_t workspace_bytes, void* stream)
+{
+    FDN_CHECK_ARG(d_in && d_out && view && kernel, "null argument");
+    int rc;
+    if ((rc = check_dtype(dtype, of != nullptr))) return rc;
+    if (!of) return fdn_gauss_axis_typed(d_in, d_out, dtype, view, kernel, klen, 1, stream);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    switch (dtype) {
+        case FDN_DTYPE_U8:
+            return filter_axis_of(static_cast<const uint8_t*>(d_in), static_cast<uint8_t*>(d_out), *view, kernel, klen, *of,
+                                  chunk, d_workspace, workspace_bytes, st);
+        case FDN_DTYPE_U16:
+            return filter_axis_of(static_cast<const uint16_t*>(d_in), static_cast<uint16_t*>(d_out), *view, kernel, klen,
+                                  *of, chunk, d_workspace, workspace_bytes, st);
+        case FDN_DTYPE_I16:
+            return filter_axis_of(static_cast<const int16_t*>(d_in), static_cast<int16_t*>(d_out), *view, kernel, klen, *of,
+                                  chunk, d_workspace, workspace_bytes, st);
+        default:
+            return fdn_filter_axis(static_cast<const float*>(d_in), static_cast<float*>(d_out), view, kernel, klen, of,
+                                   chunk, d_workspace, workspace_bytes, stream);
+    }
+}
+
+int fdn_gauss_axis_typed(const void* d_in, void* d_out, int dtype, const fdn_view* view, const double* kernel, int klen,
+                         int exact, void* stream)
+{
+    int rc;
+    if ((rc = check_dtype(dtype, false))) return rc;
+    if (dtype == FDN_DTYPE_F32)
+        return fdn_gauss_axis(static_cast<const float*>(d_in), static_cast<float*>(d_out), view, kernel, klen, exact,
+                              stream);
+    FDN_CHECK_ARG(exact, "typed volumes run the exact no-OF arithmetic only (the fast mode moves truncation boundaries)");
+    FDN_CHECK_ARG(d_in && d_out && view && kernel, "null argument");
+    const fdn_view& v = *view;
+    FDN_CHECK_ARG(klen >= 1 && (klen & 1), "kernel length must be odd");
+    FDN_CHECK_ARG(v.n_in >= 1 && v.n_out >= 1 && v.H >= 1 && v.W >= 1, "empty view");
+    if (v.periodic) FDN_CHECK_ARG(v.halo >= 0 && v.halo < v.n_in && v.n_out <= v.n_in,
+                                  "periodic views need 0 <= halo < n_in and n_out <= n_in");
+    else FDN_CHECK_ARG(v.halo >= klen / 2 && v.n_in >= v.n_out + v.halo + klen / 2, "halo too small");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    switch (dtype) {
+        case FDN_DTYPE_U8:
+            rc = launch_gauss_axis_typed(static_cast<const uint8_t*>(d_in), static_cast<uint8_t*>(d_out), v, kernel, klen, st);
+            break;
+        case FDN_DTYPE_I8:
+            rc = launch_gauss_axis_typed(static_cast<const int8_t*>(d_in), static_cast<int8_t*>(d_out), v, kernel, klen, st);
+            break;
+        case FDN_DTYPE_U16:
+            rc = launch_gauss_axis_typed(static_cast<const uint16_t*>(d_in), static_cast<uint16_t*>(d_out), v, kernel, klen,
+                                         st);
+            break;
+        default:
+            rc = launch_gauss_axis_typed(static_cast<const int16_t*>(d_in), static_cast<int16_t*>(d_out), v, kernel, klen, st);
+            break;
+    }
+    if (rc == FDN_OK) progress_add(st, 1000ll * v.n_out);
+    return rc;
+}
+
+int fdn_gauss_rows_typed(const void* d_in, void* d_out, int dtype, int64_t n_rows, int W, const double* kernel, int klen,
+                         int exact, void* stream)
+{
+    int rc;
+    if ((rc = check_dtype(dtype, false))) return rc;
+    if (dtype == FDN_DTYPE_F32)
+        return fdn_gauss_rows(static_cast<const float*>(d_in), static_cast<float*>(d_out), n_rows, W, kernel, klen, exact,
+                              stream);
+    FDN_CHECK_ARG(exact, "typed volumes run the exact no-OF arithmetic only (the fast mode moves truncation boundaries)");
+    FDN_CHECK_ARG(d_in && d_out && kernel && n_rows >= 1 && W >= 1, "bad argument");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    switch (dtype) {
+        case FDN_DTYPE_U8:
+            return launch_gauss_rows_typed(static_cast<const uint8_t*>(d_in), static_cast<uint8_t*>(d_out), n_rows, W, kernel,
+                                           klen, st);
+        case FDN_DTYPE_I8:
+            return launch_gauss_rows_typed(static_cast<const int8_t*>(d_in), static_cast<int8_t*>(d_out), n_rows, W, kernel,
+                                           klen, st);
+        case FDN_DTYPE_U16:
+            return launch_gauss_rows_typed(static_cast<const uint16_t*>(d_in), static_cast<uint16_t*>(d_out), n_rows, W,
+                                           kernel, klen, st);
+        default:
+            return launch_gauss_rows_typed(static_cast<const int16_t*>(d_in), static_cast<int16_t*>(d_out), n_rows, W, kernel,
+                                           klen, st);
+    }
+}
+
+int fdn_transpose_yx_typed(const void* d_in, void* d_out, int dtype, int n, int A, int B, void* stream)
+{
+    int rc;
+    if ((rc = check_dtype(dtype, false))) return rc;
+    FDN_CHECK_ARG(d_in && d_out && n >= 1 && A >= 1 && B >= 1, "bad argument");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    switch (dtype_size(dtype)) {   // a transpose moves bits: one kernel per element size
+        case 1: return launch_transpose(static_cast<const uint8_t*>(d_in), static_cast<uint8_t*>(d_out), n, A, B, st);
+        case 2: return launch_transpose(static_cast<const uint16_t*>(d_in), static_cast<uint16_t*>(d_out), n, A, B, st);
+        default: return launch_transpose(static_cast<const float*>(d_in), static_cast<float*>(d_out), n, A, B, st);
+    }
+}
+
+int fdn_remap_typed(const void* d_src, const float* d_flow, void* d_dst, int dtype, int n, int H, int W, void* stream)
+{
+    int rc;
+    if ((rc = check_dtype(dtype, true))) return rc;
+    FDN_CHECK_ARG(d_src && d_flow && d_dst && n >= 1 && H >= 1 && W >= 1, "bad argument");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    switch (dtype) {
+        case FDN_DTYPE_U8:
+            return launch_remap(static_cast<const uint8_t*>(d_src), d_flow, static_cast<uint8_t*>(d_dst), n, H, W, st);
+        case FDN_DTYPE_U16:
+            return launch_remap(static_cast<const uint16_t*>(d_src), d_flow, static_cast<uint16_t*>(d_dst), n, H, W, st);
+        case FDN_DTYPE_I16:
+            return launch_remap(static_cast<const int16_t*>(d_src), d_flow, static_cast<int16_t*>(d_dst), n, H, W, st);
+        default: {   // float32: the float path's remap (f32(0 + f64(v) * 1) == v)
+            float* dst = static_cast<float*>(d_dst);
+            return launch_warp_acc(static_cast<const float*>(d_src), (int64_t)H * W, W, SlotMap{0, 0}, d_flow, 1.0, dst,
+                                   (int64_t)H * W, W, n, H, W, 1, st);
+        }
+    }
 }
 
 int fdn_gauss_axis(const float* d_in, float* d_out, const fdn_view* view, const double* kernel, int klen, int exact,

@@ -5,6 +5,7 @@
 
 #include <atomic>
 #include <stdio.h>
+#include <type_traits>
 
 #include "fdn_b200.h"
 
@@ -104,8 +105,10 @@ struct SlotMap {
 
 // ---- launchers (each returns an FDN_* status) ----
 // Stage 1
-int launch_blur_rows(const float* in, int64_t in_ss, int64_t in_rs, SlotMap in_map, float* out, int n, int H,
-                     int W, const BlurTaps& bt, cudaStream_t st);
+// T: float, or an integer element type of a typed volume (each value read as float32, like OpenCV's convertTo)
+template <typename T>
+int launch_blur_rows(const T* in, int64_t in_ss, int64_t in_rs, SlotMap in_map, float* out, int n, int H, int W,
+                     const BlurTaps& bt, cudaStream_t st);
 int launch_blur_cols(const float* in, float* out, int n, int H, int W, const BlurTaps& bt, cudaStream_t st);
 int launch_resize_linear_img(const float* in, int n, int H, int W, float* out, int64_t out_stride, int h, int w,
                              cudaStream_t st);
@@ -145,27 +148,79 @@ int launch_warp_acc(const float* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_ma
                     float* acc, int64_t a_ss, int64_t a_rs, int n, int H, int W, int first, cudaStream_t st);
 // One chain step of both directions: images [0, n) (backward neighbours, flows flow[0..n)) are remapped and
 // accumulated into acc with `weight`; images [n, 2n) (forward neighbours, flows flow[n..2n)) are remapped into
-// stash (dense [n][H][W]) for launch_acc_finish.
-int launch_warp_pair(const float* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_map, const float* flow, double weight,
-                     float* acc, int64_t a_ss, int64_t a_rs, float* stash, int n, int H, int W, int first,
-                     cudaStream_t st);
+// stash (dense [n][H][W]) for launch_acc_finish. T: element type of the volume and the stash (integer T: OpenCV's
+// integer remap, the accumulator stays float32).
+template <typename T>
+int launch_warp_pair(const T* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_map, const float* flow, double weight,
+                     float* acc, int64_t a_ss, int64_t a_rs, T* stash, int n, int H, int W, int first, cudaStream_t st);
 // acc = fold over [centre * k[0], stash[0] * k[1], ..., stash[r-1] * k[r]] of f32(f64(acc) + f64(v) * k), in that
-// order; have_acc == 0 starts from 0 (no backward taps).
-int launch_acc_finish(const float* centre, int64_t c_ss, int64_t c_rs, SlotMap c_map, const float* stash, int r,
-                      const double* k, float* acc, int64_t a_ss, int64_t a_rs, int n, int H, int W, int have_acc,
-                      cudaStream_t st);
+// order; have_acc == 0 starts from 0 (no backward taps). float: the result stays in acc (out unused); integer T: the
+// float32 result is truncated into out (the reference's `int_vol[z] = tmp_slice`).
+template <typename T>
+int launch_acc_finish(const T* centre, int64_t c_ss, int64_t c_rs, SlotMap c_map, const T* stash, int r, const double* k,
+                      float* acc, int64_t a_ss, int64_t a_rs, T* out, int64_t o_ss, int64_t o_rs, int n, int H, int W,
+                      int have_acc, cudaStream_t st);
+// cv2.remap of n dense T images (FDN_DTYPE_* other than int8)
+template <typename T>
+int launch_remap(const T* src, const float* flow, T* dst, int n, int H, int W, cudaStream_t st);
 // no-OF
 int launch_gauss_axis(const float* in, float* out, const fdn_view& v, const double* k, int klen, int exact,
                       cudaStream_t st);
 int launch_gauss_rows(const float* in, float* out, int64_t rows, int W, const double* k, int klen, int exact,
                       cudaStream_t st);
-int launch_transpose(const float* in, float* out, int n, int A, int B, cudaStream_t st);
-int launch_transpose_strided(const float* in, int64_t in_sn, int64_t in_sa, float* out, int64_t out_sn, int64_t out_sb,
-                             int n, int A, int B, cudaStream_t st);
+// typed no-OF passes: T in, T out, exact arithmetic only, truncated store
+template <typename T>
+int launch_gauss_axis_typed(const T* in, T* out, const fdn_view& v, const double* k, int klen, cudaStream_t st);
+template <typename T>
+int launch_gauss_rows_typed(const T* in, T* out, int64_t rows, int W, const double* k, int klen, cudaStream_t st);
+template <typename T>
+int launch_transpose(const T* in, T* out, int n, int A, int B, cudaStream_t st);
+template <typename T>
+int launch_transpose_strided(const T* in, int64_t in_sn, int64_t in_sa, T* out, int64_t out_sn, int64_t out_sb, int n,
+                             int A, int B, cudaStream_t st);
 int launch_copy3d(const float* in, int64_t in_sa, int64_t in_sb, int b0, int bw, int c0, int cw, float* out,
                   int64_t out_sa, int64_t out_sb, int A, int B, int C, cudaStream_t st);
 
 #ifdef __CUDACC__
+// ---- typed volumes (FDN_DTYPE_*): element range and the reference's truncating store `int_vol[z] = float32_tmp` ----
+template <typename T> struct TypeRange;
+template <> struct TypeRange<uint8_t> { static constexpr int lo = 0, hi = 255; };
+template <> struct TypeRange<int8_t> { static constexpr int lo = -128, hi = 127; };
+template <> struct TypeRange<uint16_t> { static constexpr int lo = 0, hi = 65535; };
+template <> struct TypeRange<int16_t> { static constexpr int lo = -32768, hi = 32767; };
+// float32 -> T toward zero (NumPy's cast; the accumulated values lie in T's range, the clamp only guards rounding)
+template <typename T>
+__device__ __forceinline__ T store_cast(float a)
+{
+    if constexpr (std::is_same<T, float>::value) return a;
+    else return (T)min(max(__float2int_rz(a), TypeRange<T>::lo), TypeRange<T>::hi);
+}
+// four consecutive elements (one 4-, 8- or 16-byte access; p aligned to 4 * sizeof(T))
+template <typename T> struct __align__(4 * sizeof(T)) Vec4T { T e[4]; };
+template <typename T>
+__device__ __forceinline__ void load4(const T* p, float* d)
+{
+    if constexpr (std::is_same<T, float>::value) {
+        const float4 q = __ldg(reinterpret_cast<const float4*>(p));
+        d[0] = q.x; d[1] = q.y; d[2] = q.z; d[3] = q.w;
+    } else {
+        const Vec4T<T> q = *reinterpret_cast<const Vec4T<T>*>(p);
+#pragma unroll
+        for (int i = 0; i < 4; i++) d[i] = (float)q.e[i];
+    }
+}
+template <typename T>
+__device__ __forceinline__ void store4(T* p, float a, float b, float c, float d)
+{
+    if constexpr (std::is_same<T, float>::value) {
+        *reinterpret_cast<float4*>(p) = make_float4(a, b, c, d);
+    } else {
+        Vec4T<T> q;
+        q.e[0] = store_cast<T>(a); q.e[1] = store_cast<T>(b); q.e[2] = store_cast<T>(c); q.e[3] = store_cast<T>(d);
+        *reinterpret_cast<Vec4T<T>*>(p) = q;
+    }
+}
+
 // ---- shared-memory barrier helpers (mbarrier: waiting threads sleep in hardware instead of polling) ----
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count)

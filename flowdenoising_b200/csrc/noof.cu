@@ -89,11 +89,13 @@ static bool taps_benign(const double* k, int n)
 }
 
 // ------------------------------------------------------------------------------------------------
-// generic fallbacks (any odd kernel length): one thread per output, neighbours re-read through L1 / L2
+// generic fallbacks (any odd kernel length): one thread per output, neighbours re-read through L1 / L2. They also run
+// the typed volumes (T = uint8 / int8 / uint16 / int16, exact mode only): every input is converted to float32 as
+// NumPy does for `int_slice * kernel[i]`, the float32 sum is truncated toward zero into T once, at the store.
 // ------------------------------------------------------------------------------------------------
-template <bool EXACT>
+template <typename T, bool EXACT>
 __global__ void __launch_bounds__(256)
-k_gauss_axis(const float* __restrict__ in, float* __restrict__ out, fdn_view v, Taps64 t64, Taps32 t32)
+k_gauss_axis(const T* __restrict__ in, T* __restrict__ out, fdn_view v, Taps64 t64, Taps32 t32)
 {
     const int x = blockIdx.x * 256 + threadIdx.x;
     const int y = blockIdx.y;
@@ -109,29 +111,29 @@ k_gauss_axis(const float* __restrict__ in, float* __restrict__ out, fdn_view v, 
             j %= v.n_in;
             if (j < 0) j += v.n_in;
         }
-        const float val = in[(int64_t)j * v.in_slice_stride + off];
+        const float val = (float)in[(int64_t)j * v.in_slice_stride + off];
         if (EXACT) acc = (float)__dadd_rn((double)acc, __dmul_rn((double)val, t64.k[i]));
         else acc = fmaf(val, t32.k[i], acc);
     }
-    out[(int64_t)s * v.out_slice_stride + (int64_t)y * v.out_row_stride + x] = acc;
+    out[(int64_t)s * v.out_slice_stride + (int64_t)y * v.out_row_stride + x] = store_cast<T>(acc);
 }
 
 #define GR_TILE 512
-template <bool EXACT>
+template <typename T, bool EXACT>
 __global__ void __launch_bounds__(256)
-k_gauss_rows(const float* __restrict__ in, float* __restrict__ out, int W, Taps64 t64, Taps32 t32)
+k_gauss_rows(const T* __restrict__ in, T* __restrict__ out, int W, Taps64 t64, Taps32 t32)
 {
     extern __shared__ float s_seg[];  // GR_TILE + klen - 1
     const int klen = EXACT ? t64.klen : t32.klen;
     const int r = klen >> 1;
     const int64_t row = blockIdx.y;
     const int x0 = blockIdx.x * GR_TILE;
-    const float* src = in + row * W;
+    const T* src = in + row * W;
     const int nload = min(GR_TILE, W - x0) + 2 * r;
     for (int i = threadIdx.x; i < nload; i += 256) {
         int j = (x0 - r + i) % W;
         if (j < 0) j += W;
-        s_seg[i] = src[j];
+        s_seg[i] = (float)src[j];
     }
     __syncthreads();
     for (int i = threadIdx.x; i < GR_TILE && x0 + i < W; i += 256) {
@@ -141,7 +143,7 @@ k_gauss_rows(const float* __restrict__ in, float* __restrict__ out, int W, Taps6
             if (EXACT) acc = (float)__dadd_rn((double)acc, __dmul_rn((double)val, t64.k[t]));
             else acc = fmaf(val, t32.k[t], acc);
         }
-        out[row * W + x0 + i] = acc;
+        out[row * W + x0 + i] = store_cast<T>(acc);
     }
 }
 
@@ -325,8 +327,8 @@ int launch_gauss_axis(const float* in, float* out, const fdn_view& v, const doub
     for (int i = 0; i < klen; i++) { t64.k[i] = k[i]; t32.k[i] = (float)k[i]; }
     dim3 grid((unsigned)cdiv(v.W, 256), (unsigned)v.H, (unsigned)v.n_out);
     ProfScope ps(K_GAUSS_AXIS, 8.0 * v.n_out * v.H * v.W, st);
-    if (exact) k_gauss_axis<true><<<grid, 256, 0, st>>>(in, out, v, t64, t32);
-    else k_gauss_axis<false><<<grid, 256, 0, st>>>(in, out, v, t64, t32);
+    if (exact) k_gauss_axis<float, true><<<grid, 256, 0, st>>>(in, out, v, t64, t32);
+    else k_gauss_axis<float, false><<<grid, 256, 0, st>>>(in, out, v, t64, t32);
     FDN_LAUNCHED("k_gauss_axis");
     return FDN_OK;
 }
@@ -470,11 +472,59 @@ int launch_gauss_rows(const float* in, float* out, int64_t rows, int W, const do
         const int64_t nr = rows - r0 < 65535 ? rows - r0 : 65535;
         dim3 grid((unsigned)cdiv(W, GR_TILE), (unsigned)nr);
         ProfScope ps(K_GAUSS_ROWS, 8.0 * nr * W, st);
-        if (exact) k_gauss_rows<true><<<grid, 256, smem, st>>>(in + r0 * W, out + r0 * W, W, t64, t32);
-        else k_gauss_rows<false><<<grid, 256, smem, st>>>(in + r0 * W, out + r0 * W, W, t64, t32);
+        if (exact) k_gauss_rows<float, true><<<grid, 256, smem, st>>>(in + r0 * W, out + r0 * W, W, t64, t32);
+        else k_gauss_rows<float, false><<<grid, 256, smem, st>>>(in + r0 * W, out + r0 * W, W, t64, t32);
         FDN_LAUNCHED("k_gauss_rows");
     }
     return FDN_OK;
 }
+
+// ------------------------------------------------------------------------------------------------
+// typed volumes: the generic kernels in exact mode (the fast FMA mode would move the truncation boundaries)
+// ------------------------------------------------------------------------------------------------
+template <typename T>
+int launch_gauss_axis_typed(const T* in, T* out, const fdn_view& v, const double* k, int klen, cudaStream_t st)
+{
+    FDN_CHECK_ARG(klen >= 1 && klen <= FDN_MAX_KLEN && (klen & 1), "kernel length %d unsupported (odd, <= %d)", klen,
+                  FDN_MAX_KLEN);
+    FDN_CHECK_ARG(v.H <= 65535 && v.n_out <= 65535, "view too large for one launch");
+    Taps64 t64;
+    Taps32 t32;
+    t64.klen = t32.klen = klen;
+    for (int i = 0; i < klen; i++) { t64.k[i] = k[i]; t32.k[i] = (float)k[i]; }
+    dim3 grid((unsigned)cdiv(v.W, 256), (unsigned)v.H, (unsigned)v.n_out);
+    ProfScope ps(K_GAUSS_AXIS, 2.0 * sizeof(T) * v.n_out * v.H * v.W, st);
+    k_gauss_axis<T, true><<<grid, 256, 0, st>>>(in, out, v, t64, t32);
+    FDN_LAUNCHED("k_gauss_axis");
+    return FDN_OK;
+}
+
+template <typename T>
+int launch_gauss_rows_typed(const T* in, T* out, int64_t rows, int W, const double* k, int klen, cudaStream_t st)
+{
+    FDN_CHECK_ARG(klen >= 1 && klen <= FDN_MAX_KLEN && (klen & 1), "kernel length %d unsupported (odd, <= %d)", klen,
+                  FDN_MAX_KLEN);
+    Taps64 t64;
+    Taps32 t32;
+    t64.klen = t32.klen = klen;
+    for (int i = 0; i < klen; i++) { t64.k[i] = k[i]; t32.k[i] = (float)k[i]; }
+    const size_t smem = sizeof(float) * (GR_TILE + klen - 1);
+    for (int64_t r0 = 0; r0 < rows; r0 += 65535) {
+        const int64_t nr = rows - r0 < 65535 ? rows - r0 : 65535;
+        dim3 grid((unsigned)cdiv(W, GR_TILE), (unsigned)nr);
+        ProfScope ps(K_GAUSS_ROWS, 2.0 * sizeof(T) * nr * W, st);
+        k_gauss_rows<T, true><<<grid, 256, smem, st>>>(in + r0 * W, out + r0 * W, W, t64, t32);
+        FDN_LAUNCHED("k_gauss_rows");
+    }
+    return FDN_OK;
+}
+
+#define FDN_INST_NOOF(T)                                                                                              \
+    template int launch_gauss_axis_typed<T>(const T*, T*, const fdn_view&, const double*, int, cudaStream_t);         \
+    template int launch_gauss_rows_typed<T>(const T*, T*, int64_t, int, const double*, int, cudaStream_t);
+FDN_INST_NOOF(uint8_t)
+FDN_INST_NOOF(int8_t)
+FDN_INST_NOOF(uint16_t)
+FDN_INST_NOOF(int16_t)
 
 }  // namespace fdn

@@ -122,36 +122,40 @@ __device__ __forceinline__ int reflect101(int p, int len)
     return p;
 }
 
-// One thread per output pixel; the taps of neighbouring threads overlap in L1.
+// One thread per output pixel; the taps of neighbouring threads overlap in L1. The input is float32 or the integer
+// element type of a typed volume: calcOpticalFlowFarneback converts its images with convertTo(CV_32F) before this
+// blur, so every value is read and converted here and no float32 copy of the volume exists.
+template <typename T>
 __global__ void __launch_bounds__(128)
-k_blur_rows(const float* __restrict__ in, int64_t in_ss, int64_t in_rs, SlotMap in_map, float* __restrict__ out,
-            int H, int W, BlurTaps bt)
+k_blur_rows(const T* __restrict__ in_, int64_t in_ss, int64_t in_rs, SlotMap in_map, float* __restrict__ out, int H,
+            int W, BlurTaps bt)
 {
     const int x = blockIdx.x * 128 + threadIdx.x;
     const int y = blockIdx.y;
     const int b = blockIdx.z;
     if (x >= W) return;
-    const float* s = in + (int64_t)in_map.slot(b) * in_ss + (int64_t)y * in_rs;
+    const T* s_ = in_ + (int64_t)in_map.slot(b) * in_ss + (int64_t)y * in_rs;
+    auto s = [&](int i) { return (float)s_[i]; };
     const int ksz = bt.ksz, r = ksz >> 1;
     float acc;
     if (ksz == 3) {
         // SymmRowSmallVec_32f: fma(centre, k1, (l + r) * k0); a last odd column is OpenCV's scalar tail
-        float lr = __fadd_rn(s[reflect101(x - 1, W)], s[reflect101(x + 1, W)]);
-        acc = x < (W & ~1) ? fmaf(s[x], bt.k[1], __fmul_rn(lr, bt.k[0])) : fmaf(lr, bt.k[0], __fmul_rn(s[x], bt.k[1]));
+        float lr = __fadd_rn(s(reflect101(x - 1, W)), s(reflect101(x + 1, W)));
+        acc = x < (W & ~1) ? fmaf(s(x), bt.k[1], __fmul_rn(lr, bt.k[0])) : fmaf(lr, bt.k[0], __fmul_rn(s(x), bt.k[1]));
     } else if (x >= r && x + r < W) {
-        const float* p = s + (x - r);
-        acc = __fmul_rn(p[0], bt.k[0]);
+        const int p0 = x - r;
+        acc = __fmul_rn(s(p0), bt.k[0]);
         if (x < (W & ~3)) {
-            for (int i = 1; i < ksz; i++) acc = fmaf(p[i], bt.k[i], acc);
+            for (int i = 1; i < ksz; i++) acc = fmaf(s(p0 + i), bt.k[i], acc);
         } else {
-            for (int i = 1; i < ksz; i++) acc = __fadd_rn(acc, __fmul_rn(p[i], bt.k[i]));
+            for (int i = 1; i < ksz; i++) acc = __fadd_rn(acc, __fmul_rn(s(p0 + i), bt.k[i]));
         }
     } else {
-        acc = __fmul_rn(s[reflect101(x - r, W)], bt.k[0]);
+        acc = __fmul_rn(s(reflect101(x - r, W)), bt.k[0]);
         if (x < (W & ~3)) {
-            for (int i = 1; i < ksz; i++) acc = fmaf(s[reflect101(x - r + i, W)], bt.k[i], acc);
+            for (int i = 1; i < ksz; i++) acc = fmaf(s(reflect101(x - r + i, W)), bt.k[i], acc);
         } else {
-            for (int i = 1; i < ksz; i++) acc = __fadd_rn(acc, __fmul_rn(s[reflect101(x - r + i, W)], bt.k[i]));
+            for (int i = 1; i < ksz; i++) acc = __fadd_rn(acc, __fmul_rn(s(reflect101(x - r + i, W)), bt.k[i]));
         }
     }
     out[((int64_t)b * H + y) * W + x] = acc;
@@ -181,9 +185,9 @@ k_blur_cols(const float* __restrict__ in, float* __restrict__ out, int H, int W,
 // with sigma_k = (2^k - 1) / 2 -> 3, 3, 9, 19, 39, 79 taps for levels 0..5 (half widths 1, 4, 9, 19, 39; SURVEY.md
 // App. A.0). Same arithmetic per output as k_blur_rows / k_blur_cols; each thread produces 4 outputs from one window of
 // 4 + 2R inputs instead of 4 * (2R + 1) loads with their address arithmetic.
-template <int R>
+template <typename T, int R>
 __global__ void __launch_bounds__(128)
-k_blur_rows4(const float* __restrict__ in, int64_t in_ss, int64_t in_rs, SlotMap in_map, float* __restrict__ out, int H,
+k_blur_rows4(const T* __restrict__ in, int64_t in_ss, int64_t in_rs, SlotMap in_map, float* __restrict__ out, int H,
              int W, BlurTaps bt)
 {
     constexpr int KS = 2 * R + 1;
@@ -191,14 +195,14 @@ k_blur_rows4(const float* __restrict__ in, int64_t in_ss, int64_t in_rs, SlotMap
     const int y = blockIdx.y;
     const int b = blockIdx.z;
     if (x0 >= W) return;
-    const float* s = in + (int64_t)in_map.slot(b) * in_ss + (int64_t)y * in_rs;
+    const T* s = in + (int64_t)in_map.slot(b) * in_ss + (int64_t)y * in_rs;
     float v[4 + 2 * R];
     if (x0 >= R && x0 + 3 + R < W) {
 #pragma unroll
-        for (int i = 0; i < 4 + 2 * R; i++) v[i] = __ldg(s + x0 - R + i);
+        for (int i = 0; i < 4 + 2 * R; i++) v[i] = (float)__ldg(s + x0 - R + i);
     } else {
 #pragma unroll
-        for (int i = 0; i < 4 + 2 * R; i++) v[i] = __ldg(s + reflect101(x0 - R + i, W));
+        for (int i = 0; i < 4 + 2 * R; i++) v[i] = (float)__ldg(s + reflect101(x0 - R + i, W));
     }
     float o[4];
 #pragma unroll
@@ -252,8 +256,9 @@ k_blur_cols4(const float* __restrict__ in, float* __restrict__ out, int H, int W
     }
 }
 
-int launch_blur_rows(const float* in, int64_t in_ss, int64_t in_rs, SlotMap in_map, float* out, int n, int H,
-                     int W, const BlurTaps& bt, cudaStream_t st)
+template <typename T>
+int launch_blur_rows(const T* in, int64_t in_ss, int64_t in_rs, SlotMap in_map, float* out, int n, int H, int W,
+                     const BlurTaps& bt, cudaStream_t st)
 {
     const bool win4 = (bt.ksz == 3 || bt.ksz == 9 || bt.ksz == 19 || bt.ksz == 39 || bt.ksz == 79) && W % 4 == 0 &&
                       W >= 4 + bt.ksz && (reinterpret_cast<uintptr_t>(out) & 15) == 0 && H <= 65535;
@@ -261,24 +266,33 @@ int launch_blur_rows(const float* in, int64_t in_ss, int64_t in_rs, SlotMap in_m
         int nb = n - b0 < 65535 ? n - b0 : 65535;
         SlotMap m = in_map;
         m.base += b0;
-        ProfScope ps(K_BLUR_ROWS, 8.0 * nb * H * W, st);
+        ProfScope ps(K_BLUR_ROWS, (4.0 + sizeof(T)) * nb * H * W, st);
         if (win4) {
             dim3 grid((unsigned)cdiv(W, 512), (unsigned)H, (unsigned)nb);
             float* o = out + (int64_t)b0 * H * W;
-            if (bt.ksz == 3) k_blur_rows4<1><<<grid, 128, 0, st>>>(in, in_ss, in_rs, m, o, H, W, bt);
-            else if (bt.ksz == 9) k_blur_rows4<4><<<grid, 128, 0, st>>>(in, in_ss, in_rs, m, o, H, W, bt);
-            else if (bt.ksz == 19) k_blur_rows4<9><<<grid, 128, 0, st>>>(in, in_ss, in_rs, m, o, H, W, bt);
-            else if (bt.ksz == 39) k_blur_rows4<19><<<grid, 128, 0, st>>>(in, in_ss, in_rs, m, o, H, W, bt);
-            else k_blur_rows4<39><<<grid, 128, 0, st>>>(in, in_ss, in_rs, m, o, H, W, bt);
+            if (bt.ksz == 3) k_blur_rows4<T, 1><<<grid, 128, 0, st>>>(in, in_ss, in_rs, m, o, H, W, bt);
+            else if (bt.ksz == 9) k_blur_rows4<T, 4><<<grid, 128, 0, st>>>(in, in_ss, in_rs, m, o, H, W, bt);
+            else if (bt.ksz == 19) k_blur_rows4<T, 9><<<grid, 128, 0, st>>>(in, in_ss, in_rs, m, o, H, W, bt);
+            else if (bt.ksz == 39) k_blur_rows4<T, 19><<<grid, 128, 0, st>>>(in, in_ss, in_rs, m, o, H, W, bt);
+            else k_blur_rows4<T, 39><<<grid, 128, 0, st>>>(in, in_ss, in_rs, m, o, H, W, bt);
             FDN_LAUNCHED("k_blur_rows4");
             continue;
         }
         dim3 grid((unsigned)cdiv(W, 128), (unsigned)H, (unsigned)nb);
-        k_blur_rows<<<grid, 128, 0, st>>>(in, in_ss, in_rs, m, out + (int64_t)b0 * H * W, H, W, bt);
+        k_blur_rows<T><<<grid, 128, 0, st>>>(in, in_ss, in_rs, m, out + (int64_t)b0 * H * W, H, W, bt);
         FDN_LAUNCHED("k_blur_rows");
     }
     return FDN_OK;
 }
+
+template int launch_blur_rows<float>(const float*, int64_t, int64_t, SlotMap, float*, int, int, int, const BlurTaps&,
+                                     cudaStream_t);
+template int launch_blur_rows<uint8_t>(const uint8_t*, int64_t, int64_t, SlotMap, float*, int, int, int, const BlurTaps&,
+                                       cudaStream_t);
+template int launch_blur_rows<uint16_t>(const uint16_t*, int64_t, int64_t, SlotMap, float*, int, int, int,
+                                        const BlurTaps&, cudaStream_t);
+template int launch_blur_rows<int16_t>(const int16_t*, int64_t, int64_t, SlotMap, float*, int, int, int, const BlurTaps&,
+                                       cudaStream_t);
 
 int launch_blur_cols(const float* in, float* out, int n, int H, int W, const BlurTaps& bt, cudaStream_t st)
 {

@@ -56,8 +56,18 @@ k_warp_acc(const float* __restrict__ neigh, int64_t n_ss, int64_t n_rs, SlotMap 
 
 // Four consecutive pixels per thread (128-bit flow / accumulator accesses, four independent gathers in flight).
 // Same arithmetic as k_warp_acc. Needs W % 4 == 0 and 16-byte aligned rows.
-__device__ __forceinline__ float remap_px(const float* __restrict__ src, int64_t n_rs, float fx, float fy, int x, int y,
-                                          int H, int W)
+//
+// remap_px<T> is cv2.remap of a T image with the same quantised map (SURVEY App. B Q3), returned as a float:
+//   float      the float path above;
+//   uint8      OpenCV's fixed point: weights rint(wy * wx * 2^15) of the 1/32-px table, (sum + 2^14) >> 15, saturated.
+//              wy, wx are multiples of 1/32, so every entry is the exact integer (32 - ay or ay) * (32 - ax or ax) * 32:
+//              it is computed in registers instead of read from a table (no per-lane divergent lookups). The one entry
+//              OpenCV saturates to 32767 (ax = ay = 0) gives the same result for every 8-bit value;
+//              tests/test_integer_volume_oracle.py pins all 1024 entries against cv2.
+//   16U / 16S  the float32 weights and tap order of the float path, then rint and saturate (Cast<float, T>).
+template <typename T>
+__device__ __forceinline__ float remap_px(const T* __restrict__ src, int64_t n_rs, float fx, float fy, int x, int y, int H,
+                                          int W)
 {
     const float mx = __fadd_rn(fx, (float)x), my = __fadd_rn(fy, (float)y);
     const int sx = __float2int_rn(__fmul_rn(mx, 32.f)), sy = __float2int_rn(__fmul_rn(my, 32.f));
@@ -65,15 +75,26 @@ __device__ __forceinline__ float remap_px(const float* __restrict__ src, int64_t
     int ix = sx >> 5, iy = sy >> 5;
     ix = min(max(ix, -32768), 32767);
     iy = min(max(iy, -32768), 32767);
-    const float tx1 = __fmul_rn((float)ax, 0.03125f), tx0 = __fsub_rn(1.f, tx1);
-    const float ty1 = __fmul_rn((float)ay, 0.03125f), ty0 = __fsub_rn(1.f, ty1);
-    const float w0 = __fmul_rn(ty0, tx0), w1 = __fmul_rn(ty0, tx1), w2 = __fmul_rn(ty1, tx0), w3 = __fmul_rn(ty1, tx1);
     const int x0 = min(max(ix, 0), W - 1), x1 = min(max(ix + 1, 0), W - 1);
     const int y0 = min(max(iy, 0), H - 1), y1 = min(max(iy + 1, 0), H - 1);
-    const float* r0 = src + (int64_t)y0 * n_rs;
-    const float* r1 = src + (int64_t)y1 * n_rs;
-    const float v0 = __ldg(r0 + x0), v1 = __ldg(r0 + x1), v2 = __ldg(r1 + x0), v3 = __ldg(r1 + x1);
-    return __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(v0, w0), __fmul_rn(v1, w1)), __fmul_rn(v2, w2)), __fmul_rn(v3, w3));
+    const T* r0 = src + (int64_t)y0 * n_rs;
+    const T* r1 = src + (int64_t)y1 * n_rs;
+    if constexpr (std::is_same<T, uint8_t>::value) {
+        const int v0 = __ldg(r0 + x0), v1 = __ldg(r0 + x1), v2 = __ldg(r1 + x0), v3 = __ldg(r1 + x1);
+        const int s = v0 * (((32 - ay) * (32 - ax)) << 5) + v1 * (((32 - ay) * ax) << 5) + v2 * ((ay * (32 - ax)) << 5) +
+                      v3 * ((ay * ax) << 5);
+        return (float)min(max((s + (1 << 14)) >> 15, 0), 255);
+    } else {
+        const float tx1 = __fmul_rn((float)ax, 0.03125f), tx0 = __fsub_rn(1.f, tx1);
+        const float ty1 = __fmul_rn((float)ay, 0.03125f), ty0 = __fsub_rn(1.f, ty1);
+        const float w0 = __fmul_rn(ty0, tx0), w1 = __fmul_rn(ty0, tx1), w2 = __fmul_rn(ty1, tx0), w3 = __fmul_rn(ty1, tx1);
+        const float v0 = (float)__ldg(r0 + x0), v1 = (float)__ldg(r0 + x1), v2 = (float)__ldg(r1 + x0),
+                    v3 = (float)__ldg(r1 + x1);
+        const float s =
+            __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(v0, w0), __fmul_rn(v1, w1)), __fmul_rn(v2, w2)), __fmul_rn(v3, w3));
+        if constexpr (std::is_same<T, float>::value) return s;
+        else return (float)min(max(__float2int_rn(s), (int)TypeRange<T>::lo), (int)TypeRange<T>::hi);
+    }
 }
 
 __global__ void __launch_bounds__(128)
@@ -150,18 +171,20 @@ int launch_warp_acc(const float* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_ma
 // images [0, n) are the backward neighbours -- remapped and accumulated in place, the reference's order -- and images
 // [n, 2n) the forward neighbours, whose remapped values wait in `stash` until the backward chain and the centre tap
 // are in the accumulator (k_acc_finish applies them in the reference's order: centre, +1, ..., +r).
+// T is the element type of the volume and of the stash (a remapped integer image is an integer image); the
+// accumulator is float32 for every T.
 // ------------------------------------------------------------------------------------------------
-template <int VEC>
+template <typename T, int VEC>
 __global__ void __launch_bounds__(128)
-k_warp_pair(const float* __restrict__ neigh, int64_t n_ss, int64_t n_rs, SlotMap n_map, const float* __restrict__ flow,
-            double weight, float* __restrict__ acc, int64_t a_ss, int64_t a_rs, float* __restrict__ stash, int n, int b0,
+k_warp_pair(const T* __restrict__ neigh, int64_t n_ss, int64_t n_rs, SlotMap n_map, const float* __restrict__ flow,
+            double weight, float* __restrict__ acc, int64_t a_ss, int64_t a_rs, T* __restrict__ stash, int n, int b0,
             int H, int W, int first)
 {
     const int x = (blockIdx.x * 128 + threadIdx.x) * VEC;
     const int y = blockIdx.y;
     const int b = b0 + blockIdx.z;   // 0 .. 2n-1
     if (x >= W) return;
-    const float* src = neigh + (int64_t)n_map.slot(b) * n_ss;
+    const T* src = neigh + (int64_t)n_map.slot(b) * n_ss;
     const int64_t fpx = ((int64_t)b * H + y) * W + x;
     float v[VEC];
     if (VEC == 4) {
@@ -190,32 +213,34 @@ k_warp_pair(const float* __restrict__ neigh, int64_t n_ss, int64_t n_rs, SlotMap
             *ap = (float)__dadd_rn(first ? 0.0 : (double)*ap, __dmul_rn((double)v[0], weight));
         }
     } else {
-        float* sp = stash + ((int64_t)(b - n) * H + y) * W + x;
-        if (VEC == 4) *reinterpret_cast<float4*>(sp) = make_float4(v[0], v[1 % VEC], v[2 % VEC], v[3 % VEC]);
-        else *sp = v[0];
+        T* sp = stash + ((int64_t)(b - n) * H + y) * W + x;
+        if (VEC == 4) store4(sp, v[0], v[1 % VEC], v[2 % VEC], v[3 % VEC]);
+        else *sp = store_cast<T>(v[0]);
     }
 }
 
-int launch_warp_pair(const float* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_map, const float* flow, double weight,
-                     float* acc, int64_t a_ss, int64_t a_rs, float* stash, int n, int H, int W, int first,
-                     cudaStream_t st)
+template <typename T>
+int launch_warp_pair(const T* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_map, const float* flow, double weight,
+                     float* acc, int64_t a_ss, int64_t a_rs, T* stash, int n, int H, int W, int first, cudaStream_t st)
 {
     const bool vec4 = W % 4 == 0 && n_ss % 4 == 0 && n_rs % 4 == 0 && a_ss % 4 == 0 && a_rs % 4 == 0 &&
                       (reinterpret_cast<uintptr_t>(neigh) & 15) == 0 && (reinterpret_cast<uintptr_t>(acc) & 15) == 0 &&
-                      (reinterpret_cast<uintptr_t>(flow) & 15) == 0 && (reinterpret_cast<uintptr_t>(stash) & 15) == 0;
+                      (reinterpret_cast<uintptr_t>(flow) & 15) == 0 &&
+                      (reinterpret_cast<uintptr_t>(stash) & (4 * sizeof(T) - 1)) == 0;
     FDN_CHECK_ARG(H <= 65535, "image too tall for one launch");
+    const double es = (double)sizeof(T);
     for (int b0 = 0; b0 < 2 * n; b0 += 65535) {
         const int nb = 2 * n - b0 < 65535 ? 2 * n - b0 : 65535;
-        // remap: flow 8 + neighbour 4; backward half: accumulator 4 (+4 unless first), forward half: stash 4
-        ProfScope ps(K_WARP_ACC, (double)nb * H * W * (12.0 + (first ? 4.0 : 6.0)), st);
+        // remap: flow 8 + neighbour; backward half: float32 accumulator 4 (+4 unless first), forward half: stash
+        ProfScope ps(K_WARP_ACC, (double)nb * H * W * (8.0 + es + (first ? 4.0 + es : 8.0 + es) / 2), st);
         if (vec4) {
             dim3 grid((unsigned)cdiv(W, 512), (unsigned)H, (unsigned)nb);
-            k_warp_pair<4><<<grid, 128, 0, st>>>(neigh, n_ss, n_rs, n_map, flow, weight, acc, a_ss, a_rs, stash, n, b0, H, W,
-                                                 first);
+            k_warp_pair<T, 4><<<grid, 128, 0, st>>>(neigh, n_ss, n_rs, n_map, flow, weight, acc, a_ss, a_rs, stash, n, b0, H,
+                                                    W, first);
         } else {
             dim3 grid((unsigned)cdiv(W, 128), (unsigned)H, (unsigned)nb);
-            k_warp_pair<1><<<grid, 128, 0, st>>>(neigh, n_ss, n_rs, n_map, flow, weight, acc, a_ss, a_rs, stash, n, b0, H, W,
-                                                 first);
+            k_warp_pair<T, 1><<<grid, 128, 0, st>>>(neigh, n_ss, n_rs, n_map, flow, weight, acc, a_ss, a_rs, stash, n, b0, H,
+                                                    W, first);
         }
         FDN_LAUNCHED("k_warp_pair");
     }
@@ -227,26 +252,27 @@ struct FinishTaps {
     double k[FDN_MAX_R + 1];   // centre, +1, ..., +r
 };
 
-template <int VEC>
+template <typename T, int VEC>
 __global__ void __launch_bounds__(128)
-k_acc_finish(const float* __restrict__ centre, int64_t c_ss, int64_t c_rs, SlotMap c_map, const float* __restrict__ stash,
-             int64_t stash_stride, int r, FinishTaps taps, float* __restrict__ acc, int64_t a_ss, int64_t a_rs, int b0,
-             int H, int W, int have_acc)
+k_acc_finish(const T* __restrict__ centre, int64_t c_ss, int64_t c_rs, SlotMap c_map, const T* __restrict__ stash,
+             int64_t stash_stride, int r, FinishTaps taps, float* __restrict__ acc, int64_t a_ss, int64_t a_rs,
+             T* __restrict__ out, int64_t o_ss, int64_t o_rs, int b0, int H, int W, int have_acc)
 {
     const int x = (blockIdx.x * 128 + threadIdx.x) * VEC;
     const int y = blockIdx.y;
     const int b = b0 + blockIdx.z;
     if (x >= W) return;
-    const float* cp = centre + (int64_t)c_map.slot(b) * c_ss + (int64_t)y * c_rs + x;
+    const T* cp = centre + (int64_t)c_map.slot(b) * c_ss + (int64_t)y * c_rs + x;
     float* ap = acc + (int64_t)b * a_ss + (int64_t)y * a_rs + x;
-    const float* sp = stash + ((int64_t)b * H + y) * W + x;
+    const T* sp = stash + ((int64_t)b * H + y) * W + x;
     float a[VEC], v[VEC];
-    auto load = [&](const float* p, float* dst) {
+    auto load = [&](const T* p, float* dst) {
         if (VEC == 4) {
-            const float4 q = __ldg(reinterpret_cast<const float4*>(p));
-            dst[0] = q.x; dst[1 % VEC] = q.y; dst[2 % VEC] = q.z; dst[3 % VEC] = q.w;
+            float q[4];
+            load4(p, q);
+            dst[0] = q[0]; dst[1 % VEC] = q[1]; dst[2 % VEC] = q[2]; dst[3 % VEC] = q[3];
         } else {
-            dst[0] = __ldg(p);
+            dst[0] = (float)__ldg(p);
         }
     };
 #pragma unroll
@@ -267,36 +293,73 @@ k_acc_finish(const float* __restrict__ centre, int64_t c_ss, int64_t c_rs, SlotM
 #pragma unroll
         for (int i = 0; i < VEC; i++) a[i] = (float)__dadd_rn((double)a[i], __dmul_rn((double)v[i], taps.k[d + 1]));
     }
-    if (VEC == 4) *reinterpret_cast<float4*>(ap) = make_float4(a[0], a[1 % VEC], a[2 % VEC], a[3 % VEC]);
-    else *ap = a[0];
+    if constexpr (std::is_same<T, float>::value) {
+        if (VEC == 4) *reinterpret_cast<float4*>(ap) = make_float4(a[0], a[1 % VEC], a[2 % VEC], a[3 % VEC]);
+        else *ap = a[0];
+    } else {   // filtered_vol[z] = tmp_slice (:325): truncation toward zero
+        T* op = out + (int64_t)b * o_ss + (int64_t)y * o_rs + x;
+        if (VEC == 4) store4(op, a[0], a[1 % VEC], a[2 % VEC], a[3 % VEC]);
+        else *op = store_cast<T>(a[0]);
+    }
 }
 
-int launch_acc_finish(const float* centre, int64_t c_ss, int64_t c_rs, SlotMap c_map, const float* stash, int r,
-                      const double* k, float* acc, int64_t a_ss, int64_t a_rs, int n, int H, int W, int have_acc,
-                      cudaStream_t st)
+template <typename T>
+int launch_acc_finish(const T* centre, int64_t c_ss, int64_t c_rs, SlotMap c_map, const T* stash, int r, const double* k,
+                      float* acc, int64_t a_ss, int64_t a_rs, T* out, int64_t o_ss, int64_t o_rs, int n, int H, int W,
+                      int have_acc, cudaStream_t st)
 {
     FDN_CHECK_ARG(r >= 0 && r <= FDN_MAX_R, "kernel radius %d unsupported (<= %d)", r, FDN_MAX_R);
     FDN_CHECK_ARG(H <= 65535, "image too tall for one launch");
+    constexpr bool typed = !std::is_same<T, float>::value;
+    constexpr uintptr_t al = 4 * sizeof(T) - 1;
     FinishTaps taps;
     for (int i = 0; i <= r; i++) taps.k[i] = k[i];
-    const bool vec4 = W % 4 == 0 && c_ss % 4 == 0 && c_rs % 4 == 0 && a_ss % 4 == 0 && a_rs % 4 == 0 &&
-                      (reinterpret_cast<uintptr_t>(centre) & 15) == 0 && (reinterpret_cast<uintptr_t>(acc) & 15) == 0 &&
-                      (reinterpret_cast<uintptr_t>(stash) & 15) == 0;
+    bool vec4 = W % 4 == 0 && c_ss % 4 == 0 && c_rs % 4 == 0 && a_ss % 4 == 0 && a_rs % 4 == 0 &&
+                (reinterpret_cast<uintptr_t>(centre) & al) == 0 && (reinterpret_cast<uintptr_t>(acc) & 15) == 0 &&
+                (reinterpret_cast<uintptr_t>(stash) & al) == 0;
+    if (typed) vec4 = vec4 && o_ss % 4 == 0 && o_rs % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & al) == 0;
     const int64_t stash_stride = (int64_t)n * H * W;
+    const double es = (double)sizeof(T);
     for (int b0 = 0; b0 < n; b0 += 65535) {
         const int nb = n - b0 < 65535 ? n - b0 : 65535;
-        ProfScope ps(K_WARP_ACC, (double)nb * H * W * (4.0 * (r + 2) + (have_acc ? 4.0 : 0.0)), st);
+        // centre + r stash images + the result (in T), the float32 accumulator read when there are backward taps
+        ProfScope ps(K_WARP_ACC, (double)nb * H * W * (es * (r + 2) + (have_acc ? 4.0 : 0.0)), st);
         if (vec4) {
             dim3 grid((unsigned)cdiv(W, 512), (unsigned)H, (unsigned)nb);
-            k_acc_finish<4><<<grid, 128, 0, st>>>(centre, c_ss, c_rs, c_map, stash, stash_stride, r, taps, acc, a_ss, a_rs, b0,
-                                                  H, W, have_acc);
+            k_acc_finish<T, 4><<<grid, 128, 0, st>>>(centre, c_ss, c_rs, c_map, stash, stash_stride, r, taps, acc, a_ss, a_rs,
+                                                     out, o_ss, o_rs, b0, H, W, have_acc);
         } else {
             dim3 grid((unsigned)cdiv(W, 128), (unsigned)H, (unsigned)nb);
-            k_acc_finish<1><<<grid, 128, 0, st>>>(centre, c_ss, c_rs, c_map, stash, stash_stride, r, taps, acc, a_ss, a_rs, b0,
-                                                  H, W, have_acc);
+            k_acc_finish<T, 1><<<grid, 128, 0, st>>>(centre, c_ss, c_rs, c_map, stash, stash_stride, r, taps, acc, a_ss, a_rs,
+                                                     out, o_ss, o_rs, b0, H, W, have_acc);
         }
         FDN_LAUNCHED("k_acc_finish");
     }
+    return FDN_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// cv2.remap of dense T images alone (stage entry point fdn_remap_typed: pins the integer remap)
+// ------------------------------------------------------------------------------------------------
+template <typename T>
+__global__ void __launch_bounds__(128)
+k_remap(const T* __restrict__ src, const float2* __restrict__ flow, T* __restrict__ dst, int H, int W)
+{
+    const int x = blockIdx.x * 128 + threadIdx.x;
+    const int y = blockIdx.y;
+    const int64_t b = blockIdx.z;
+    if (x >= W) return;
+    const float2 f = flow[(b * H + y) * W + x];
+    dst[(b * H + y) * W + x] = store_cast<T>(remap_px(src + b * H * W, W, f.x, f.y, x, y, H, W));
+}
+
+template <typename T>
+int launch_remap(const T* src, const float* flow, T* dst, int n, int H, int W, cudaStream_t st)
+{
+    FDN_CHECK_ARG(H <= 65535 && n <= 65535, "batch or image too large for one launch");
+    dim3 grid((unsigned)cdiv(W, 128), (unsigned)H, (unsigned)n);
+    k_remap<T><<<grid, 128, 0, st>>>(src, reinterpret_cast<const float2*>(flow), dst, H, W);
+    FDN_LAUNCHED("k_remap");
     return FDN_OK;
 }
 
@@ -306,16 +369,17 @@ int launch_acc_finish(const float* centre, int64_t c_ss, int64_t c_rs, SlotMap c
 // Dense case ([n][A][B] -> [n][B][A]): in_sn = out_sn = A*B, in_sa = B, out_sb = A. The strided form is the
 // transposing unpack of the multi-GPU re-slab (flowdenoising_b200/dist.py).
 // ------------------------------------------------------------------------------------------------
+template <typename T>
 __global__ void __launch_bounds__(256)
-k_transpose(const float* __restrict__ in, int64_t in_sn, int64_t in_sa, float* __restrict__ out, int64_t out_sn,
-            int64_t out_sb, int A, int B)
+k_transpose(const T* __restrict__ in, int64_t in_sn, int64_t in_sa, T* __restrict__ out, int64_t out_sn, int64_t out_sb,
+            int A, int B)
 {
-    __shared__ float tile[32][33];
+    __shared__ T tile[32][33];
     const int64_t img = blockIdx.z;
     const int b0 = blockIdx.x * 32, a0 = blockIdx.y * 32;
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;  // 32 x 8
-    const float* src = in + img * in_sn;
-    float* dst = out + img * out_sn;
+    const T* src = in + img * in_sn;
+    T* dst = out + img * out_sn;
     for (int i = ty; i < 32; i += 8) {
         int a = a0 + i, b = b0 + tx;
         if (a < A && b < B) tile[i][tx] = src[(int64_t)a * in_sa + b];
@@ -327,22 +391,24 @@ k_transpose(const float* __restrict__ in, int64_t in_sn, int64_t in_sa, float* _
     }
 }
 
-int launch_transpose_strided(const float* in, int64_t in_sn, int64_t in_sa, float* out, int64_t out_sn, int64_t out_sb,
-                             int n, int A, int B, cudaStream_t st)
+template <typename T>
+int launch_transpose_strided(const T* in, int64_t in_sn, int64_t in_sa, T* out, int64_t out_sn, int64_t out_sb, int n,
+                             int A, int B, cudaStream_t st)
 {
     FDN_CHECK_ARG(cdiv(A, 32) <= 65535, "transpose: A too large");
     for (int b0 = 0; b0 < n; b0 += 65535) {
         const int nb = n - b0 < 65535 ? n - b0 : 65535;
         dim3 grid((unsigned)cdiv(B, 32), (unsigned)cdiv(A, 32), (unsigned)nb);
-        ProfScope ps(K_TRANSPOSE, 8.0 * nb * A * B, st);
-        k_transpose<<<grid, 256, 0, st>>>(in + (int64_t)b0 * in_sn, in_sn, in_sa, out + (int64_t)b0 * out_sn, out_sn,
+        ProfScope ps(K_TRANSPOSE, 2.0 * sizeof(T) * nb * A * B, st);
+        k_transpose<T><<<grid, 256, 0, st>>>(in + (int64_t)b0 * in_sn, in_sn, in_sa, out + (int64_t)b0 * out_sn, out_sn,
                                           out_sb, A, B);
         FDN_LAUNCHED("k_transpose");
     }
     return FDN_OK;
 }
 
-int launch_transpose(const float* in, float* out, int n, int A, int B, cudaStream_t st)
+template <typename T>
+int launch_transpose(const T* in, T* out, int n, int A, int B, cudaStream_t st)
 {
     return launch_transpose_strided(in, (int64_t)A * B, B, out, (int64_t)A * B, A, n, A, B, st);
 }
@@ -383,4 +449,22 @@ int launch_copy3d(const float* in, int64_t in_sa, int64_t in_sb, int b0, int bw,
     return FDN_OK;
 }
 
+#define FDN_INST_WARP(T)                                                                                              \
+    template int launch_warp_pair<T>(const T*, int64_t, int64_t, SlotMap, const float*, double, float*, int64_t, int64_t, \
+                                     T*, int, int, int, int, cudaStream_t);                                               \
+    template int launch_acc_finish<T>(const T*, int64_t, int64_t, SlotMap, const T*, int, const double*, float*, int64_t, \
+                                      int64_t, T*, int64_t, int64_t, int, int, int, int, cudaStream_t);
+FDN_INST_WARP(float)
+FDN_INST_WARP(uint8_t)
+FDN_INST_WARP(uint16_t)
+FDN_INST_WARP(int16_t)
+template int launch_remap<uint8_t>(const uint8_t*, const float*, uint8_t*, int, int, int, cudaStream_t);
+template int launch_remap<uint16_t>(const uint16_t*, const float*, uint16_t*, int, int, int, cudaStream_t);
+template int launch_remap<int16_t>(const int16_t*, const float*, int16_t*, int, int, int, cudaStream_t);
+#define FDN_INST_TRANSPOSE(T)                                                                                         \
+    template int launch_transpose<T>(const T*, T*, int, int, int, cudaStream_t);                                      \
+    template int launch_transpose_strided<T>(const T*, int64_t, int64_t, T*, int64_t, int64_t, int, int, int, cudaStream_t);
+FDN_INST_TRANSPOSE(float)
+FDN_INST_TRANSPOSE(uint8_t)
+FDN_INST_TRANSPOSE(uint16_t)
 }  // namespace fdn

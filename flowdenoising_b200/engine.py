@@ -4,7 +4,9 @@ PyTorch tensors own every device buffer (volume, output, workspace); the C libra
 Nothing here computes on the CPU.
 
 Mirrors the reference's pass driver `GaussianDenoising.filter` / `filter_along_{Z,Y,X}`
-(/root/reference/src/flowdenoising.py:175-290) for a device-resident float32 volume [Z, Y, X].
+(/root/reference/src/flowdenoising.py:175-290) for a device-resident float32 volume [Z, Y, X]. A uint8, int8, uint16 or
+int16 volume runs the reference's integer semantics in its own dtype (typed passes, fdn_*_typed: integer remap,
+float32 accumulation, truncating store); int8 without optical flow only, like cv2.remap.
 """
 from __future__ import annotations
 
@@ -71,6 +73,16 @@ def _stream_ptr(torch):
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
+def dtype_code(t) -> int:
+    """FDN_DTYPE_* of a tensor's dtype (ValueError for any other dtype)."""
+    import torch
+    codes = {torch.float32: _lib.DTYPE_F32, torch.uint8: _lib.DTYPE_U8, torch.int8: _lib.DTYPE_I8,
+             torch.uint16: _lib.DTYPE_U16, torch.int16: _lib.DTYPE_I16}
+    if t.dtype not in codes:
+        raise ValueError(f"unsupported volume dtype {t.dtype} (float32, uint8, int8, uint16 or int16)")
+    return codes[t.dtype]
+
+
 class DeviceEngine:
     """Runs passes on device-resident float32 volumes. One engine per GPU / process."""
 
@@ -93,10 +105,15 @@ class DeviceEngine:
     def release_workspace(self):
         self._ws = None
 
-    def _pick_chunk(self, view: View, klen: int, ofp: OfParams) -> int:
+    def _workspace_bytes(self, view: View, klen: int, ofp: OfParams, chunk: int, dtype: int) -> int:
+        if dtype == _lib.DTYPE_F32:
+            return self.lib.fdn_workspace_bytes(C.byref(view), klen, C.byref(ofp), chunk)
+        return self.lib.fdn_workspace_bytes_typed(C.byref(view), klen, C.byref(ofp), chunk, dtype)
+
+    def _pick_chunk(self, view: View, klen: int, ofp: OfParams, dtype: int = _lib.DTYPE_F32) -> int:
         """Largest chunk of output slices whose workspace fits the limit (default: 85 % of free HBM)."""
         torch = self.torch
-        need = lambda c: self.lib.fdn_workspace_bytes(C.byref(view), klen, C.byref(ofp), c)
+        need = lambda c: self._workspace_bytes(view, klen, ofp, c, dtype)
         full = need(view.n_out)
         if full == 0:
             _lib.check(1)
@@ -138,9 +155,12 @@ class DeviceEngine:
     # ---- one pass over an explicit view ----
     def filter_view(self, d_in, d_out, view: View, kernel, flow: Optional[FlowParams], chunk: Optional[int] = None,
                     exact: bool = True):
-        """out[s] = sum_i k[i] * warp(in[s+halo+i-r]) for the slices of `view` (see fdn_view)."""
+        """out[s] = sum_i k[i] * warp(in[s+halo+i-r]) for the slices of `view` (see fdn_view). Integer tensors run the
+        typed pass (exact arithmetic only)."""
         torch = self.torch
         k, kp = _taps(kernel)
+        if d_in.dtype != torch.float32:
+            return self._filter_view_typed(d_in, d_out, view, k, kp, flow, chunk, exact)
         with torch.cuda.device(self.device):
             if flow is None:
                 _lib.check(self.lib.fdn_gauss_axis(d_in.data_ptr(), d_out.data_ptr(), C.byref(view), kp, k.size,
@@ -157,20 +177,49 @@ class DeviceEngine:
                                                 C.byref(ofp), int(chunk), ws.data_ptr(), ws.numel(),
                                                 _stream_ptr(torch)))
 
+    def _filter_view_typed(self, d_in, d_out, view: View, k, kp, flow: Optional[FlowParams], chunk, exact):
+        torch = self.torch
+        dt = dtype_code(d_in)
+        if d_out.dtype != d_in.dtype:
+            raise ValueError("a typed pass writes the dtype it reads")
+        with torch.cuda.device(self.device):
+            if flow is None:
+                _lib.check(self.lib.fdn_gauss_axis_typed(d_in.data_ptr(), d_out.data_ptr(), dt, C.byref(view), kp,
+                                                         k.size, int(bool(exact)), _stream_ptr(torch)))
+                return
+            ofp = flow.c_struct()
+            if chunk is None:
+                chunk = self._pick_chunk(view, k.size, ofp, dt)
+            nbytes = self._workspace_bytes(view, k.size, ofp, int(chunk), dt)
+            if nbytes == 0:
+                _lib.check(1)
+            ws = self._workspace(nbytes)
+            _lib.check(self.lib.fdn_filter_axis_typed(d_in.data_ptr(), d_out.data_ptr(), dt, C.byref(view), kp,
+                                                      k.size, C.byref(ofp), int(chunk), ws.data_ptr(), ws.numel(),
+                                                      _stream_ptr(torch)))
+
     # ---- passes over a dense [Z, Y, X] volume (single GPU, periodic along the filtered axis) ----
     def _check_vol(self, t):
         torch = self.torch
-        if not (t.is_cuda and t.dtype == torch.float32 and t.dim() == 3 and t.is_contiguous()):
-            raise ValueError("expected a contiguous float32 CUDA tensor [Z, Y, X]")
+        if not (t.is_cuda and t.dim() == 3 and t.is_contiguous()):
+            raise ValueError("expected a contiguous CUDA tensor [Z, Y, X]")
+        if t.dtype != torch.float32:
+            dtype_code(t)
 
     def transpose_yx(self, src, dst=None):
-        """[n, A, B] -> [n, B, A] with the library's transpose kernel."""
+        """[n, A, B] -> [n, B, A] with the library's transpose kernel (any dtype of a typed volume)."""
         torch = self.torch
         n, A, B = src.shape
         if dst is None:
-            dst = torch.empty((n, B, A), dtype=torch.float32, device=src.device)
+            dst = torch.empty((n, B, A), dtype=src.dtype, device=src.device)
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.fdn_transpose_yx(src.data_ptr(), dst.data_ptr(), n, A, B, _stream_ptr(torch)))
+            if src.dtype == torch.float32:
+                _lib.check(self.lib.fdn_transpose_yx(src.data_ptr(), dst.data_ptr(), n, A, B, _stream_ptr(torch)))
+            else:
+                if dst.dtype != src.dtype:
+                    raise ValueError("transpose_yx keeps the dtype")
+                _lib.check(self.lib.fdn_transpose_yx_typed(src.data_ptr(), dst.data_ptr(), dtype_code(src), n, A, B,
+                                                           _stream_ptr(torch)))
         return dst
 
     def empty(self, shape):
@@ -206,6 +255,8 @@ class DeviceEngine:
         self._check_vol(vol); self._check_vol(out)
         if vol.data_ptr() == out.data_ptr():
             raise ValueError("in-place passes are not supported")
+        if vol.dtype != out.dtype:
+            raise ValueError("a pass writes the dtype it reads")
         Z, Y, X = vol.shape
         if axis == 0:
             v = View(Z, Z, 0, 1, Y, X, Y * X, X, Y * X, X)
@@ -217,8 +268,12 @@ class DeviceEngine:
             if flow is None:
                 k, kp = _taps(kernel)
                 with torch.cuda.device(self.device):
-                    _lib.check(self.lib.fdn_gauss_rows(vol.data_ptr(), out.data_ptr(), Z * Y, X, kp, k.size,
-                                                       int(bool(exact)), _stream_ptr(torch)))
+                    if vol.dtype == torch.float32:
+                        _lib.check(self.lib.fdn_gauss_rows(vol.data_ptr(), out.data_ptr(), Z * Y, X, kp, k.size,
+                                                           int(bool(exact)), _stream_ptr(torch)))
+                    else:
+                        _lib.check(self.lib.fdn_gauss_rows_typed(vol.data_ptr(), out.data_ptr(), dtype_code(vol), Z * Y,
+                                                                 X, kp, k.size, int(bool(exact)), _stream_ptr(torch)))
                 return
             # slices vol[:, :, x] are (Z, Y) images with element-strided columns: run on the [Z, X, Y] transpose
             vt = self.transpose_yx(vol, scratch[0] if scratch else None)
@@ -239,7 +294,7 @@ class DeviceEngine:
         # every volume-sized buffer exists before the first pass sizes its workspace from the free memory
         a = torch.empty_like(vol)
         b = torch.empty_like(vol)
-        ot = torch.empty((Z, X, Y), dtype=torch.float32, device=vol.device) if flow is not None else torch.empty_like(vol)
+        ot = torch.empty((Z, X, Y), dtype=vol.dtype, device=vol.device) if flow is not None else torch.empty_like(vol)
         self.filter_along_axis(vol, a, 0, kernels[0], flow, chunk, exact)
         self.filter_along_axis(a, b, 1, kernels[1], flow, chunk, exact)      # b = ZY
         if flow is None:

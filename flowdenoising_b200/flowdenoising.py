@@ -9,7 +9,9 @@ C ABI of ``libfdn_b200.so``; there is no CPU fallback.
 Differences from the reference that are deliberate (SURVEY.md App. B):
   * ``filter()`` returns ``filtered_vol`` (the reference returns None, Q1); like the reference it leaves the
     Z+Y intermediate in ``vol`` and the Z+Y+X result in ``filtered_vol``.
-  * Volumes are processed as float32; integer inputs are converted (Q3).
+  * Volumes are processed as float32; integer inputs are converted (Q3). With ``keep_dtype=True`` (CLI
+    ``--keep_dtype``) a uint8, uint16 or int16 volume (int8 without OF) keeps its dtype through every pass with the
+    reference's integer arithmetic instead, bit for bit.
   * ``l``/``w`` are instance state, not module globals (Q5); iterations / poly_n / poly_sigma are parameters.
   * ``number_of_processes`` is accepted and ignored: slices are batched on the GPU.
 '''
@@ -426,10 +428,17 @@ def get_flow_without_prev_flow(reference, target, l=OF_LEVELS, w=OF_WINDOW_SIZE,
     return _get_flow(reference, target, l, w, None, False, iterations, poly_n, poly_sigma, gaussian_window)
 
 
-class GaussianDenoising():
-    '''src/flowdenoising.py:116-295.'''
+_TYPED_DTYPES = (np.dtype(np.uint8), np.dtype(np.int8), np.dtype(np.uint16), np.dtype(np.int16))
 
-    def __init__(self, number_of_processes, vol):
+
+class GaussianDenoising():
+    '''src/flowdenoising.py:116-295.
+
+    keep_dtype=True: an integer volume is filtered in its own dtype with the reference's integer semantics (integer
+    remap of each neighbour, float32 accumulation, truncation toward zero at every pass's store, the next pass reading
+    the truncated result), bit for bit. Without it (the default), or for a float32 volume, the passes run in float32.'''
+
+    def __init__(self, number_of_processes, vol, keep_dtype=False):
         self._progress_done = 0.0
         self._progress_mark = None      # library counter at the start of the device call in flight
         self.number_of_processes = number_of_processes
@@ -448,6 +457,7 @@ class GaussianDenoising():
         self.devices = None       # CUDA devices to spread slabs over (None: the current one)
         self.slab_slices = None   # output slices per streamed slab (None: sized from the free device memory)
         self.streaming = None     # None: stream slab by slab only when needed (memory map, > device memory, ...)
+        self.keep_dtype = bool(keep_dtype)
 
     # The reference bumps `progress` once per finished slice (:139-140) and feedback() prints it (:292-295). Here the
     # count of the device call in flight comes from the library (host functions in the stream after every chain step).
@@ -472,6 +482,29 @@ class GaussianDenoising():
     # -- device plumbing --
     def _flow(self):
         return self._flow_params
+
+    def _typed(self):
+        """True when the passes run in the volume's integer dtype (keep_dtype); raises ValueError for a combination
+        that is not supported rather than converting silently."""
+        dt = self.vol.dtype
+        if not self.keep_dtype or (dt.kind == "f" and dt.itemsize >= 4):
+            return False
+        if dt not in _TYPED_DTYPES or not dt.isnative:
+            raise ValueError(f"keep_dtype: {dt} volumes are not supported (native uint8, int8, uint16 or int16; "
+                             f"float16 is out of scope)")
+        if dt == np.int8 and self._flow() is not None:
+            raise ValueError("keep_dtype: int8 volumes are supported without optical flow only (cv2.remap, which the "
+                             "reference calls, rejects int8 images)")
+        if self.streaming or isinstance(self.vol, np.memmap) or self.border != "wrap" or \
+                (self.devices and len(self.devices) > 1):
+            raise ValueError("keep_dtype: streaming (memory maps, --border mean, --gpus > 1) is not supported for "
+                             "integer volumes")
+        eng = _get_engine()
+        free, _total = eng.torch.cuda.mem_get_info(eng.device)
+        # the volume, two intermediates and the result in the dtype, the float32 chunk accumulator in the workspace
+        if 4 * dt.itemsize * self.vol.size + (2 << 30) > 0.9 * free:
+            raise ValueError("keep_dtype: integer volumes larger than the device are not supported")
+        return True
 
     def _streaming_needed(self):
         if self.streaming is not None:
@@ -498,6 +531,14 @@ class GaussianDenoising():
         torch = eng.torch
         kernel = np.asarray(kernel, dtype=np.float64)
         assert kernel.size % 2 != 0  # kernel.size must be odd (src/flowdenoising.py:309)
+        if self._typed():
+            d_in = torch.from_numpy(np.ascontiguousarray(self.vol)).to(eng.device)
+            d_out = torch.empty_like(d_in)
+            self._begin_device_call()
+            eng.filter_along_axis(d_in, d_out, axis, kernel, self._flow(), exact=self.exact)
+            self.filtered_vol[...] = d_out.cpu().numpy()
+            self._end_device_call(self.vol.shape[axis])
+            return
         if self._streaming_needed():
             sd, done0 = self._streamer()
             dst = self.filtered_vol if self.filtered_vol.dtype == np.float32 else np.empty(self.vol.shape, np.float32)
@@ -537,10 +578,12 @@ class GaussianDenoising():
         r = kernel.size // 2
         n = self.vol.shape[axis]
         idxs = [(idx + d) % n for d in range(-r, r + 1)]
-        slab = np.ascontiguousarray(np.moveaxis(np.take(self.vol, idxs, axis=axis), axis, 0), dtype=np.float32)
+        typed = self._typed()
+        slab = np.ascontiguousarray(np.moveaxis(np.take(self.vol, idxs, axis=axis), axis, 0),
+                                    dtype=self.vol.dtype if typed else np.float32)
         d_in = torch.from_numpy(slab).to(eng.device)
         H, W = slab.shape[1:]
-        d_out = torch.empty((1, H, W), dtype=torch.float32, device=eng.device)
+        d_out = torch.empty((1, H, W), dtype=d_in.dtype, device=eng.device)
         v = _engine.View(2 * r + 1, 1, r, 0, H, W, H * W, W, H * W, W)
         eng.filter_view(d_in, d_out, v, kernel, self._flow(), exact=self.exact)
         res = d_out[0].cpu().numpy()
@@ -569,10 +612,12 @@ class GaussianDenoising():
         r = kernel.size // 2
         n = self.vol.shape[axis]
         idxs = [(start + d) % n for d in range(-r, count + r)]
-        slab = np.ascontiguousarray(np.moveaxis(np.take(self.vol, idxs, axis=axis), axis, 0), dtype=np.float32)
+        typed = self._typed()
+        slab = np.ascontiguousarray(np.moveaxis(np.take(self.vol, idxs, axis=axis), axis, 0),
+                                    dtype=self.vol.dtype if typed else np.float32)
         d_in = torch.from_numpy(slab).to(eng.device)
         H, W = slab.shape[1:]
-        d_out = torch.empty((count, H, W), dtype=torch.float32, device=eng.device)
+        d_out = torch.empty((count, H, W), dtype=d_in.dtype, device=eng.device)
         v = _engine.View(count + 2 * r, count, r, 0, H, W, H * W, W, H * W, W)
         eng.filter_view(d_in, d_out, v, kernel, self._flow(), exact=self.exact)
         res = d_out.cpu().numpy()
@@ -608,6 +653,15 @@ class GaussianDenoising():
             assert np.asarray(k).size % 2 != 0
         ks = [np.asarray(k, np.float64) for k in kernels]
         Z, Y, X = (int(v) for v in self.vol.shape)
+        if self._typed():
+            # the plain sequence: upload in the dtype, three typed passes, the ZY intermediate and the result home
+            d_in = torch.from_numpy(np.ascontiguousarray(self.vol)).to(eng.device)
+            self._begin_device_call()
+            zy, zyx = eng.filter(d_in, ks, self._flow(), exact=self.exact)
+            self.vol[...] = zy.cpu().numpy()
+            self.filtered_vol[...] = zyx.cpu().numpy()
+            self._end_device_call(Z + Y + X)
+            return self.filtered_vol
         if self._streaming_needed():
             sd, done0 = self._streamer()
             fv = self.filtered_vol if self.filtered_vol.dtype == np.float32 else np.empty(self.vol.shape, np.float32)
@@ -753,8 +807,9 @@ class FlowDenoising(GaussianDenoising):
     ``warp_slice`` is accepted for signature compatibility (the remap is fused into the accumulation kernel).'''
 
     def __init__(self, number_of_processes, vol, l=OF_LEVELS, w=OF_WINDOW_SIZE, get_flow=None, warp_slice=None,
-                 iterations=OF_ITERS, poly_n=OF_POLY_N, poly_sigma=OF_POLY_SIGMA, gaussian_window=False):
-        super().__init__(number_of_processes, vol)
+                 iterations=OF_ITERS, poly_n=OF_POLY_N, poly_sigma=OF_POLY_SIGMA, gaussian_window=False,
+                 keep_dtype=False):
+        super().__init__(number_of_processes, vol, keep_dtype=keep_dtype)
         self.l = l
         self.w = w
         self.get_flow = get_flow if get_flow is not None else get_flow_with_prev_flow
@@ -816,6 +871,12 @@ def build_parser():
                         help="Farneback with a Gaussian window instead of the box window (cv2.OPTFLOW_FARNEBACK_GAUSSIAN): "
                              "changes the flow estimate, usually more accurate; it is not a speed switch. Wants a larger "
                              "--winsize for the same robustness; winsize 2m and 2m+1 give the same window")
+    parser.add_argument("--keep_dtype", action="store_true",
+                        help="Filter an integer MRC volume (modes 0, 1, 6) in its own dtype with the reference's integer "
+                             "arithmetic (integer remap, truncation after every pass), for bit-for-bit parity with "
+                             "flowdenoising.py on integer input. Without it integer volumes are filtered as float32. "
+                             "TIFF input is float32 either way; the output file is float32 (MRC mode 2). Not with -m, "
+                             "--border mean or --gpus > 1; int8 (mode 0) only with --no_OF")
     parser.add_argument("--compat_zy_output", action="store_true",
                         help="Write the Z+Y intermediate like the reference CLI does (flowdenoising.py:520) "
                              "instead of the full Z+Y+X result")
@@ -870,7 +931,11 @@ def main(argv=None):
     vol = volume_io.read_volume(args.input, memory_map=args.memory_map)
     logging.info(f"read \"{args.input}\" in {time.perf_counter() - time_0} seconds")
     mapped = isinstance(vol, np.memmap)
-    if not mapped:      # (-m: the volume stays in the file and streams through the device slab by slab)
+    if args.keep_dtype and vol.dtype.kind in "iu" and not mapped:
+        vol = np.ascontiguousarray(vol, dtype=vol.dtype.newbyteorder("="))      # (-m with it: ValueError in filter)
+    elif args.keep_dtype and vol.dtype == np.float16:
+        pass                                                                    # ValueError in filter
+    elif not mapped:      # (-m: the volume stays in the file and streams through the device slab by slab)
         vol = np.ascontiguousarray(vol, dtype=np.float32)
 
     kernels = [get_gaussian_kernel(s) for s in sigma]
@@ -881,11 +946,11 @@ def main(argv=None):
     logging.info(f"{args.input} average = {vol.mean()}")
 
     if args.no_OF:
-        fd = GaussianDenoising(args.number_of_processes, vol)
+        fd = GaussianDenoising(args.number_of_processes, vol, keep_dtype=args.keep_dtype)
     else:
         fd = FlowDenoising(args.number_of_processes, vol, args.levels, args.winsize, get_flow, warp_slice,
                            iterations=args.iterations, poly_n=args.poly_n, poly_sigma=args.poly_sigma,
-                           gaussian_window=args.gaussian_window)
+                           gaussian_window=args.gaussian_window, keep_dtype=args.keep_dtype)
     fd.border = args.border
     fd.slab_slices = args.slab_slices
     if args.gpus > 1:

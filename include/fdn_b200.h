@@ -137,6 +137,32 @@ int fdn_gauss_rows(const float* d_in, float* d_out, int64_t n_rows, int W, const
 /* Batched 2-D transpose of the last two axes: in [n][A][B] -> out [n][B][A]. */
 int fdn_transpose_yx(const float* d_in, float* d_out, int n, int A, int B, void* stream);
 
+/* ---- typed volumes: the reference's integer semantics (SURVEY App. B Q3) ----
+ * An integer volume keeps its dtype through a pass in the reference: cv2.remap of an integer neighbour returns an
+ * integer image (OpenCV's integer rounding: fixed point for 8U, float32 weights + rint + saturation for 16U/16S), the
+ * taps accumulate in float32 exactly as for float32 volumes, and the store into the integer result truncates toward
+ * zero. These entry points run that on device volumes of the given element type (d_in / d_out: T elements, strides
+ * in elements). FDN_DTYPE_F32 forwards to the float32 entry points above. Rejected with FDN_ERR_INVALID: an unknown
+ * dtype, int8 with optical flow (cv2.remap rejects int8), and exact == 0 for an integer dtype. */
+#define FDN_DTYPE_F32 0
+#define FDN_DTYPE_U8 1
+#define FDN_DTYPE_I8 2
+#define FDN_DTYPE_U16 3
+#define FDN_DTYPE_I16 4
+/* workspace of fdn_filter_axis_typed (0 on error, and for of == NULL) */
+size_t fdn_workspace_bytes_typed(const fdn_view* view, int klen, const fdn_of_params* of, int chunk, int dtype);
+/* fdn_filter_axis on a typed volume; of == NULL: the exact no-OF pass */
+int fdn_filter_axis_typed(const void* d_in, void* d_out, int dtype, const fdn_view* view, const double* kernel, int klen,
+                          const fdn_of_params* of, int chunk, void* d_workspace, size_t workspace_bytes, void* stream);
+int fdn_gauss_axis_typed(const void* d_in, void* d_out, int dtype, const fdn_view* view, const double* kernel, int klen,
+                         int exact, void* stream);
+int fdn_gauss_rows_typed(const void* d_in, void* d_out, int dtype, int64_t n_rows, int W, const double* kernel, int klen,
+                         int exact, void* stream);
+int fdn_transpose_yx_typed(const void* d_in, void* d_out, int dtype, int n, int A, int B, void* stream);
+/* Stage entry point: cv2.remap(src, flow + grid, INTER_LINEAR, BORDER_REPLICATE) of n dense (H, W) images of the
+ * dtype; flow (n, H, W, 2) float32. */
+int fdn_remap_typed(const void* d_src, const float* d_flow, void* d_dst, int dtype, int n, int H, int W, void* stream);
+
 /* Strided variants used by the multi-GPU re-slab (flowdenoising_b200/dist.py):
  *   fdn_transpose_strided: out[n*out_sn + b*out_sb + a] = in[n*in_sn + a*in_sa + b]           (a < A, b < B)
  *   fdn_copy3d           : out[a*out_sa + b*out_sb + c] = in[a*in_sa + ((b0+b) mod b_wrap)*in_sb + ((c0+c) mod c_wrap)]
