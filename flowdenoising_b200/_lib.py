@@ -99,6 +99,10 @@ SIGNATURES = {
                                        C.c_int, C.c_void_p]),
     "fdn_transpose_yx_typed": (C.c_int, [c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "fdn_remap_typed": (C.c_int, [c_f32p, c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "fdn_transpose_strided_typed": (C.c_int, [c_f32p, C.c_int, c_i64, c_i64, c_f32p, c_i64, c_i64, C.c_int, C.c_int,
+                                              C.c_int, C.c_void_p]),
+    "fdn_copy3d_typed": (C.c_int, [c_f32p, C.c_int, c_i64, c_i64, C.c_int, C.c_int, C.c_int, C.c_int, c_f32p, c_i64,
+                                   c_i64, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "fdn_warp_accumulate": (C.c_int, [c_f32p, c_i64, c_i64, c_f32p, C.c_double, c_f32p, c_i64, c_i64, C.c_int,
                                       C.c_int, C.c_int, C.c_void_p]),
 }

@@ -721,6 +721,46 @@ int fdn_copy3d(const float* d_in, int64_t in_sa, int64_t in_sb, int b0, int b_wr
                          static_cast<cudaStream_t>(stream));
 }
 
+int fdn_transpose_strided_typed(const void* d_in, int dtype, int64_t in_sn, int64_t in_sa, void* d_out, int64_t out_sn,
+                                int64_t out_sb, int n, int A, int B, void* stream)
+{
+    int rc;
+    if ((rc = check_dtype(dtype, false))) return rc;
+    FDN_CHECK_ARG(d_in && d_out && n >= 1 && A >= 1 && B >= 1, "bad argument");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    switch (dtype_size(dtype)) {   // a transpose moves bits: one kernel per element size
+        case 1:
+            return launch_transpose_strided(static_cast<const uint8_t*>(d_in), in_sn, in_sa, static_cast<uint8_t*>(d_out),
+                                            out_sn, out_sb, n, A, B, st);
+        case 2:
+            return launch_transpose_strided(static_cast<const uint16_t*>(d_in), in_sn, in_sa,
+                                            static_cast<uint16_t*>(d_out), out_sn, out_sb, n, A, B, st);
+        default:
+            return fdn_transpose_strided(static_cast<const float*>(d_in), in_sn, in_sa, static_cast<float*>(d_out), out_sn,
+                                         out_sb, n, A, B, stream);
+    }
+}
+
+int fdn_copy3d_typed(const void* d_in, int dtype, int64_t in_sa, int64_t in_sb, int b0, int b_wrap, int c0, int c_wrap,
+                     void* d_out, int64_t out_sa, int64_t out_sb, int A, int B, int C, void* stream)
+{
+    int rc;
+    if ((rc = check_dtype(dtype, false))) return rc;
+    FDN_CHECK_ARG(d_in && d_out && A >= 1 && B >= 1 && C >= 1, "bad argument");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    switch (dtype_size(dtype)) {   // a copy moves bits: one kernel per element size
+        case 1:
+            return launch_copy3d(static_cast<const uint8_t*>(d_in), in_sa, in_sb, b0, b_wrap, c0, c_wrap,
+                                 static_cast<uint8_t*>(d_out), out_sa, out_sb, A, B, C, st);
+        case 2:
+            return launch_copy3d(static_cast<const uint16_t*>(d_in), in_sa, in_sb, b0, b_wrap, c0, c_wrap,
+                                 static_cast<uint16_t*>(d_out), out_sa, out_sb, A, B, C, st);
+        default:
+            return fdn_copy3d(static_cast<const float*>(d_in), in_sa, in_sb, b0, b_wrap, c0, c_wrap,
+                              static_cast<float*>(d_out), out_sa, out_sb, A, B, C, stream);
+    }
+}
+
 int fdn_copy2d_async(void* dst, size_t dst_pitch, const void* src, size_t src_pitch, size_t width_bytes, size_t rows,
                      int direction, void* stream)
 {

@@ -178,7 +178,8 @@ int launch_transpose(const T* in, T* out, int n, int A, int B, cudaStream_t st);
 template <typename T>
 int launch_transpose_strided(const T* in, int64_t in_sn, int64_t in_sa, T* out, int64_t out_sn, int64_t out_sb, int n,
                              int A, int B, cudaStream_t st);
-int launch_copy3d(const float* in, int64_t in_sa, int64_t in_sb, int b0, int bw, int c0, int cw, float* out,
+template <typename T>
+int launch_copy3d(const T* in, int64_t in_sa, int64_t in_sb, int b0, int bw, int c0, int cw, T* out,
                   int64_t out_sa, int64_t out_sb, int A, int B, int C, cudaStream_t st);
 
 #ifdef __CUDACC__

@@ -416,12 +416,22 @@ int launch_transpose(const T* in, T* out, int n, int A, int B, cudaStream_t st)
 // ------------------------------------------------------------------------------------------------
 // Strided 3-D copy with periodic index offsets (the packing side of the re-slab / halo exchange):
 //   out[a*out_sa + b*out_sb + c] = in[a*in_sa + ((b0 + b) mod bw)*in_sb + ((c0 + c) mod cw)]
+// A copy moves bits: one kernel per element size (1, 2, 4 bytes). 4-byte elements take one per thread. Narrower ones
+// take a run of 4 bytes of consecutive c per thread (4 uint8 / 2 uint16), so that a warp's stores cover 128 contiguous
+// bytes instead of 32 / 64; the run is stored as one 32-bit word where the destination is 4-byte aligned and does not
+// end inside it. Reads follow the periodic index element by element; a run that crosses the wrap takes the guarded
+// loop.
 // ------------------------------------------------------------------------------------------------
+template <typename T>
+__host__ __device__ constexpr int copy3d_run() { return sizeof(T) >= 4 ? 1 : (int)(4 / sizeof(T)); }
+
+template <typename T>
 __global__ void __launch_bounds__(256)
-k_copy3d(const float* __restrict__ in, int64_t in_sa, int64_t in_sb, int b0, int bw, int c0, int cw,
-         float* __restrict__ out, int64_t out_sa, int64_t out_sb, int B, int C)
+k_copy3d(const T* __restrict__ in, int64_t in_sa, int64_t in_sb, int b0, int bw, int c0, int cw,
+         T* __restrict__ out, int64_t out_sa, int64_t out_sb, int B, int C)
 {
-    const int c = blockIdx.x * 256 + threadIdx.x;
+    constexpr int R = copy3d_run<T>();
+    const int c = (blockIdx.x * 256 + threadIdx.x) * R;
     const int b = blockIdx.y;
     const int64_t a = blockIdx.z;
     if (c >= C) return;
@@ -430,20 +440,46 @@ k_copy3d(const float* __restrict__ in, int64_t in_sa, int64_t in_sb, int b0, int
     int ci = (c0 + c) % cw;
     if (ci < 0) ci += cw;
     (void)B;
-    out[a * out_sa + (int64_t)b * out_sb + c] = in[a * in_sa + (int64_t)bi * in_sb + ci];
+    if constexpr (R == 1) {
+        out[a * out_sa + (int64_t)b * out_sb + c] = in[a * in_sa + (int64_t)bi * in_sb + ci];
+    } else {
+        const T* src = in + a * in_sa + (int64_t)bi * in_sb;
+        T* dst = out + a * out_sa + (int64_t)b * out_sb + c;
+        const int n = C - c < R ? C - c : R;
+        union { uint32_t w; T e[R]; } v;
+        v.w = 0;
+        if (ci + n <= cw) {
+#pragma unroll
+            for (int j = 0; j < R; j++)
+                if (j < n) v.e[j] = src[ci + j];
+        } else {                                    // the run crosses the wrap (possibly more than once: cw < R)
+#pragma unroll
+            for (int j = 0; j < R; j++)
+                if (j < n) v.e[j] = src[(ci + j) % cw];
+        }
+        if (n == R && (reinterpret_cast<uintptr_t>(dst) & 3) == 0) {
+            *reinterpret_cast<uint32_t*>(dst) = v.w;
+        } else {
+#pragma unroll
+            for (int j = 0; j < R; j++)
+                if (j < n) dst[j] = v.e[j];
+        }
+    }
 }
 
-int launch_copy3d(const float* in, int64_t in_sa, int64_t in_sb, int b0, int bw, int c0, int cw, float* out,
+template <typename T>
+int launch_copy3d(const T* in, int64_t in_sa, int64_t in_sb, int b0, int bw, int c0, int cw, T* out,
                   int64_t out_sa, int64_t out_sb, int A, int B, int C, cudaStream_t st)
 {
     FDN_CHECK_ARG(B <= 65535, "copy3d: B too large");
     FDN_CHECK_ARG(bw >= 1 && cw >= 1, "copy3d: wrap lengths must be >= 1");
+    constexpr int R = copy3d_run<T>();
     for (int a0 = 0; a0 < A; a0 += 65535) {
         const int na = A - a0 < 65535 ? A - a0 : 65535;
-        dim3 grid((unsigned)cdiv(C, 256), (unsigned)B, (unsigned)na);
-        ProfScope ps(K_COPY3D, 8.0 * na * B * C, st);
-        k_copy3d<<<grid, 256, 0, st>>>(in + (int64_t)a0 * in_sa, in_sa, in_sb, b0, bw, c0, cw,
-                                       out + (int64_t)a0 * out_sa, out_sa, out_sb, B, C);
+        dim3 grid((unsigned)cdiv(C, 256 * R), (unsigned)B, (unsigned)na);
+        ProfScope ps(K_COPY3D, 2.0 * sizeof(T) * na * B * C, st);
+        k_copy3d<T><<<grid, 256, 0, st>>>(in + (int64_t)a0 * in_sa, in_sa, in_sb, b0, bw, c0, cw,
+                                          out + (int64_t)a0 * out_sa, out_sa, out_sb, B, C);
         FDN_LAUNCHED("k_copy3d");
     }
     return FDN_OK;
@@ -463,7 +499,9 @@ template int launch_remap<uint16_t>(const uint16_t*, const float*, uint16_t*, in
 template int launch_remap<int16_t>(const int16_t*, const float*, int16_t*, int, int, int, cudaStream_t);
 #define FDN_INST_TRANSPOSE(T)                                                                                         \
     template int launch_transpose<T>(const T*, T*, int, int, int, cudaStream_t);                                      \
-    template int launch_transpose_strided<T>(const T*, int64_t, int64_t, T*, int64_t, int64_t, int, int, int, cudaStream_t);
+    template int launch_transpose_strided<T>(const T*, int64_t, int64_t, T*, int64_t, int64_t, int, int, int, cudaStream_t); \
+    template int launch_copy3d<T>(const T*, int64_t, int64_t, int, int, int, int, T*, int64_t, int64_t, int, int, int,      \
+                                  cudaStream_t);
 FDN_INST_TRANSPOSE(float)
 FDN_INST_TRANSPOSE(uint8_t)
 FDN_INST_TRANSPOSE(uint16_t)

@@ -18,6 +18,10 @@ Packing / transposing are the library's own kernels (fdn_copy3d, fdn_transpose_s
 all-to-all / grouped send-recv (torch.distributed is plumbing only). Results are bit-identical for any number of
 ranks because every slice is computed from identical inputs by the same kernels.
 
+A typed slab (keep_dtype: uint8, int8, uint16 or int16) runs the same sequence in its own dtype: every buffer has the
+slab's dtype, the kernels are the typed ones (fdn_copy3d_typed, fdn_transpose_strided_typed, typed passes), and the
+exchanges carry byte views of the buffers, because NCCL has no 16-bit integer type (an exchange only moves bits).
+
 The compute object (`ops`) is a DeviceEngine; tests inject a CPU stand-in to exercise this host logic with the gloo
 backend (tests/test_dist_gloo.py).
 """
@@ -57,11 +61,35 @@ class DistributedDenoiser:
         self.y_range = split_range(Y, self.world, self.rank)
         self.x_range = split_range(X, self.world, self.rank)
         self.backend = dist.get_backend(group)
+        self.dtype = self.torch.float32       # of the slab being filtered (set by filter / filter_host)
+
+    def _empty(self, shape):
+        """A buffer in the slab's dtype (float32 slabs: the one-argument call of the float route)."""
+        if self.dtype == self.torch.float32:
+            return self.ops.empty(shape)
+        return self.ops.empty(shape, self.dtype)
+
+    def _wire(self, t):
+        """What an exchange carries for the contiguous tensor t: t itself for float32, its bytes otherwise (NCCL has no
+        16-bit integer type; the exchanges only move bits, so a byte view is right for every dtype)."""
+        if t.dtype == self.torch.float32:
+            return t
+        return t.reshape(-1).view(self.torch.uint8)
+
+    def _use_dtype(self, t):
+        if t.dtype != self.torch.float32:
+            from .engine import dtype_code
+            dtype_code(t)                     # ValueError for an unsupported dtype
+        self.dtype = t.dtype
 
     # ------------------------------------------------------------------ communication primitives
     def _all_to_all(self, send_flat, send_sizes, recv_flat, recv_sizes):
-        """One flat float32 buffer per direction, split per peer (own block included)."""
+        """One flat buffer per direction, split per peer (own block included); typed buffers travel as bytes."""
         dist = self.dist
+        if send_flat.dtype != self.torch.float32:
+            k = send_flat.element_size()
+            send_flat, recv_flat = self._wire(send_flat), self._wire(recv_flat)
+            send_sizes, recv_sizes = [k * int(n) for n in send_sizes], [k * int(n) for n in recv_sizes]
         if self.backend == "nccl":
             dist.all_to_all_single(recv_flat, send_flat, list(recv_sizes), list(send_sizes), group=self.group)
             return
@@ -89,8 +117,8 @@ class DistributedDenoiser:
         ops = self.ops
         ssz = [int(np.prod(sh)) for sh in send_shapes]
         rsz = [int(np.prod(sh)) for sh in recv_shapes]
-        send_flat = ops.empty((sum(ssz),))
-        recv_flat = ops.empty((sum(rsz),))
+        send_flat = self._empty((sum(ssz),))
+        recv_flat = self._empty((sum(rsz),))
         off = 0
         for p in range(self.world):
             pack(p, send_flat[off:off + ssz[p]])
@@ -132,16 +160,21 @@ class DistributedDenoiser:
                 continue
             mine = [(e, z) for (e, z) in need if owner_of(z) == p]
             if mine:
-                buf = ops.empty((len(mine), Y, X))
+                buf = self._empty((len(mine), Y, X))
                 recv_bufs[p] = (buf, mine)
-                p2p.append(dist.P2POp(dist.irecv, buf, self._global_rank(p), self.group))
+                p2p.append(dist.P2POp(dist.irecv, self._wire(buf), self._global_rank(p), self.group))
             pzs, pze = owner_ranges[p]
             pl = pze - pzs
             theirs = [(pzs - r + e) % Z for e in list(range(r)) + list(range(r + pl, pl + 2 * r))]
             theirs = [z for z in theirs if zs <= z < ze]
-            if theirs:
+            if theirs and self.dtype != torch.float32:
+                sbuf = self._empty((len(theirs), Y, X))          # (plain copies: torch has few uint16 device kernels)
+                for i, z in enumerate(theirs):
+                    sbuf[i].copy_(slab[z - zs])
+            elif theirs:
                 sbuf = torch.stack([slab[z - zs] for z in theirs]) if len(theirs) > 1 else slab[theirs[0] - zs][None].contiguous()
-                p2p.append(dist.P2POp(dist.isend, sbuf.contiguous(), self._global_rank(p), self.group))
+            if theirs:
+                p2p.append(dist.P2POp(dist.isend, self._wire(sbuf.contiguous()), self._global_rank(p), self.group))
         for (e, z) in need:                      # halo slices that wrap onto my own slab (few ranks / tiny Z)
             if zs <= z < ze:
                 ext[e].copy_(slab[z - zs])
@@ -157,7 +190,7 @@ class DistributedDenoiser:
         """Returns [r + Zl + r][Y][X]: the local Z-slab with r periodic halo slices on both sides."""
         Z, Y, X = self.shape
         Zl = self.z_range[1] - self.z_range[0]
-        ext = self.ops.empty((Zl + 2 * r, Y, X))
+        ext = self._empty((Zl + 2 * r, Y, X))
         ext[r:r + Zl].copy_(slab)
         return self._z_halo_fill(ext, r)
 
@@ -183,7 +216,7 @@ class DistributedDenoiser:
         blocks = self._alltoall_blocks([(Zl, (yr[p][1] - yr[p][0]) + 2 * ry, X) for p in range(G)],
                                        [(zr[p][1] - zr[p][0], Yl + 2 * ry, X) for p in range(G)], pack_zy)
         Ye = Yl + 2 * ry
-        Ae = ops.empty((Z, Ye, X))
+        Ae = self._empty((Z, Ye, X))
         flatA = Ae.view(-1)
         for p in range(G):
             a, b = zr[p]
@@ -203,7 +236,7 @@ class DistributedDenoiser:
             ops.copy3d(B, a * Yl * X, Yl * X, X, 0, Yl, 0, X, buf, 0, Yl * X, X, b - a, Yl, X)
         blocks = self._alltoall_blocks([(zr[p][1] - zr[p][0], Yl, X) for p in range(G)],
                                        [(Zl, yr[p][1] - yr[p][0], X) for p in range(G)], pack_b)
-        zy_slab = ops.empty((Zl, Y, X))
+        zy_slab = self._empty((Zl, Y, X))
         for p in range(G):
             a, b = yr[p]
             ops.copy3d(blocks[p], 0, (b - a) * X, X, 0, b - a, 0, X, zy_slab, a * X, Y * X, X, Zl, b - a, X)
@@ -225,7 +258,7 @@ class DistributedDenoiser:
         Xe = Xl + 2 * rx
         blocks = self._alltoall_blocks([(Z, Yl, (xr[p][1] - xr[p][0]) + 2 * rx) for p in range(G)],
                                        [(Z, yr[p][1] - yr[p][0], Xe) for p in range(G)], pack_yx)
-        Ce = ops.empty((Z, Xe, Y))
+        Ce = self._empty((Z, Xe, Y))
         for p in range(G):
             a, b = yr[p]
             # block[z][y][x] -> Ce[z][x][a + y]
@@ -264,7 +297,9 @@ class DistributedDenoiser:
 
     # ------------------------------------------------------------------ the three passes
     def filter(self, slab, kernels, want_zy: bool = False):
-        """slab: this rank's Z-slab [Zl][Y][X] (float32, device). Returns (zy_slab or None, zyx_slab), both Z-slabs."""
+        """slab: this rank's Z-slab [Zl][Y][X] (device; float32, or a typed volume's uint8 / int8 / uint16 / int16:
+        every buffer and exchange is then in that dtype and each pass truncates like the reference's integer
+        `filtered_vol`). Returns (zy_slab or None, zyx_slab), both Z-slabs in the slab's dtype."""
         ops = self.ops
         Z, Y, X = self.shape
         Zl = self.z_range[1] - self.z_range[0]
@@ -274,10 +309,11 @@ class DistributedDenoiser:
         rz, ry, rx = kz.size // 2, ky.size // 2, kx.size // 2
         if tuple(slab.shape) != (Zl, Y, X):
             raise ValueError(f"rank {self.rank} expects a Z-slab of shape {(Zl, Y, X)}, got {tuple(slab.shape)}")
+        self._use_dtype(slab)
 
         # ---- Z pass
         ext = self._z_halo_extended(slab, rz)
-        A = ops.empty((Zl, Y, X))
+        A = self._empty((Zl, Y, X))
         v = View(Zl + 2 * rz, Zl, rz, 0, Y, X, Y * X, X, Y * X, X)
         ops.filter_view(ext, A, v, kz, self.flow, self.chunk, self.exact)
         del ext
@@ -298,7 +334,7 @@ class DistributedDenoiser:
         Ye = Yl + 2 * ry
 
         # ---- Y pass
-        B = ops.empty((Z, Yl, X))
+        B = self._empty((Z, Yl, X))
         v = View(Ye, Yl, ry, 0, Z, X, X, Ye * X, X, Yl * X)
         ops.filter_view(Ae, B, v, ky, self.flow, self.chunk, self.exact)
         del Ae
@@ -312,20 +348,20 @@ class DistributedDenoiser:
         Xe = Xl + 2 * rx
 
         # ---- X pass, re-slab X -> Z
-        D = ops.empty((Z, Xl, Y))
+        D = self._empty((Z, Xl, Y))
         if finish_x is not None:
             return zy_slab, finish_x(Ce, D, Xe)
         v = View(Xe, Xl, rx, 0, Z, Y, Y, Xe * Y, Y, Xl * Y)
         ops.filter_view(Ce, D, v, kx, self.flow, self.chunk, self.exact)
         del Ce
-        out = ops.empty((Zl, Y, X))
+        out = self._empty((Zl, Y, X))
         self._reslab_xz(D, out)
         return zy_slab, out
 
     # ------------------------------------------------------------------ host slabs in, host slabs out
     def filter_host(self, host_slab, out_host, kernels, head: Optional[int] = None, tail: Optional[int] = None):
-        """The same three passes for a Z-slab that lives on the HOST (page-locked float32 tensors [Zl][Y][X]; the
-        result is written to out_host), with the transfers hidden behind the passes like the single-device plugin
+        """The same three passes for a Z-slab that lives on the HOST (page-locked tensors [Zl][Y][X] of one dtype, float32
+        or a typed volume's; the result is written to out_host), with the transfers hidden behind the passes like the single-device plugin
         (flowdenoising.py:_filter_overlapped): the slab's edge slices go up first and feed the halo exchange, the Z
         pass starts on its first `head` slices while the rest is still on its way, and the last `tail` columns of
         every rank's X-slab are computed while the other columns are already re-slabbed and travelling home.
@@ -338,6 +374,9 @@ class DistributedDenoiser:
         rz, rx = kz.size // 2, kx.size // 2
         if tuple(host_slab.shape) != (Zl, Y, X) or tuple(out_host.shape) != (Zl, Y, X):
             raise ValueError(f"rank {self.rank} expects Z-slabs of shape {(Zl, Y, X)}")
+        if out_host.dtype != host_slab.dtype:
+            raise ValueError("filter_host writes the dtype it reads")
+        self._use_dtype(host_slab)
         cp = _Copies(ops)
         _zr, _yr, xr = self._ranges()
         min_Zl = min(b - a for a, b in _zr)
@@ -351,7 +390,7 @@ class DistributedDenoiser:
         split_x = 1 <= tail < min_Xl
 
         # ---- upload (copy stream) and Z pass
-        ext = ops.empty((Zl + 2 * rz, Y, X))
+        ext = self._empty((Zl + 2 * rz, Y, X))
         mid = ext[rz:rz + Zl]
         cp.fence()
         if split_z:
@@ -367,7 +406,7 @@ class DistributedDenoiser:
             e_edges = e_head = e_all = cp.mark()
         cp.compute_waits(e_edges)
         self._z_halo_fill(ext, rz)
-        A = ops.empty((Zl, Y, X))
+        A = self._empty((Zl, Y, X))
         if split_z:
             cp.compute_waits(e_head)
             ops.filter_view(ext, A, View(head + 2 * rz, head, rz, 0, Y, X, Y * X, X, Y * X, X), kz, self.flow,
@@ -383,7 +422,7 @@ class DistributedDenoiser:
 
         # ---- X pass in two column ranges, each re-slabbed and sent home as soon as it is done
         def finish_x(Ce, D, Xe):
-            out = ops.empty((Zl, Y, X))
+            out = self._empty((Zl, Y, X))
             flatC, flatD = Ce.view(-1), D.view(-1)
             parts = [("body", 0, Xl - tail), ("tail", Xl - tail, tail)] if split_x else [("all", 0, Xl)]
             for part, first, n in parts:
@@ -432,8 +471,9 @@ class _Copies:
         """Columns [x0, x1) of a device volume [n][Y][X] -> the same columns of a host volume (pitched copy)."""
         if self.cuda:
             n, Y, X = (int(v) for v in src_dev.shape)
-            self.ops.copy2d_async(dst_host.data_ptr() + 4 * x0, 4 * X, src_dev.data_ptr() + 4 * x0, 4 * X,
-                                  4 * (x1 - x0), n * Y, 1, self.stream)
+            es = src_dev.element_size()
+            self.ops.copy2d_async(dst_host.data_ptr() + es * x0, es * X, src_dev.data_ptr() + es * x0, es * X,
+                                  es * (x1 - x0), n * Y, 1, self.stream)
         else:
             dst_host[:, :, x0:x1].copy_(src_dev[:, :, x0:x1])
 

@@ -222,17 +222,31 @@ class DeviceEngine:
                                                            _stream_ptr(torch)))
         return dst
 
-    def empty(self, shape):
-        return self.torch.empty(tuple(int(s) for s in shape), dtype=self.torch.float32, device=self.device)
+    def empty(self, shape, dtype=None):
+        dtype = self.torch.float32 if dtype is None else dtype
+        return self.torch.empty(tuple(int(s) for s in shape), dtype=dtype, device=self.device)
+
+    @staticmethod
+    def _same_dtype(src, dst, what):
+        if dst.dtype != src.dtype:
+            raise ValueError(f"{what} keeps the dtype ({src.dtype} -> {dst.dtype})")
 
     def copy3d(self, src, src_off, in_sa, in_sb, b0, bw, c0, cw, dst, dst_off, out_sa, out_sb, A, B, C):
         """dst[a*out_sa + b*out_sb + c] = src[a*in_sa + ((b0+b) % bw)*in_sb + (c0+c) % cw]  (element offsets/strides
-        into flat float32 buffers) -- the packing kernel of the multi-GPU re-slab."""
+        into flat buffers of one dtype) -- the packing kernel of the multi-GPU re-slab."""
         torch = self.torch
+        self._same_dtype(src, dst, "copy3d")
+        es = src.element_size()
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.fdn_copy3d(src.data_ptr() + 4 * int(src_off), int(in_sa), int(in_sb), int(b0), int(bw),
-                                           int(c0), int(cw), dst.data_ptr() + 4 * int(dst_off), int(out_sa),
-                                           int(out_sb), int(A), int(B), int(C), _stream_ptr(torch)))
+            if src.dtype == torch.float32:
+                _lib.check(self.lib.fdn_copy3d(src.data_ptr() + es * int(src_off), int(in_sa), int(in_sb), int(b0),
+                                               int(bw), int(c0), int(cw), dst.data_ptr() + es * int(dst_off),
+                                               int(out_sa), int(out_sb), int(A), int(B), int(C), _stream_ptr(torch)))
+            else:
+                _lib.check(self.lib.fdn_copy3d_typed(src.data_ptr() + es * int(src_off), dtype_code(src), int(in_sa),
+                                                     int(in_sb), int(b0), int(bw), int(c0), int(cw),
+                                                     dst.data_ptr() + es * int(dst_off), int(out_sa), int(out_sb),
+                                                     int(A), int(B), int(C), _stream_ptr(torch)))
 
     def copy2d_async(self, dst_ptr, dst_pitch, src_ptr, src_pitch, width_bytes, rows, direction, stream):
         """fdn_copy2d_async on a torch stream: direction 0 = host to device, 1 = device to host, 2 = on the device."""
@@ -243,10 +257,18 @@ class DeviceEngine:
     def transpose_strided(self, src, src_off, in_sn, in_sa, dst, dst_off, out_sn, out_sb, n, A, B):
         """dst[i*out_sn + b*out_sb + a] = src[i*in_sn + a*in_sa + b] -- the transposing unpack of the re-slab."""
         torch = self.torch
+        self._same_dtype(src, dst, "transpose_strided")
+        es = src.element_size()
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.fdn_transpose_strided(src.data_ptr() + 4 * int(src_off), int(in_sn), int(in_sa),
-                                                      dst.data_ptr() + 4 * int(dst_off), int(out_sn), int(out_sb),
-                                                      int(n), int(A), int(B), _stream_ptr(torch)))
+            if src.dtype == torch.float32:
+                _lib.check(self.lib.fdn_transpose_strided(src.data_ptr() + es * int(src_off), int(in_sn), int(in_sa),
+                                                          dst.data_ptr() + es * int(dst_off), int(out_sn), int(out_sb),
+                                                          int(n), int(A), int(B), _stream_ptr(torch)))
+            else:
+                _lib.check(self.lib.fdn_transpose_strided_typed(src.data_ptr() + es * int(src_off), dtype_code(src),
+                                                                int(in_sn), int(in_sa),
+                                                                dst.data_ptr() + es * int(dst_off), int(out_sn),
+                                                                int(out_sb), int(n), int(A), int(B), _stream_ptr(torch)))
 
     def filter_along_axis(self, vol, out, axis: int, kernel, flow: Optional[FlowParams], chunk: Optional[int] = None,
                           exact: bool = True, scratch=None):

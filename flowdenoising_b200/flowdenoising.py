@@ -484,8 +484,9 @@ class GaussianDenoising():
         return self._flow_params
 
     def _typed(self):
-        """True when the passes run in the volume's integer dtype (keep_dtype); raises ValueError for a combination
-        that is not supported rather than converting silently."""
+        """True when the passes run in the volume's integer dtype (keep_dtype), in core or streamed (memory maps,
+        several devices, volumes larger than the device); raises ValueError for a combination that is not supported
+        rather than converting silently."""
         dt = self.vol.dtype
         if not self.keep_dtype or (dt.kind == "f" and dt.itemsize >= 4):
             return False
@@ -495,15 +496,9 @@ class GaussianDenoising():
         if dt == np.int8 and self._flow() is not None:
             raise ValueError("keep_dtype: int8 volumes are supported without optical flow only (cv2.remap, which the "
                              "reference calls, rejects int8 images)")
-        if self.streaming or isinstance(self.vol, np.memmap) or self.border != "wrap" or \
-                (self.devices and len(self.devices) > 1):
-            raise ValueError("keep_dtype: streaming (memory maps, --border mean, --gpus > 1) is not supported for "
-                             "integer volumes")
-        eng = _get_engine()
-        free, _total = eng.torch.cuda.mem_get_info(eng.device)
-        # the volume, two intermediates and the result in the dtype, the float32 chunk accumulator in the workspace
-        if 4 * dt.itemsize * self.vol.size + (2 << 30) > 0.9 * free:
-            raise ValueError("keep_dtype: integer volumes larger than the device are not supported")
+        if self.border != "wrap":
+            raise ValueError("keep_dtype: streaming with --border mean is not supported for integer volumes (the "
+                             "reference defines no integer mean padding)")
         return True
 
     def _streaming_needed(self):
@@ -513,8 +508,10 @@ class GaussianDenoising():
             return True
         eng = _get_engine()
         free, _total = eng.torch.cuda.mem_get_info(eng.device)
-        # in core: the volume, two intermediates and the result as float32, plus a workspace worth having
-        return 4 * 4 * self.vol.size + (2 << 30) > 0.9 * free
+        # in core: the volume, two intermediates and the result in the pass dtype (float32, or the integer dtype of a
+        # typed volume, whose float32 chunk accumulator lives in the workspace), plus a workspace worth having
+        itemsize = self.vol.dtype.itemsize if self._typed() else 4
+        return 4 * itemsize * self.vol.size + (2 << 30) > 0.9 * free
 
     def _streamer(self):
         from .streaming import StreamingDenoiser
@@ -523,7 +520,7 @@ class GaussianDenoising():
         def report(slices):
             self._progress_done = done0[0] + slices
         sd = StreamingDenoiser(self._flow(), exact=self.exact, border=self.border, slab_slices=self.slab_slices,
-                               devices=self.devices, progress=report)
+                               devices=self.devices, progress=report, keep_dtype=self._typed())
         return sd, done0
 
     def _pass(self, axis, kernel):
@@ -531,7 +528,8 @@ class GaussianDenoising():
         torch = eng.torch
         kernel = np.asarray(kernel, dtype=np.float64)
         assert kernel.size % 2 != 0  # kernel.size must be odd (src/flowdenoising.py:309)
-        if self._typed():
+        typed = self._typed()
+        if typed and not self._streaming_needed():
             d_in = torch.from_numpy(np.ascontiguousarray(self.vol)).to(eng.device)
             d_out = torch.empty_like(d_in)
             self._begin_device_call()
@@ -541,7 +539,10 @@ class GaussianDenoising():
             return
         if self._streaming_needed():
             sd, done0 = self._streamer()
-            dst = self.filtered_vol if self.filtered_vol.dtype == np.float32 else np.empty(self.vol.shape, np.float32)
+            # the pass dtype (float32, or the typed volume's own), or float32: exact for the integers of a typed pass
+            pd = self.vol.dtype if typed else np.dtype(np.float32)
+            ok = self.filtered_vol.dtype in (pd, np.dtype(np.float32))
+            dst = self.filtered_vol if ok else np.empty(self.vol.shape, pd)
             sd.filter_axis(self.vol, dst, axis, kernel)
             if dst is not self.filtered_vol:
                 self.filtered_vol[...] = dst
@@ -653,7 +654,8 @@ class GaussianDenoising():
             assert np.asarray(k).size % 2 != 0
         ks = [np.asarray(k, np.float64) for k in kernels]
         Z, Y, X = (int(v) for v in self.vol.shape)
-        if self._typed():
+        typed = self._typed()
+        if typed and not self._streaming_needed():
             # the plain sequence: upload in the dtype, three typed passes, the ZY intermediate and the result home
             d_in = torch.from_numpy(np.ascontiguousarray(self.vol)).to(eng.device)
             self._begin_device_call()
@@ -664,16 +666,20 @@ class GaussianDenoising():
             return self.filtered_vol
         if self._streaming_needed():
             sd, done0 = self._streamer()
-            fv = self.filtered_vol if self.filtered_vol.dtype == np.float32 else np.empty(self.vol.shape, np.float32)
+            # typed: every pass truncates into the volume's dtype, so the intermediates are arrays of that dtype; the
+            # result may land in a float32 array (an output map), which holds these integers exactly
+            pd = self.vol.dtype if typed else np.dtype(np.float32)
+            ok = self.filtered_vol.dtype in (pd, np.dtype(np.float32))
+            fv = self.filtered_vol if ok else np.empty(self.vol.shape, pd)
             base = done0[0]
             zy, zyx = None, None
             # three passes with the reference's buffer roles: vol -> scratch -> vol (Z+Y) -> filtered_vol
-            writable = isinstance(self.vol, np.ndarray) and self.vol.dtype == np.float32 and self.vol.flags.writeable
-            scratch = np.empty(self.vol.shape, np.float32)
+            writable = isinstance(self.vol, np.ndarray) and self.vol.dtype == pd and self.vol.flags.writeable
+            scratch = np.empty(self.vol.shape, pd)
             mean = float(np.float32(np.mean(self.vol))) if self.border == "mean" else None
             sd.filter_axis(self.vol, scratch, 0, ks[0], mean)
             done0[0] = base + Z
-            zy = self.vol if writable else np.empty(self.vol.shape, np.float32)
+            zy = self.vol if writable else np.empty(self.vol.shape, pd)
             sd.filter_axis(scratch, zy, 1, ks[1], mean)
             done0[0] = base + Z + Y
             del scratch
@@ -875,8 +881,10 @@ def build_parser():
                         help="Filter an integer MRC volume (modes 0, 1, 6) in its own dtype with the reference's integer "
                              "arithmetic (integer remap, truncation after every pass), for bit-for-bit parity with "
                              "flowdenoising.py on integer input. Without it integer volumes are filtered as float32. "
-                             "TIFF input is float32 either way; the output file is float32 (MRC mode 2). Not with -m, "
-                             "--border mean or --gpus > 1; int8 (mode 0) only with --no_OF")
+                             "Works in core, with -m (the map stays in its dtype and streams through the device) and "
+                             "with --gpus N. TIFF input is float32 either way; the output file is float32 (MRC mode 2), "
+                             "which holds the integer result exactly. Not with --border mean; int8 (mode 0) only with "
+                             "--no_OF")
     parser.add_argument("--compat_zy_output", action="store_true",
                         help="Write the Z+Y intermediate like the reference CLI does (flowdenoising.py:520) "
                              "instead of the full Z+Y+X result")
@@ -932,7 +940,7 @@ def main(argv=None):
     logging.info(f"read \"{args.input}\" in {time.perf_counter() - time_0} seconds")
     mapped = isinstance(vol, np.memmap)
     if args.keep_dtype and vol.dtype.kind in "iu" and not mapped:
-        vol = np.ascontiguousarray(vol, dtype=vol.dtype.newbyteorder("="))      # (-m with it: ValueError in filter)
+        vol = np.ascontiguousarray(vol, dtype=vol.dtype.newbyteorder("="))      # (-m: the map keeps its dtype)
     elif args.keep_dtype and vol.dtype == np.float16:
         pass                                                                    # ValueError in filter
     elif not mapped:      # (-m: the volume stays in the file and streams through the device slab by slab)

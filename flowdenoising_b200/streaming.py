@@ -20,10 +20,16 @@ into pinned staging memory and uploaded on a copy stream and slab k-1 is downloa
 PCIe transfers and kernels overlap. Results are bit-identical to the in-core passes (same kernels, same inputs per
 slice); tests/test_gpu_streaming.py forces small slabs on toy volumes and demands equality.
 
+Typed mode (keep_dtype=True, an integer volume: uint8, int8, uint16 or int16): staging buffers, device slabs and the
+X pass's transposes are in the volume's dtype T, so nothing is cast while gathering and every transfer carries
+1 or 2 B/voxel. Each pass truncates into T (the reference's integer `filtered_vol`), so the intermediates of filter()
+are T arrays; the last pass may scatter into a float32 array, which holds integers of up to 16 bits exactly.
+
 Nothing here computes on the CPU: the host side only copies slabs.
 """
 from __future__ import annotations
 
+import ctypes as C
 from typing import Callable, List, Optional, Sequence
 
 import numpy as np
@@ -31,6 +37,19 @@ import numpy as np
 from . import _lib
 from ._lib import View
 from .engine import DeviceEngine, FlowParams
+
+
+_TYPED = tuple(np.dtype(t) for t in (np.uint8, np.int8, np.uint16, np.int16))
+
+
+def _torch_dtype(torch, dt):
+    return {np.dtype(np.uint8): torch.uint8, np.dtype(np.int8): torch.int8, np.dtype(np.uint16): torch.uint16,
+            np.dtype(np.int16): torch.int16}[np.dtype(dt)]
+
+
+def _lib_dtype(dt):
+    return {np.dtype(np.uint8): _lib.DTYPE_U8, np.dtype(np.int8): _lib.DTYPE_I8, np.dtype(np.uint16): _lib.DTYPE_U16,
+            np.dtype(np.int16): _lib.DTYPE_I16}[np.dtype(dt)]
 
 
 def _runs(lo: int, hi: int, n: int):
@@ -64,24 +83,28 @@ class _DeviceLane:
         self.dev_tmp = [None, None]     # X pass: transposed input / output
         self.jobs: List[dict] = []      # slabs in flight, oldest first
 
-    def buffers(self, slot, n_in_elems, n_out_elems, need_tmp):
+    def buffers(self, slot, n_in_elems, n_out_elems, need_tmp, dtype=None):
         torch = self.torch
+        dtype = torch.float32 if dtype is None else dtype
+
+        def stale(t, n):
+            return t is None or t.numel() < n or t.dtype != dtype
 
         def grow(lst, n, pinned):
-            if lst[slot] is None or lst[slot].numel() < n:
+            if stale(lst[slot], n):
                 lst[slot] = None
-                lst[slot] = (torch.empty(n, dtype=torch.float32, pin_memory=True) if pinned else
-                             torch.empty(n, dtype=torch.float32, device=self.device))
+                lst[slot] = (torch.empty(n, dtype=dtype, pin_memory=True) if pinned else
+                             torch.empty(n, dtype=dtype, device=self.device))
             return lst[slot]
         grow(self.pin_in, n_in_elems, True)
         grow(self.pin_out, n_out_elems, True)
         grow(self.dev_in, n_in_elems, False)
         grow(self.dev_out, n_out_elems, False)
         if need_tmp:
-            if self.dev_tmp[0] is None or self.dev_tmp[0].numel() < n_in_elems:
-                self.dev_tmp[0] = torch.empty(n_in_elems, dtype=torch.float32, device=self.device)
-            if self.dev_tmp[1] is None or self.dev_tmp[1].numel() < n_out_elems:
-                self.dev_tmp[1] = torch.empty(n_out_elems, dtype=torch.float32, device=self.device)
+            if stale(self.dev_tmp[0], n_in_elems):
+                self.dev_tmp[0] = torch.empty(n_in_elems, dtype=dtype, device=self.device)
+            if stale(self.dev_tmp[1], n_out_elems):
+                self.dev_tmp[1] = torch.empty(n_out_elems, dtype=dtype, device=self.device)
 
 
 class StreamingDenoiser:
@@ -89,13 +112,17 @@ class StreamingDenoiser:
 
     border: "wrap" (the reference, src/flowdenoising.py:312) or "mean" (the sequential variant's padding).
     slab_slices: output slices per slab (None: sized from `device_budget_bytes` / the free device memory).
-    devices: CUDA device indices to spread the slabs over (default: the current device)."""
+    devices: CUDA device indices to spread the slabs over (default: the current device).
+    keep_dtype: an integer volume runs the typed passes in its own dtype (see the module docstring); otherwise every
+    volume is filtered as float32."""
 
     def __init__(self, flow: Optional[FlowParams], exact: bool = True, border: str = "wrap",
                  slab_slices: Optional[int] = None, devices: Optional[Sequence[int]] = None,
-                 device_budget_bytes: Optional[int] = None, progress: Optional[Callable[[float], None]] = None):
+                 device_budget_bytes: Optional[int] = None, progress: Optional[Callable[[float], None]] = None,
+                 keep_dtype: bool = False):
         if border not in ("wrap", "mean"):
             raise ValueError("border must be 'wrap' or 'mean'")
+        self.keep_dtype = bool(keep_dtype)
         torch = _lib.require_cuda()
         self.torch = torch
         self.flow = flow
@@ -107,22 +134,35 @@ class StreamingDenoiser:
         devs = list(devices) if devices else [torch.cuda.current_device()]
         self.lanes = [_DeviceLane(f"cuda:{d}", None) for d in devs]
 
+    def pass_dtype(self, src):
+        """NumPy dtype the passes over `src` run in: its own for an integer volume in typed mode, float32 otherwise."""
+        dt = np.dtype(src.dtype)
+        if not self.keep_dtype or dt not in _TYPED:
+            return np.dtype(np.float32)
+        if self.border != "wrap":
+            raise ValueError("keep_dtype: streaming with --border mean is not supported for integer volumes (the "
+                             "reference defines no integer mean padding)")
+        return dt
+
     # ---------------------------------------------------------------------------------------------- slab sizing
-    def _slab_len(self, shape, axis, r):
+    def _slab_len(self, shape, axis, r, dtype=np.float32):
         if self.slab_slices:
             return max(1, int(self.slab_slices))
         torch = self.torch
         n = shape[axis]
-        per_slice = int(np.prod(shape)) // n * 4                     # bytes of one slice
         budget = self.device_budget_bytes
         if budget is None:
             free = min(torch.cuda.mem_get_info(l.device)[0] for l in self.lanes)
             budget = int(free * 0.8)
-        # per output slice: 2 x (input + output) slabs (+ transposes on the X pass) and the pass workspace (cached
-        # polynomial expansions 26.6 B/px, three flow buffers for both chain directions 48 B/px, stash 4 r B/px)
-        ws = (27 + 48 + 4 * r) / 4.0 if self.flow is not None else 0.0
-        cost = per_slice * (2 * 2 + (2 if axis == 2 else 0) + ws)
-        fixed = per_slice * 2 * r * (2 + 27 / 4.0)                   # halo slices: input copies + their expansions
+        if np.dtype(dtype) != np.float32:
+            cost, fixed = self._typed_slice_cost(shape, axis, r, np.dtype(dtype))
+        else:
+            per_slice = int(np.prod(shape)) // n * 4                 # bytes of one slice
+            # per output slice: 2 x (input + output) slabs (+ transposes on the X pass) and the pass workspace (cached
+            # polynomial expansions 26.6 B/px, three flow buffers for both chain directions 48 B/px, stash 4 r B/px)
+            ws = (27 + 48 + 4 * r) / 4.0 if self.flow is not None else 0.0
+            cost = per_slice * (2 * 2 + (2 if axis == 2 else 0) + ws)
+            fixed = per_slice * 2 * r * (2 + 27 / 4.0)               # halo slices: input copies + their expansions
         length = int((budget - fixed) // cost)
         if length < 1:
             raise _lib.FdnError("device budget too small for a one-slice slab of this volume")
@@ -130,6 +170,30 @@ class StreamingDenoiser:
         parts = max(len(self.lanes), -(-n // length))
         parts = -(-parts // len(self.lanes)) * len(self.lanes) if n >= len(self.lanes) else parts
         return max(1, -(-n // parts))
+
+    def _typed_slice_cost(self, shape, axis, r, dt):
+        """(bytes per output slice, fixed bytes) of a typed slab: 2 x (input + output) slabs in T (+ transposes on the
+        X pass) and the typed pass workspace, fdn_workspace_bytes_typed (stash in T, float32 chunk accumulator) at one
+        and two output slices."""
+        n = shape[axis]
+        px = int(np.prod(shape)) // n
+        per_slice = px * dt.itemsize
+        cost, fixed = per_slice * (2 * 2 + (2 if axis == 2 else 0)), per_slice * 2 * r * 2
+        if self.flow is not None:
+            H, W = [s for i, s in enumerate(shape) if i != axis]
+            ofp = self.flow.c_struct()
+            lib = _lib.load()
+
+            def ws(k):
+                v = View(k + 2 * r, k, r, 0, H, W, H * W, W, H * W, W)
+                nbytes = lib.fdn_workspace_bytes_typed(C.byref(v), 2 * r + 1, C.byref(ofp), k, _lib_dtype(dt))
+                if nbytes == 0:
+                    _lib.check(1)
+                return nbytes
+            w1, w2 = ws(1), ws(2)
+            cost += w2 - w1
+            fixed += max(0, 2 * w1 - w2)
+        return cost, fixed
 
     # ---------------------------------------------------------------------------------------------- host <-> staging
     def _gather(self, src, axis, lo, hi, dst, mean):
@@ -148,8 +212,13 @@ class StreamingDenoiser:
     # ---------------------------------------------------------------------------------------------- one pass
     def filter_axis(self, src, dst, axis: int, kernel, mean: Optional[float] = None):
         """dst = one pass of the reference's filter_along_{Z,Y,X} over the host volume `src` ([Z, Y, X], any dtype
-        NumPy can cast to float32; np.memmap welcome). `dst`: float32 host array / memmap of the same shape, != src."""
+        NumPy can cast to float32; np.memmap welcome). `dst`: float32 host array / memmap of the same shape, != src.
+        Typed mode on an integer `src`: the pass runs in src's dtype T and truncates into T; `dst` is a T array, or
+        float32 (exact for these integers)."""
         torch = self.torch
+        pd = self.pass_dtype(src)
+        if pd != np.float32 and np.dtype(dst.dtype) not in (pd, np.dtype(np.float32)):
+            raise ValueError(f"a typed pass over a {pd} volume writes {pd} or float32, not {dst.dtype}")
         kernel = np.ascontiguousarray(kernel, dtype=np.float64)
         if kernel.ndim != 1 or kernel.size % 2 == 0:
             raise ValueError("kernel.size must be odd")
@@ -163,7 +232,7 @@ class StreamingDenoiser:
         n = shape[axis]
         if self.border == "mean" and mean is None:
             mean = float(np.float32(np.mean(src)))
-        L = self._slab_len(shape, axis, r)
+        L = self._slab_len(shape, axis, r, pd)
         slabs = [(a, min(a + L, n)) for a in range(0, n, L)]
         done = 0
         for k, (a, b) in enumerate(slabs):
@@ -171,7 +240,7 @@ class StreamingDenoiser:
             if len(lane.jobs) == 2:
                 done += self._finish(lane, lane.jobs.pop(0), dst, axis)
                 self._report(done, n)
-            self._start(lane, src, axis, a, b, r, kernel, mean)
+            self._start(lane, src, axis, a, b, r, kernel, mean, pd)
         for lane in self.lanes:
             while lane.jobs:
                 done += self._finish(lane, lane.jobs.pop(0), dst, axis)
@@ -181,7 +250,7 @@ class StreamingDenoiser:
         if self.progress is not None:
             self.progress(done)
 
-    def _start(self, lane: _DeviceLane, src, axis, a, b, r, kernel, mean):
+    def _start(self, lane: _DeviceLane, src, axis, a, b, r, kernel, mean, pd=np.float32):
         torch = self.torch
         Z, Y, X = (int(s) for s in src.shape)
         nl = b - a
@@ -191,7 +260,7 @@ class StreamingDenoiser:
         n_in, n_out = int(np.prod(in_shape)), int(np.prod(out_shape))
         slot = 0 if not lane.jobs else 1 - lane.jobs[-1]["slot"]
         with torch.cuda.device(lane.device):
-            lane.buffers(slot, n_in, n_out, axis == 2)
+            lane.buffers(slot, n_in, n_out, axis == 2, None if pd == np.float32 else _torch_dtype(torch, pd))
             pin = lane.pin_in[slot][:n_in].view(in_shape)
             # the staging buffer may still be the source of the previous upload from this slot
             prev = getattr(lane, f"h2d_done_{slot}", None)
@@ -244,19 +313,21 @@ class StreamingDenoiser:
     # ---------------------------------------------------------------------------------------------- three passes
     def filter(self, vol, kernels, filtered_vol=None, scratch=None):
         """Z, Y, X passes (src/flowdenoising.py:285-290) of the host volume `vol`. Like the reference, `vol` ends up
-        holding the Z+Y intermediate and `filtered_vol` the Z+Y+X result; `scratch` (a float32 array / memmap of the
-        volume's shape) holds the Z result in between. `vol` must be writable float32 for the in-place semantics;
-        otherwise a float32 copy of the Z+Y result is returned as the first element."""
+        holding the Z+Y intermediate and `filtered_vol` the Z+Y+X result; `scratch` (an array / memmap of the volume's
+        shape in the pass dtype) holds the Z result in between. `vol` must be writable and of the pass dtype (float32;
+        in typed mode the integer volume's own) for the in-place semantics; otherwise a copy of the Z+Y result in the
+        pass dtype is returned as the first element. In typed mode `filtered_vol` may be float32."""
         shape = tuple(vol.shape)
+        pd = self.pass_dtype(vol)
         if scratch is None:
-            scratch = np.empty(shape, np.float32)
+            scratch = np.empty(shape, pd)
         if filtered_vol is None:
-            filtered_vol = np.empty(shape, np.float32)
+            filtered_vol = np.empty(shape, pd)
         # the sequential variant pads all three passes with the mean of the ORIGINAL volume (vol.mean(), :420-430)
         mean = float(np.float32(np.mean(vol))) if self.border == "mean" else None
         self.filter_axis(vol, scratch, 0, kernels[0], mean)
-        writable = isinstance(vol, np.ndarray) and vol.dtype == np.float32 and vol.flags.writeable
-        zy = vol if writable else np.empty(shape, np.float32)
+        writable = isinstance(vol, np.ndarray) and vol.dtype == pd and vol.flags.writeable
+        zy = vol if writable else np.empty(shape, pd)
         self.filter_axis(scratch, zy, 1, kernels[1], mean)
         self.filter_axis(zy, filtered_vol, 2, kernels[2], mean)
         return zy, filtered_vol

@@ -171,6 +171,13 @@ int fdn_transpose_strided(const float* d_in, int64_t in_sn, int64_t in_sa, float
                           int n, int A, int B, void* stream);
 int fdn_copy3d(const float* d_in, int64_t in_sa, int64_t in_sb, int b0, int b_wrap, int c0, int c_wrap, float* d_out,
                int64_t out_sa, int64_t out_sb, int A, int B, int C, void* stream);
+/* The same two on elements of any FDN_DTYPE_* (strides and offsets in elements): they move bits, so the signed types
+ * share the kernel of their size, and FDN_DTYPE_F32 forwards to the float32 entry points. A re-slab of a typed volume
+ * moves 1 or 2 B/voxel. An unknown dtype is rejected with FDN_ERR_INVALID. */
+int fdn_transpose_strided_typed(const void* d_in, int dtype, int64_t in_sn, int64_t in_sa, void* d_out, int64_t out_sn,
+                                int64_t out_sb, int n, int A, int B, void* stream);
+int fdn_copy3d_typed(const void* d_in, int dtype, int64_t in_sa, int64_t in_sb, int b0, int b_wrap, int c0, int c_wrap,
+                     void* d_out, int64_t out_sa, int64_t out_sb, int A, int B, int C, void* stream);
 
 /* Pitched copy on a stream (cudaMemcpy2DAsync): `rows` rows of `width_bytes`, direction 0 = host to device, 1 = device
  * to host, 2 = device to device. Plumbing of the plugin's staging: a range of columns of the result volume goes home
