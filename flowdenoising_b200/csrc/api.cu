@@ -271,7 +271,7 @@ static int make_plan(const fdn_view& v, int klen, const fdn_of_params& of, int c
     p->off_S1 = off; off += align_up(fl, 256);
     p->off_S2 = off; off += align_up(fl, 256);
     p->off_stash = off; off += align_up(esize * px * (size_t)p->r, 256);   // remapped forward neighbours
-    p->scratch_bytes = flow_iter_scratch_bytes(2 * chunk, v.H, v.W);  // level 0 is the largest
+    p->scratch_bytes = flow_iter_scratch_bytes(2 * chunk, p->g.nl + 1, p->g.hs, p->g.ws);   // every level of the pass
     p->off_scratch = off; off += align_up(p->scratch_bytes, 256);
     p->off_acc = off;
     if (esize != sizeof(float)) off += align_up(sizeof(float) * px, 256);
@@ -301,7 +301,8 @@ static int filter_axis_of(const T* d_in, T* d_out, const fdn_view& v, const doub
     float* S2 = reinterpret_cast<float*>(base + p.off_S2);
     T* stash = reinterpret_cast<T*>(base + p.off_stash);
     FlowScratch fs;
-    if ((rc = flow_scratch_make(base + p.off_scratch, p.scratch_bytes, 2 * p.chunk, H, W, &fs))) return rc;
+    if ((rc = flow_scratch_make(base + p.off_scratch, p.scratch_bytes, 2 * p.chunk, p.g.nl + 1, p.g.hs, p.g.ws, &fs)))
+        return rc;
     if ((rc = flow_iter_scratch_init(fs, st))) return rc;
     PolyConsts pc;
     prepare_poly_consts(of.poly_n, of.poly_sigma, &pc);
@@ -802,7 +803,7 @@ int fdn_polyexp(const float* d_img, int n, int h, int w, int poly_n, double poly
 
 size_t fdn_polyexp_floats(int h, int w) { return R_image_floats(h, w); }
 
-size_t fdn_flow_iteration_scratch_bytes(int n, int h, int w) { return flow_iter_scratch_bytes(n, h, w); }
+size_t fdn_flow_iteration_scratch_bytes(int n, int h, int w) { return flow_iter_scratch_bytes(n, 1, &h, &w); }
 
 void fdn_set_flow_iter_variant(int variant) { set_flow_iter_variant(variant); }
 
@@ -816,7 +817,7 @@ int fdn_flow_iterations(const float* d_R0, const float* d_R1, float* d_flow, flo
     int rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     FlowScratch fs;
-    if ((rc = flow_scratch_make(d_scratch, scratch_bytes, n, h, w, &fs))) return rc;
+    if ((rc = flow_scratch_make(d_scratch, scratch_bytes, n, 1, &h, &w, &fs))) return rc;
     if ((rc = flow_iter_scratch_init(fs, st))) return rc;
     const ptrdiff_t delta = d_R1 - d_R0;
     FDN_CHECK_ARG(delta % stride == 0, "R1 - R0 must be a multiple of one image (fdn_polyexp_floats(h, w))");
@@ -869,7 +870,8 @@ size_t fdn_farneback_workspace_bytes(int n, int H, int W, const fdn_of_params* o
     Geometry g;
     if (make_geometry(H, W, of->levels, &g)) return 0;
     const size_t fl = align_up(sizeof(float) * 2 * (size_t)n * H * W, 256);
-    return align_up(sizeof(float) * g.R_slot * 2 * (size_t)n, 256) + 2 * fl + align_up(flow_iter_scratch_bytes(n, H, W), 256);
+    return align_up(sizeof(float) * g.R_slot * 2 * (size_t)n, 256) + 2 * fl +
+           align_up(flow_iter_scratch_bytes(n, g.nl + 1, g.hs, g.ws), 256);
 }
 
 int fdn_farneback(const float* d_prev, const float* d_next, float* d_flow, int n, int H, int W,
@@ -892,7 +894,9 @@ int fdn_farneback(const float* d_prev, const float* d_next, float* d_flow, int n
     float* S1 = reinterpret_cast<float*>(base + align_up(sizeof(float) * g.R_slot * 2 * (size_t)n, 256));
     float* S2 = reinterpret_cast<float*>(reinterpret_cast<char*>(S1) + fl);
     FlowScratch fs;
-    if ((rc = flow_scratch_make(reinterpret_cast<char*>(S2) + fl, flow_iter_scratch_bytes(n, H, W), n, H, W, &fs))) return rc;
+    if ((rc = flow_scratch_make(reinterpret_cast<char*>(S2) + fl, flow_iter_scratch_bytes(n, g.nl + 1, g.hs, g.ws), n,
+                                g.nl + 1, g.hs, g.ws, &fs)))
+        return rc;
     if ((rc = flow_iter_scratch_init(fs, st))) return rc;
     PolyConsts pc;
     prepare_poly_consts(of->poly_n, of->poly_sigma, &pc);

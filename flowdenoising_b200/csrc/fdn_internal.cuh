@@ -119,15 +119,20 @@ int launch_polyexp(const float* img, int64_t img_stride, float* R, int64_t R_str
 // floats one polynomial-expansion image occupies: [h*w] float4 (channels 0-3) + [h*w] float (channel 4), padded to 16 B
 static inline size_t R_image_floats(int h, int w) { size_t p = (size_t)h * w; return 4 * p + ((p + 3) / 4) * 4; }
 // Scratch of the flow iteration (counters, strip-to-strip carries). Every offset depends only on the CAPACITY the
-// scratch was sized for (pairs, level-0 image size), never on the size of an individual launch.
+// scratch was sized for (pairs, and the largest strip count and strips x rows over the levels it serves), never on
+// the size of an individual launch.
 struct FlowScratch {
     char* base;
     size_t bytes;
-    int cap_n, H, W;
+    int cap_n, H, W;                    // largest level height and width
+    int flag_strips;                    // k_flow_iter strips per pair
+    int64_t packet_rows, carry_rows;    // strips x rows per pair: k_flow_iter_ws packets, k_flow_iter carries
     size_t off_done, off_flags, off_packets, off_carry;
 };
-size_t flow_iter_scratch_bytes(int cap_n, int H, int W);
-int flow_scratch_make(void* scratch, size_t bytes, int cap_n, int H, int W, FlowScratch* fs);   // layout only
+// levels k < nlev of hs[k] x ws[k] pixels (one level: nlev = 1)
+size_t flow_iter_scratch_bytes(int cap_n, int nlev, const int* hs, const int* ws);
+int flow_scratch_make(void* scratch, size_t bytes, int cap_n, int nlev, const int* hs, const int* ws,
+                      FlowScratch* fs);                                                           // layout only
 int flow_iter_scratch_init(const FlowScratch& fs, cudaStream_t st);                              // zero-fill
 // `iters` Farneback iterations of one pyramid level for n image pairs: cur -> ... rotating through {cur, a, b}
 // (iteration i reads bufs[i % 3] and writes bufs[(i + 1) % 3]); *result = the buffer holding the last output.

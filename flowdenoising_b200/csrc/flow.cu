@@ -946,7 +946,6 @@ k_flow_iter_ws(WsArgs wa)
 static std::atomic<unsigned long long> g_flow_epoch{1};
 static std::atomic<int> g_flow_variant{1};
 void set_flow_iter_variant(int v) { g_flow_variant.store(v ? 1 : 0); }
-#define FDN_MAX_STRIPS 64
 
 static int strip_width(int w) { return w > 96 ? 128 : 32; }   // k_flow_iter
 
@@ -979,24 +978,34 @@ static size_t align256(size_t v) { return (v + 255) / 256 * 256; }
 // Scratch layout (offsets depend on the capacity only, see FlowScratch):
 //   [ctl: tickets taken, warps / blocks finished]                                    256 B, zero between launches
 //   [done: FDN_WS_MAX_ITERS x cap_n counters of k_flow_iter_ws]                       zero between launches
-//   [flags: cap_n x FDN_MAX_STRIPS epochs of k_flow_iter]                             only ever grow
-//   [packets of k_flow_iter_ws: cap_n x strips x H x 5 tagged 16-byte pairs]
-//   [carries of k_flow_iter:    cap_n x strips x H x 5 doubles]
-// The two carry areas are disjoint, so a level run by one kernel never writes where the other kernel polls at
-// another level (a plain double must never be mistaken for a tagged packet). A smaller launch (coarser level, last
-// chunk of a pass) uses a prefix of each area.
-int flow_scratch_make(void* scratch, size_t bytes, int cap_n, int H, int W, FlowScratch* fs)
+//   [flags: cap_n x strips epochs of k_flow_iter]                                     only ever grow
+//   [packets of k_flow_iter_ws: cap_n x strips x h x 5 tagged 16-byte pairs]
+//   [carries of k_flow_iter:    cap_n x strips x h x 5 doubles]
+// Each area holds the largest of the nlev levels (hs[k] x ws[k]) it may serve. That is not always level 0: a
+// narrower level can need more strips (97..128 px: 1 strip of k_flow_iter, 48..64 px: 2), and cvRound rounds an odd
+// height up (67 rows -> 34). The two carry areas are disjoint, so a level run by one kernel never writes where the
+// other kernel polls at another level (a plain double must never be mistaken for a tagged packet). A smaller launch
+// (coarser level, last chunk of a pass) uses a prefix of each area.
+int flow_scratch_make(void* scratch, size_t bytes, int cap_n, int nlev, const int* hs, const int* ws, FlowScratch* fs)
 {
     fs->base = static_cast<char*>(scratch);
     fs->bytes = bytes;
-    fs->cap_n = cap_n; fs->H = H; fs->W = W;
+    fs->cap_n = cap_n; fs->H = 0; fs->W = 0;
+    fs->flag_strips = 0; fs->packet_rows = 0; fs->carry_rows = 0;
+    for (int k = 0; k < nlev; k++) {
+        const int h = hs[k], w = ws[k];
+        const int strips = (int)cdiv(w, strip_width(w));
+        if (h > fs->H) fs->H = h;
+        if (w > fs->W) fs->W = w;
+        if (strips > fs->flag_strips) fs->flag_strips = strips;
+        if ((int64_t)ws_strips_max(w) * h > fs->packet_rows) fs->packet_rows = (int64_t)ws_strips_max(w) * h;
+        if ((int64_t)strips * h > fs->carry_rows) fs->carry_rows = (int64_t)strips * h;
+    }
     size_t off = 256;
     fs->off_done = off;    off += align256(sizeof(unsigned) * FDN_WS_MAX_ITERS * (size_t)cap_n);
-    fs->off_flags = off;   off += align256(sizeof(unsigned long long) * (size_t)cap_n * FDN_MAX_STRIPS);
-    fs->off_packets = off;
-    off += align256(sizeof(ulonglong2) * 5 * (size_t)cap_n * (size_t)ws_strips_max(W) * H);
-    fs->off_carry = off;
-    off += align256(sizeof(double) * 5 * (size_t)cap_n * (size_t)cdiv(W, strip_width(W)) * H);
+    fs->off_flags = off;   off += align256(sizeof(unsigned long long) * (size_t)cap_n * fs->flag_strips);
+    fs->off_packets = off; off += align256(sizeof(ulonglong2) * 5 * (size_t)cap_n * (size_t)fs->packet_rows);
+    fs->off_carry = off;   off += align256(sizeof(double) * 5 * (size_t)cap_n * (size_t)fs->carry_rows);
     if (scratch && bytes < off) {
         set_error("flow iteration scratch too small: need %zu bytes, got %zu", off, bytes);
         return FDN_ERR_WORKSPACE;
@@ -1005,10 +1014,10 @@ int flow_scratch_make(void* scratch, size_t bytes, int cap_n, int H, int W, Flow
     return FDN_OK;
 }
 
-size_t flow_iter_scratch_bytes(int cap_n, int H, int W)
+size_t flow_iter_scratch_bytes(int cap_n, int nlev, const int* hs, const int* ws)
 {
     FlowScratch fs;
-    flow_scratch_make(nullptr, 0, cap_n, H, W, &fs);
+    flow_scratch_make(nullptr, 0, cap_n, nlev, hs, ws, &fs);
     return fs.bytes;
 }
 
@@ -1058,7 +1067,9 @@ static int launch_flow_iter_strip(const float* R, int64_t R_stride, SlotMap map0
     const int TR = (wide && m == 2) ? 6 : 4;
     a.strips = (int)cdiv(w, CW);
     a.LS = tile_line_stride(CW, m);
-    FDN_CHECK_ARG(a.strips <= FDN_MAX_STRIPS, "image too wide (%d strips)", a.strips);
+    FDN_CHECK_ARG(a.strips <= fs.flag_strips && (int64_t)a.strips * h <= fs.carry_rows,
+                  "flow iteration scratch was not sized for a %d x %d level", h, w);
+    FDN_CHECK_ARG((int64_t)n * a.strips < (1ll << 31), "too many image pairs in one launch");
     a.ctl = reinterpret_cast<unsigned*>(fs.base);
     a.flags = reinterpret_cast<unsigned long long*>(fs.base + fs.off_flags);
     a.carry = reinterpret_cast<double*>(fs.base + fs.off_carry);
@@ -1114,7 +1125,6 @@ int launch_flow_level(const float* R, int64_t R_stride, SlotMap map0, SlotMap ma
     FDN_CHECK_ARG((int64_t)h * w < (1ll << 28), "level image too large");
     FDN_CHECK_ARG(n >= 1 && n <= fs.cap_n && h <= fs.H && w <= fs.W, "flow iteration scratch was sized for %d pairs of %d x %d",
                   fs.cap_n, fs.H, fs.W);
-    FDN_CHECK_ARG((int64_t)n * FDN_MAX_STRIPS * FDN_WS_MAX_ITERS < (1ll << 31), "too many image pairs in one launch");
     float* bufs[3] = {cur, bufa, bufb};
     const int m = winsize / 2;
     // warp-specialised variant (default for winsize 5 on images that are not tiny)
@@ -1136,7 +1146,9 @@ int launch_flow_level(const float* R, int64_t R_stride, SlotMap map0, SlotMap ma
     wa.scale = 1. / ((double)winsize * winsize);
     wa.CW = ws_strip_width(w, m == 2 ? WsCfg2::CWMAX : WsCfg4::CWMAX);
     wa.strips = (int)cdiv(w, wa.CW);
-    FDN_CHECK_ARG(wa.strips <= FDN_MAX_STRIPS, "image too wide (%d strips)", wa.strips);
+    FDN_CHECK_ARG((int64_t)wa.strips * h <= fs.packet_rows, "flow iteration scratch was not sized for a %d x %d level",
+                  h, w);
+    FDN_CHECK_ARG((int64_t)n * wa.strips * FDN_WS_MAX_ITERS < (1ll << 31), "too many image pairs in one launch");
     wa.ctl = reinterpret_cast<unsigned*>(fs.base);
     wa.done = reinterpret_cast<unsigned*>(fs.base + fs.off_done);
     wa.packets = reinterpret_cast<ulonglong2*>(fs.base + fs.off_packets);

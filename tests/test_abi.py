@@ -51,7 +51,8 @@ def test_bad_arguments_are_reported_not_crashed():
         _lib.check(rc)
 
 
-def test_workspace_grows_with_chunk():
+def test_workspace_layout_grows_with_chunk():
+    """The exact pass workspace, its flow-iteration flags sized by the real strip count (not a fixed 64 per pair)."""
     lib = _lib.load()
     v = _lib.View(64, 64, 0, 1, 256, 256, 65536, 256, 65536, 256)
     p = _lib.OfParams(3, 5, 3, 5, 1.2, 1)
@@ -62,10 +63,10 @@ def test_workspace_grows_with_chunk():
     # together: 3 flow buffers of 2 * 64 pairs; the remapped forward neighbours wait in a stash of r = 8 chunk volumes;
     # + the scratch of the flow iteration for 128 pairs: ticket / finish counters, 3 * 128 dependency counters, the
     # flags + carries of the strip kernel (2 strips of 128 columns per image) and the carry packets of the
-    # warp-specialised kernel (3 strips of <= 120 columns, 16 bytes per carry)
+    # warp-specialised kernel (3 strips of <= 120 columns, 16 bytes per carry), all sized by level 0, the largest here
     R = 64 * 5 * (256 * 256 + 128 * 128 + 64 * 64 + 32 * 32) * 4
     flows = 3 * (128 * 256 * 256 * 2 * 4)
     stash = 8 * 64 * 256 * 256 * 4
     al = lambda v: (v + 255) // 256 * 256
-    scratch = 256 + al(3 * 128 * 4) + 128 * 64 * 8 + 128 * 3 * 256 * 5 * 16 + 128 * 2 * 256 * 5 * 8
+    scratch = 256 + al(3 * 128 * 4) + 128 * 2 * 8 + 128 * 3 * 256 * 5 * 16 + 128 * 2 * 256 * 5 * 8
     assert b == R + flows + stash + scratch
