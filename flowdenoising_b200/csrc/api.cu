@@ -245,6 +245,8 @@ static int make_plan(const fdn_view& v, int klen, const fdn_of_params& of, int c
 {
     int rc;
     FDN_CHECK_ARG(klen >= 1 && (klen & 1), "kernel length must be odd (src/flowdenoising.py:309)");
+    // checked here, before the first launch of the pass: the centre / forward taps (launch_acc_finish) take r <= 128
+    FDN_CHECK_ARG(klen <= FDN_MAX_KLEN, "kernel length %d unsupported (<= %d, sigma < 32.125)", klen, FDN_MAX_KLEN);
     FDN_CHECK_ARG(v.n_in >= 1 && v.n_out >= 1 && v.H >= 1 && v.W >= 1, "empty view");
     p->r = klen / 2;
     if (v.periodic) {
@@ -492,7 +494,10 @@ int fdn_gaussian_kernel(double sigma, double* taps, int cap)
     // scipy.ndimage._filters._gaussian_kernel1d(sigma, 0, radius=int(4*sigma+0.5)), which is what the reference's
     // delta-response loop (src/flowdenoising.py:34-45) returns after trimming the two exact zeros:
     // phi = exp(-0.5 / sigma^2 * x^2); phi / phi.sum()
-    if (!(sigma > 0)) { set_error("sigma must be > 0"); return 0; }
+    // with the C library's exp, which differs from NumPy's in the last bit for some arguments (include/fdn_b200.h); the
+    // Python package computes the taps with NumPy instead (engine.gaussian_kernel)
+    // (the upper bound keeps int(4 * sigma + 0.5) and the tap count inside int: infinity used to reach that cast)
+    if (!(sigma > 0 && sigma <= 1e8)) { set_error("sigma must be > 0 and at most 1e8"); return 0; }
     const int r = (int)(4.0 * sigma + 0.5);
     const int n = 2 * r + 1;
     if (n > cap || !taps) return -n;

@@ -38,8 +38,7 @@
 
 namespace fdn {
 
-#define FDN_MAX_KLEN 257
-struct Taps64 {
+struct Taps64 {   // FDN_MAX_KLEN: include/fdn_b200.h
     int klen;
     double k[FDN_MAX_KLEN];
 };

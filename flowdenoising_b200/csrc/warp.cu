@@ -248,6 +248,7 @@ int launch_warp_pair(const T* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_map, 
 }
 
 #define FDN_MAX_R 128
+static_assert(2 * FDN_MAX_R + 1 == FDN_MAX_KLEN, "k_acc_finish must take every kernel make_plan accepts");
 struct FinishTaps {
     double k[FDN_MAX_R + 1];   // centre, +1, ..., +r
 };

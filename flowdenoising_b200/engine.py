@@ -11,6 +11,7 @@ float32 accumulation, truncating store); int8 without optical flow only, like cv
 from __future__ import annotations
 
 import ctypes as C
+import math
 from dataclasses import dataclass
 from typing import Optional, Sequence
 
@@ -46,13 +47,19 @@ class FlowParams:
 
 
 def gaussian_kernel(sigma: float) -> np.ndarray:
-    """get_gaussian_kernel (src/flowdenoising.py:34-45): float64 taps, length 2*int(4*sigma+0.5)+1."""
-    lib = _lib.load()
-    buf = (C.c_double * 4096)()
-    n = lib.fdn_gaussian_kernel(float(sigma), buf, 4096)
-    if n <= 0:
+    """get_gaussian_kernel (src/flowdenoising.py:34-45): float64 taps, length 2*int(4*sigma+0.5)+1.
+
+    The reference's loop returns SciPy's kernel, scipy.ndimage._filters._gaussian_kernel1d(sigma, 0,
+    int(4*sigma+0.5)). It is computed here the way SciPy computes it, with NumPy's exp and NumPy's pairwise sum: the C
+    library's exp (fdn_gaussian_kernel) differs from NumPy's in the last bit for some arguments (exp(-0.125), taps 7
+    and 9 of sigma = 2), and the filter would then not be the reference's."""
+    s = float(sigma)
+    r = int(4 * s + 0.5) if math.isfinite(s) else 0
+    if not (s > 0 and math.isfinite(s)) or 2 * r + 1 > 4096:
         raise ValueError(f"cannot build a Gaussian kernel for sigma={sigma}")
-    return np.frombuffer(buf, dtype=np.float64, count=n).copy()
+    x = np.arange(-r, r + 1)
+    phi = np.exp(-0.5 / (s * s) * x ** 2)
+    return phi / phi.sum()
 
 
 def level_geometry(H: int, W: int, levels: int):

@@ -44,6 +44,10 @@ extern "C" {
 #define FDN_ERR_WORKSPACE 3 /* workspace too small */
 
 #define FDN_MAX_LEVELS 16
+/* Longest kernel a pass accepts (radius 128): the Gaussian of sigma < 32.125. Every pass entry point (with and
+ * without optical flow, float32 and typed) rejects a longer one with FDN_ERR_INVALID before it launches anything, and
+ * fdn_workspace_bytes(_typed) returns 0 for it. */
+#define FDN_MAX_KLEN 257
 
 /* fdn_of_params.flags: OpenCV's OPTFLOW_FARNEBACK_GAUSSIAN (same value). The matrices of the displacement update are
  * smoothed by a separable Gaussian window (2m+1 taps, m = winsize/2, sigma = 0.3 m) instead of the winsize x winsize
@@ -109,8 +113,11 @@ int fdn_profile_record_count(void);
 int fdn_profile_record(int i, int* id, int* n, int* h, int* w, double* ms, double* algorithmic_bytes);
 
 /* ---- host-side helpers ---- */
-/* get_gaussian_kernel (src/flowdenoising.py:34-45): writes 2*int(4*sigma+0.5)+1 float64 taps, returns the
- * count (or -needed if cap is too small). */
+/* get_gaussian_kernel (src/flowdenoising.py:34-45) for C callers: writes 2*int(4*sigma+0.5)+1 float64 taps, returns
+ * the count (-needed if cap is too small; 0 unless 0 < sigma <= 1e8). SciPy's formula and NumPy's summation order, but the C library's exp:
+ * NumPy's exp differs from it in the last bit for some arguments, so a tap may differ from the reference's (SciPy's)
+ * by a few ulp. The Python package computes the taps with NumPy (engine.gaussian_kernel) and equals SciPy bit for
+ * bit; a C caller who needs the reference's exact taps should take them from SciPy. */
 int fdn_gaussian_kernel(double sigma, double* taps, int cap);
 /* Pyramid geometry (OpenCV level cropping, SURVEY App. A.0): returns the number of EXTRA levels run (nl) and
  * fills hs/ws/ksz/sigma[0..nl]. Any output pointer may be NULL. */
@@ -127,7 +134,9 @@ int fdn_filter_axis(const float* d_in, float* d_out, const fdn_view* view, const
                     const fdn_of_params* of, int chunk, void* d_workspace, size_t workspace_bytes, void* stream);
 
 /* No-OF pass only, selectable arithmetic: exact != 0 reproduces NumPy's per-tap
- * float32(float64(acc) + float64(v)*k) bit for bit; exact == 0 uses float32 FMA (<= ~2 ulp, HBM-bound). */
+ * float32(float64(acc) + float64(v)*k) bit for bit; exact == 0 uses float32 FMA (HBM-bound): within 4 ulp of the exact
+ * mode for Gaussian taps of any length on 8-bit-like data, within (klen + 2) 2^-24 sum |k_i| |v_i| of the float64 sum for
+ * any taps. klen <= FDN_MAX_KLEN. */
 int fdn_gauss_axis(const float* d_in, float* d_out, const fdn_view* view, const double* kernel, int klen,
                    int exact, void* stream);
 /* Plain separable Gaussian along the contiguous x axis of a dense [n][W] array (X pass without transposes),

@@ -53,30 +53,8 @@ static inline int reflect101(int p, int len)
     return p;
 }
 
-/* ------------------------------------------------------------------------------------------
- * a1: get_gaussian_kernel(sigma)  (src/flowdenoising.py:34-45).
- * The reference grows a delta until scipy.ndimage.gaussian_filter1d shows >= 2 exact zeros and
- * returns coeffs[1:-1]; that is SciPy's own kernel with radius r = int(4*sigma + 0.5):
- * w[j] = exp(-0.5*j^2/sigma^2) / sum  (scipy/ndimage/_filters.py _gaussian_kernel1d).
- * Returns the number of taps (2r+1); out must hold them.
- * ------------------------------------------------------------------------------------------ */
-FDO_API int fdo_gaussian_kernel(double sigma, double* out, int cap)
-{
-    int r = (int)(4.0 * sigma + 0.5);
-    int n = 2 * r + 1;
-    if (n > cap) return -n;
-    double sigma2 = sigma * sigma;
-    double s = 0.0;
-    for (int j = -r; j <= r; j++) {
-        double x = (double)j;
-        out[j + r] = exp(-0.5 / sigma2 * (x * x));
-    }
-    /* numpy sum() is pairwise for n >= 8 blocks of 8..., for these short vectors (n<128) it is a
-       plain unrolled-by-8 partial-sum scheme; tests pin the result against scipy to 1 ulp. */
-    for (int j = 0; j < n; j++) s += out[j];
-    for (int j = 0; j < n; j++) out[j] /= s;
-    return n;
-}
+/* (a1, get_gaussian_kernel, is the reference's own SciPy loop in fd_oracle.py: NumPy's exp is not the C
+ * library's in the last bit, so a C restatement of the taps would not be the reference's taps.) */
 
 /* ------------------------------------------------------------------------------------------
  * cv::getGaussianKernel(ksz, sigma, CV_32F): double taps, normalised, stored as float.

@@ -58,7 +58,6 @@ def lib():
     if _lib is None:
         build()
         _lib = C.CDLL(_LIB_PATH)
-        _lib.fdo_gaussian_kernel.restype = C.c_int
         _lib.fdo_level_geometry.restype = C.c_int
         _lib.fdo_farneback.restype = C.c_int
     return _lib
@@ -75,15 +74,6 @@ def _f32(a):
 # ----------------------------------------------------------------------------------------------
 # Layer 1: C restatement, stage by stage
 # ----------------------------------------------------------------------------------------------
-def gaussian_kernel(sigma: float) -> np.ndarray:
-    """a1: get_gaussian_kernel (src/flowdenoising.py:34-45) in closed form."""
-    out = np.zeros(4096, np.float64)
-    n = lib().fdo_gaussian_kernel(C.c_double(sigma), _p(out, _f64p), C.c_int(out.size))
-    if n < 0:
-        raise ValueError("sigma too large")
-    return out[:n].copy()
-
-
 def gauss_blur(img, ksz, sigma):
     img = _f32(img)
     out = np.empty_like(img)
@@ -208,8 +198,18 @@ def flow_axis_c(vol, axis, kernel, levels=OF_LEVELS, winsize=OF_WINDOW_SIZE, ite
 # Layer 2: the reference's driver, restated (cv2 backend = what the reference executes)
 # ----------------------------------------------------------------------------------------------
 def get_gaussian_kernel(sigma=1.0):
-    """src/flowdenoising.py:34-45 (closed form; tests pin it against the SciPy-driven original)."""
-    return gaussian_kernel(float(sigma))
+    """src/flowdenoising.py:34-45, the reference's own loop: grow a delta until scipy.ndimage.gaussian_filter1d
+    leaves at least two exact zeros, return the response without its two ends (SciPy's kernel, computed by SciPy)."""
+    import scipy.ndimage
+    number_of_coeffs = 3
+    number_of_zeros = 0
+    while number_of_zeros < 2:
+        delta = np.zeros(number_of_coeffs)
+        delta[delta.size // 2] = 1
+        coeffs = scipy.ndimage.gaussian_filter1d(delta, sigma=sigma)
+        number_of_zeros = coeffs.size - np.count_nonzero(coeffs)
+        number_of_coeffs += 1
+    return coeffs[1:-1]
 
 
 def warp_slice(reference, flow):

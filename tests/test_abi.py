@@ -28,7 +28,7 @@ def test_header_symbols_exported():
 def test_gaussian_kernel_matches_reference(golden):
     g = golden("kernels.npz")
     for s in g["sigmas"]:
-        np.testing.assert_allclose(engine.gaussian_kernel(float(s)), g[f"k_{s}"], rtol=4e-16, atol=0)
+        assert np.array_equal(engine.gaussian_kernel(float(s)), g[f"k_{s}"]), s
     with pytest.raises(ValueError):
         engine.gaussian_kernel(0.0)
 
@@ -49,6 +49,42 @@ def test_bad_arguments_are_reported_not_crashed():
     assert lib.fdn_workspace_bytes(C.byref(v), 3, C.byref(p), 0) == 0 and b"winsize" in lib.fdn_last_error()
     with pytest.raises(ValueError):
         _lib.check(rc)
+
+
+@pytest.mark.parametrize("klen", [259, 261, 4095])
+def test_kernel_longer_than_257_taps_is_rejected_before_any_launch(klen):
+    """FDN_MAX_KLEN = 257 (sigma < 32.125). Every pass entry point refuses a longer kernel before it enqueues anything:
+    the device pointers below are never dereferenced and no CUDA call is made (no GPU here)."""
+    lib = _lib.load()
+    k = np.full(klen, 1.0 / klen)
+    kp = k.ctypes.data_as(C.POINTER(C.c_double))
+    v =_lib.View(300, 300, 0, 1, 16, 16, 256, 16, 256, 16)
+    of = _lib.OfParams(3, 5, 3, 5, 1.2, 1, 0)
+    # optical flow: the workspace query and the pass itself
+    assert lib.fdn_workspace_bytes(C.byref(v), 257, C.byref(of), 0) > 0
+    assert lib.fdn_workspace_bytes(C.byref(v), klen, C.byref(of), 0) == 0
+    assert b"257" in lib.fdn_last_error()
+    for dt in (_lib.DTYPE_U8, _lib.DTYPE_U16, _lib.DTYPE_I16):
+        assert lib.fdn_workspace_bytes_typed(C.byref(v), 257, C.byref(of), 0, dt) > 0
+        assert lib.fdn_workspace_bytes_typed(C.byref(v), klen, C.byref(of), 0, dt) == 0
+    rc = lib.fdn_filter_axis(16, 16, C.byref(v), kp, klen, C.byref(of), 0, 16, 1 << 40, None)
+    assert rc == 1 and b"257" in lib.fdn_last_error()
+    for dt in (_lib.DTYPE_F32, _lib.DTYPE_U8, _lib.DTYPE_U16, _lib.DTYPE_I16):
+        rc = lib.fdn_filter_axis_typed(16, 16, dt, C.byref(v), kp, klen, C.byref(of), 0, 16, 1 << 40, None)
+        assert rc == 1 and b"257" in lib.fdn_last_error(), dt
+    # without optical flow: the strided-axis and the row passes, float32 and typed, both arithmetic modes
+    for exact in (1, 0):
+        assert lib.fdn_gauss_axis(16, 16, C.byref(v), kp, klen, exact, None) == 1
+        assert b"257" in lib.fdn_last_error()
+        assert lib.fdn_gauss_rows(16, 16, 300 * 16, 16, kp, klen, exact, None) == 1
+        assert b"257" in lib.fdn_last_error()
+    assert lib.fdn_filter_axis(16, 16, C.byref(v), kp, klen, None, 0, None, 0, None) == 1
+    for dt in (_lib.DTYPE_U8, _lib.DTYPE_I8, _lib.DTYPE_U16, _lib.DTYPE_I16):
+        assert lib.fdn_gauss_axis_typed(16, 16, dt, C.byref(v), kp, klen, 1, None) == 1
+        assert b"257" in lib.fdn_last_error()
+        assert lib.fdn_gauss_rows_typed(16, 16, dt, 300 * 16, 16, kp, klen, 1, None) == 1
+        assert b"257" in lib.fdn_last_error()
+        assert lib.fdn_filter_axis_typed(16, 16, dt, C.byref(v), kp, klen, None, 0, None, 0, None) == 1
 
 
 def test_workspace_layout_grows_with_chunk():
