@@ -66,6 +66,11 @@ SIGNATURES = {
     "fdn_gauss_rows": (C.c_int, [c_f32p, c_f32p, c_i64, C.c_int, C.POINTER(C.c_double), C.c_int, C.c_int,
                                  C.c_void_p]),
     "fdn_transpose_yx": (C.c_int, [c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "fdn_workspace_bytes_batch": (C.c_size_t, [C.POINTER(View), C.c_int, C.c_int, C.POINTER(OfParams)]),
+    "fdn_filter_axis_batch": (C.c_int, [c_f32p, c_f32p, C.POINTER(View), C.c_int, c_i64, c_i64, C.POINTER(C.c_double),
+                                        C.c_int, C.POINTER(OfParams), C.c_void_p, C.c_size_t, C.c_void_p]),
+    "fdn_gauss_axis_batch": (C.c_int, [c_f32p, c_f32p, C.POINTER(View), C.c_int, c_i64, c_i64, C.POINTER(C.c_double),
+                                       C.c_int, C.c_int, C.c_void_p]),
     "fdn_transpose_strided": (C.c_int, [c_f32p, c_i64, c_i64, c_f32p, c_i64, c_i64, C.c_int, C.c_int, C.c_int,
                                         C.c_void_p]),
     "fdn_copy3d": (C.c_int, [c_f32p, c_i64, c_i64, C.c_int, C.c_int, C.c_int, C.c_int, c_f32p, c_i64, c_i64, C.c_int,

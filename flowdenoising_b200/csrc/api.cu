@@ -234,14 +234,17 @@ static int farneback_batch(const float* R, const Geometry& g, SlotMap map0, Slot
 }
 
 struct PassPlan {
-    int chunk, r, slots, full_wrap;
+    int chunk, r, slots, full_wrap;   // slots: R-cache slots per volume (the cache holds batch * slots)
+    int batch;
     Geometry g;
     size_t off_R, off_P, off_S1, off_S2, off_stash, off_scratch, scratch_bytes, off_acc, total;
 };
 
 // esize: bytes per element of the volume (4: float32, whose accumulator is the output itself; 1 or 2: a typed volume,
 // whose stash holds T and whose float32 accumulator for one chunk follows the other buffers)
-static int make_plan(const fdn_view& v, int klen, const fdn_of_params& of, int chunk, size_t esize, PassPlan* p)
+// batch > 1: volumes of one whole periodic axis each (fdn_filter_axis_batch), every per-chunk buffer holds batch chunks
+static int make_plan(const fdn_view& v, int klen, const fdn_of_params& of, int chunk, size_t esize, PassPlan* p,
+                     int batch = 1)
 {
     int rc;
     FDN_CHECK_ARG(klen >= 1 && (klen & 1), "kernel length must be odd (src/flowdenoising.py:309)");
@@ -260,20 +263,26 @@ static int make_plan(const fdn_view& v, int klen, const fdn_of_params& of, int c
     }
     if ((rc = check_of(&of))) return rc;
     if ((rc = make_geometry(v.H, v.W, of.levels, &p->g))) return rc;
-    if (chunk <= 0 || chunk > v.n_out) chunk = v.n_out;
+    FDN_CHECK_ARG(batch >= 1, "batch must be >= 1");
+    FDN_CHECK_ARG(batch == 1 || (v.periodic && v.halo == 0 && v.n_out == v.n_in),
+                  "a batch member must be a whole periodic axis (periodic = 1, halo = 0, n_out = n_in)");
+    // image pairs of one launch: 2 * batch * chunk (kept inside int, like every image index of the kernels)
+    FDN_CHECK_ARG(2ll * batch * v.n_out < (1ll << 31), "too many image pairs in one batch");
+    p->batch = batch;
+    if (chunk <= 0 || chunk > v.n_out || batch > 1) chunk = v.n_out;
     p->chunk = chunk;
     p->full_wrap = v.periodic && (chunk + 2 * p->r >= v.n_in);
     p->slots = p->full_wrap ? v.n_in : chunk + 2 * p->r;
     // both chain directions advance together: 2 * chunk image pairs per launch
-    const size_t px = (size_t)chunk * v.H * v.W;
+    const size_t px = (size_t)batch * chunk * v.H * v.W;
     const size_t fl = sizeof(float) * 2 * 2 * px;
     size_t off = 0;
-    p->off_R = off;  off += align_up(sizeof(float) * p->g.R_slot * (size_t)p->slots, 256);
+    p->off_R = off;  off += align_up(sizeof(float) * p->g.R_slot * (size_t)p->slots * batch, 256);
     p->off_P = off;  off += align_up(fl, 256);
     p->off_S1 = off; off += align_up(fl, 256);
     p->off_S2 = off; off += align_up(fl, 256);
     p->off_stash = off; off += align_up(esize * px * (size_t)p->r, 256);   // remapped forward neighbours
-    p->scratch_bytes = flow_iter_scratch_bytes(2 * chunk, p->g.nl + 1, p->g.hs, p->g.ws);   // every level of the pass
+    p->scratch_bytes = flow_iter_scratch_bytes(2 * batch * chunk, p->g.nl + 1, p->g.hs, p->g.ws);   // every level
     p->off_scratch = off; off += align_up(p->scratch_bytes, 256);
     p->off_acc = off;
     if (esize != sizeof(float)) off += align_up(sizeof(float) * px, 256);
@@ -283,14 +292,18 @@ static int make_plan(const fdn_view& v, int klen, const fdn_of_params& of, int c
 
 // T = float: the accumulator is d_out itself. Integer T: a float32 accumulator of one chunk in the workspace; the last
 // tap truncates it into d_out (the reference's `filtered_vol[z] = tmp_slice` into an integer volume).
+// batch > 1 (make_plan: whole periodic axes, one chunk): volume g reads d_in + g * in_bs and writes d_out + g * out_bs.
+// A launch's images are ordered [chain][volume][slice]: pairs [0, B*C) are the backward neighbours, [B*C, 2*B*C) the
+// forward ones, and the SlotMaps resolve image j of a chain to volume j / C, slice j % C.
 template <typename T>
 static int filter_axis_of(const T* d_in, T* d_out, const fdn_view& v, const double* kernel, int klen,
-                          const fdn_of_params& of, int chunk, void* ws, size_t ws_bytes, cudaStream_t st)
+                          const fdn_of_params& of, int chunk, void* ws, size_t ws_bytes, cudaStream_t st,
+                          int batch = 1, int64_t in_bs = 0, int64_t out_bs = 0)
 {
     constexpr bool typed = !std::is_same<T, float>::value;
     int rc;
     PassPlan p;
-    if ((rc = make_plan(v, klen, of, chunk, sizeof(T), &p))) return rc;
+    if ((rc = make_plan(v, klen, of, chunk, sizeof(T), &p, batch))) return rc;
     if (ws_bytes < p.total || ws == nullptr) {
         set_error("workspace too small: need %zu bytes, got %zu", p.total, ws_bytes);
         return FDN_ERR_WORKSPACE;
@@ -303,12 +316,14 @@ static int filter_axis_of(const T* d_in, T* d_out, const fdn_view& v, const doub
     float* S2 = reinterpret_cast<float*>(base + p.off_S2);
     T* stash = reinterpret_cast<T*>(base + p.off_stash);
     FlowScratch fs;
-    if ((rc = flow_scratch_make(base + p.off_scratch, p.scratch_bytes, 2 * p.chunk, p.g.nl + 1, p.g.hs, p.g.ws, &fs)))
+    if ((rc = flow_scratch_make(base + p.off_scratch, p.scratch_bytes, 2 * batch * p.chunk, p.g.nl + 1, p.g.hs, p.g.ws,
+                                &fs)))
         return rc;
     if ((rc = flow_iter_scratch_init(fs, st))) return rc;
     PolyConsts pc;
     prepare_poly_consts(of.poly_n, of.poly_sigma, &pc);
     const int wrap_in = v.periodic ? v.n_in : 0;
+    const int64_t R_vs = (int64_t)p.slots * p.g.R_slot;   // R-cache floats per volume
     bool cache_full = false;
 
     for (int c0 = 0; c0 < v.n_out; c0 += p.chunk) {
@@ -318,11 +333,14 @@ static int filter_axis_of(const T* d_in, T* d_out, const fdn_view& v, const doub
         if (!(p.full_wrap && cache_full)) {
             const int need = p.full_wrap ? v.n_in : C + 2 * r;
             float* tmpA = S1;
-            float* tmpB = S1 + (size_t)p.chunk * H * W;
+            float* tmpB = S1 + (size_t)batch * p.chunk * H * W;
             float* img = S2;
-            for (int sb = 0; sb < need; sb += p.chunk) {
-                const int nb = need - sb < p.chunk ? need - sb : p.chunk;
+            // batch > 1: one sub-batch of every slice of every volume (need == chunk); R slot b = volume * n_in + slice
+            for (int sb = 0; sb < batch * need; sb += batch * p.chunk) {
+                const int nb = batch * need - sb < batch * p.chunk ? batch * need - sb : batch * p.chunk;
                 SlotMap in_map{p.full_wrap ? sb : ubase + sb, wrap_in};
+                in_map.per = need;
+                in_map.vstride = in_bs;
                 SlotMap R_map{sb, 0};
                 if ((rc = build_R(d_in, v.in_slice_stride, v.in_row_stride, in_map, nb, H, W, p.g, pc, R, R_map, tmpA,
                                   tmpB, img, st)))
@@ -334,28 +352,38 @@ static int filter_axis_of(const T* d_in, T* d_out, const fdn_view& v, const doub
         //      pairs [0, C) = (slice, slice - d), pairs [C, 2C) = (slice, slice + d) ----
         const int cbase = p.full_wrap ? c0 + v.halo : r;             // R slot of the chunk's first centre slice
         const int swrap = p.full_wrap ? v.n_in : 0;
-        SlotMap map0{cbase, swrap, C, cbase};
+        const int BC = batch * C;                                    // pairs of one chain
+        // every map below resolves image j of a chain to volume j / C, slice j % C (one volume: always volume 0)
+        auto vmap = [&](int b1, int wrap, int split, int b2, int64_t vstride) {
+            SlotMap m{b1, wrap, split, b2};
+            m.per = C;
+            m.vstride = vstride;
+            return m;
+        };
+        const SlotMap map0 = vmap(cbase, swrap, BC, cbase, R_vs);
         T* out = d_out + (int64_t)c0 * v.out_slice_stride;
         float* acc = typed ? reinterpret_cast<float*>(base + p.off_acc) : reinterpret_cast<float*>(out);
         const int64_t a_ss = typed ? (int64_t)H * W : v.out_slice_stride, a_rs = typed ? (int64_t)W : v.out_row_stride;
-        const size_t fbytes = sizeof(float) * 2 * 2 * (size_t)C * H * W;
+        const SlotMap amap = vmap(0, 0, 0x7fffffff, 0, typed ? 0 : out_bs);   // (typed: batch == 1)
+        const SlotMap omap = vmap(0, 0, 0x7fffffff, 0, out_bs);
+        const size_t fbytes = sizeof(float) * 2 * 2 * (size_t)BC * H * W;
         if (r > 0) FDN_CUDA(cudaMemsetAsync(P, 0, fbytes, st));  // prev_flow = zeros (:310, :318)
         for (int d = 1; d <= r; d++) {
-            SlotMap map1{cbase - d, swrap, C, cbase + d};
-            if ((rc = farneback_batch(R, p.g, map0, map1, P, S1, S2, 2 * C, H, W, of, fs, st))) return rc;
+            const SlotMap map1 = vmap(cbase - d, swrap, BC, cbase + d, R_vs);
+            if ((rc = farneback_batch(R, p.g, map0, map1, P, S1, S2, 2 * BC, H, W, of, fs, st))) return rc;
             // backward neighbour: tap r-d accumulated now (reference order -1, -2, ..., -r); forward neighbour:
             // remapped now, applied by launch_acc_finish after the centre tap (order 0, +1, ..., +r)
-            SlotMap nmap{c0 + v.halo - d, wrap_in, C, c0 + v.halo + d};
+            const SlotMap nmap = vmap(c0 + v.halo - d, wrap_in, BC, c0 + v.halo + d, in_bs);
             if ((rc = launch_warp_pair(d_in, v.in_slice_stride, v.in_row_stride, nmap, P, kernel[r - d], acc, a_ss, a_rs,
-                                       stash + (size_t)(d - 1) * C * H * W, C, H, W, d == 1 ? 1 : 0, st)))
+                                       amap, stash + (size_t)(d - 1) * BC * H * W, BC, H, W, d == 1 ? 1 : 0, st)))
                 return rc;
-            progress_add(st, 1000ll * C / (r + 1));
+            progress_add(st, 1000ll * BC / (r + 1));
         }
-        SlotMap cmap{c0 + v.halo, wrap_in};
+        const SlotMap cmap = vmap(c0 + v.halo, wrap_in, 0x7fffffff, 0, in_bs);
         if ((rc = launch_acc_finish(d_in, v.in_slice_stride, v.in_row_stride, cmap, stash, r, kernel + r, acc, a_ss, a_rs,
-                                    out, v.out_slice_stride, v.out_row_stride, C, H, W, r > 0 ? 1 : 0, st)))
+                                    amap, out, v.out_slice_stride, v.out_row_stride, omap, BC, H, W, r > 0 ? 1 : 0, st)))
             return rc;
-        progress_add(st, 1000ll * C - (long long)r * (1000ll * C / (r + 1)));
+        progress_add(st, 1000ll * BC - (long long)r * (1000ll * BC / (r + 1)));
     }
     return FDN_OK;
 }
@@ -550,6 +578,42 @@ int fdn_filter_axis(const float* d_in, float* d_out, const fdn_view* view, const
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (!of) return fdn_gauss_axis(d_in, d_out, view, kernel, klen, 1, stream);
     return filter_axis_of(d_in, d_out, *view, kernel, klen, *of, chunk, d_workspace, workspace_bytes, st);
+}
+
+size_t fdn_workspace_bytes_batch(const fdn_view* view, int batch, int klen, const fdn_of_params* of)
+{
+    if (!view || !of) { set_error("null argument"); return 0; }
+    PassPlan p;
+    if (make_plan(*view, klen, *of, 0, sizeof(float), &p, batch)) return 0;
+    return p.total;
+}
+
+int fdn_filter_axis_batch(const float* d_in, float* d_out, const fdn_view* view, int batch, int64_t in_batch_stride,
+                          int64_t out_batch_stride, const double* kernel, int klen, const fdn_of_params* of,
+                          void* d_workspace, size_t workspace_bytes, void* stream)
+{
+    FDN_CHECK_ARG(d_in && d_out && view && kernel, "null argument");
+    if (!of) return fdn_gauss_axis_batch(d_in, d_out, view, batch, in_batch_stride, out_batch_stride, kernel, klen, 1,
+                                         stream);
+    return filter_axis_of(d_in, d_out, *view, kernel, klen, *of, 0, d_workspace, workspace_bytes,
+                          static_cast<cudaStream_t>(stream), batch, in_batch_stride, out_batch_stride);
+}
+
+int fdn_gauss_axis_batch(const float* d_in, float* d_out, const fdn_view* view, int batch, int64_t in_batch_stride,
+                         int64_t out_batch_stride, const double* kernel, int klen, int exact, void* stream)
+{
+    FDN_CHECK_ARG(d_in && d_out && view && kernel, "null argument");
+    const fdn_view& v = *view;
+    FDN_CHECK_ARG(batch >= 1, "batch must be >= 1");
+    FDN_CHECK_ARG(klen >= 1 && (klen & 1), "kernel length must be odd");
+    FDN_CHECK_ARG(klen <= FDN_MAX_KLEN, "kernel length %d unsupported (<= %d, sigma < 32.125)", klen, FDN_MAX_KLEN);
+    FDN_CHECK_ARG(v.n_in >= 1 && v.H >= 1 && v.W >= 1, "empty view");
+    FDN_CHECK_ARG(v.periodic && v.halo == 0 && v.n_out == v.n_in,
+                  "a batch member must be a whole periodic axis (periodic = 1, halo = 0, n_out = n_in)");
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int rc = launch_gauss_axis(d_in, d_out, v, kernel, klen, exact, st, batch, in_batch_stride, out_batch_stride);
+    if (rc == FDN_OK) progress_add(st, 1000ll * batch * v.n_out);
+    return rc;
 }
 
 size_t fdn_workspace_bytes_typed(const fdn_view* view, int klen, const fdn_of_params* of, int chunk, int dtype)

@@ -89,17 +89,29 @@ int prepare_blur_taps(int ksz, double sigma, BlurTaps* bt);
 //   s = (base + b) mod wrap (wrap  > 0)
 // A batch may be the concatenation of two runs (the backward and the forward chain of a pass advance together):
 // images b >= split continue at base2 + (b - split).
+// A run may span several volumes of a batch (fdn_filter_axis_batch): image j of a run belongs to volume j / per, and
+// the slot above is taken with the volume-local index j % per; the volume adds vstride to the offset. One volume:
+// per = 0x7fffffff, so every index is local. b0 shifts a launch's images (launchers that split over blockIdx.z).
 struct SlotMap {
     int base, wrap;
     int split = 0x7fffffff, base2 = 0;
-    __host__ __device__ inline int slot(int b) const
+    int per = 0x7fffffff;
+    int64_t vstride = 0;
+    int b0 = 0;
+    // element (or float) offset of image b's data: slot * stride + volume * vstride
+    __host__ __device__ inline int64_t offset(int b, int64_t stride) const
     {
-        int s = b < split ? base + b : base2 + (b - split);
+        b += b0;
+        const bool first = b < split;
+        int j = first ? b : b - split;
+        const int g = j / per;
+        j -= g * per;
+        int s = (first ? base : base2) + j;
         if (wrap > 0) {
             s %= wrap;
             if (s < 0) s += wrap;
         }
-        return s;
+        return (int64_t)s * stride + (int64_t)g * vstride;
     }
 };
 
@@ -152,25 +164,27 @@ int launch_flow_upsample(const float* flow, int n, int hin, int win, float* out,
 int launch_warp_acc(const float* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_map, const float* flow, double weight,
                     float* acc, int64_t a_ss, int64_t a_rs, int n, int H, int W, int first, cudaStream_t st);
 // One chain step of both directions: images [0, n) (backward neighbours, flows flow[0..n)) are remapped and
-// accumulated into acc with `weight`; images [n, 2n) (forward neighbours, flows flow[n..2n)) are remapped into
+// accumulated into acc (image b at a_map.offset(b, a_ss)) with `weight`; images [n, 2n) (forward neighbours, flows flow[n..2n)) are remapped into
 // stash (dense [n][H][W]) for launch_acc_finish. T: element type of the volume and the stash (integer T: OpenCV's
 // integer remap, the accumulator stays float32).
 template <typename T>
 int launch_warp_pair(const T* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_map, const float* flow, double weight,
-                     float* acc, int64_t a_ss, int64_t a_rs, T* stash, int n, int H, int W, int first, cudaStream_t st);
+                     float* acc, int64_t a_ss, int64_t a_rs, SlotMap a_map, T* stash, int n, int H, int W, int first,
+                     cudaStream_t st);
 // acc = fold over [centre * k[0], stash[0] * k[1], ..., stash[r-1] * k[r]] of f32(f64(acc) + f64(v) * k), in that
 // order; have_acc == 0 starts from 0 (no backward taps). float: the result stays in acc (out unused); integer T: the
 // float32 result is truncated into out (the reference's `int_vol[z] = tmp_slice`).
 template <typename T>
 int launch_acc_finish(const T* centre, int64_t c_ss, int64_t c_rs, SlotMap c_map, const T* stash, int r, const double* k,
-                      float* acc, int64_t a_ss, int64_t a_rs, T* out, int64_t o_ss, int64_t o_rs, int n, int H, int W,
-                      int have_acc, cudaStream_t st);
+                      float* acc, int64_t a_ss, int64_t a_rs, SlotMap a_map, T* out, int64_t o_ss, int64_t o_rs,
+                      SlotMap o_map, int n, int H, int W, int have_acc, cudaStream_t st);
 // cv2.remap of n dense T images (FDN_DTYPE_* other than int8)
 template <typename T>
 int launch_remap(const T* src, const float* flow, T* dst, int n, int H, int W, cudaStream_t st);
 // no-OF
+// batch volumes of view v, volume g at in + g * in_bs / out + g * out_bs (elements)
 int launch_gauss_axis(const float* in, float* out, const fdn_view& v, const double* k, int klen, int exact,
-                      cudaStream_t st);
+                      cudaStream_t st, int batch = 1, int64_t in_bs = 0, int64_t out_bs = 0);
 int launch_gauss_rows(const float* in, float* out, int64_t rows, int W, const double* k, int klen, int exact,
                       cudaStream_t st);
 // typed no-OF passes: T in, T out, exact arithmetic only, truncated store

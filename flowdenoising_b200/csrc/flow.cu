@@ -167,8 +167,8 @@ k_flow_iter(FlowIterArgs a)
     const float sxc = __fmul_rn(xcl < 5 ? (xcl < 2 ? 0.14f : 0.4472f) : 1.f,
                                 xcl >= w - 5 ? (w - xcl - 1 < 2 ? 0.14f : 0.4472f) : 1.f);
 
-    const float* R0 = a.R + (int64_t)a.map0.slot(b) * a.R_stride;
-    const float* R1 = a.R + (int64_t)a.map1.slot(b) * a.R_stride;
+    const float* R0 = a.R + a.map0.offset(b, a.R_stride);
+    const float* R1 = a.R + a.map1.offset(b, a.R_stride);
     const float4* R0a = reinterpret_cast<const float4*>(R0);
     const float4* R1a = reinterpret_cast<const float4*>(R1);
     const float* R0b = R0 + (int64_t)4 * h * w;
@@ -817,8 +817,8 @@ k_flow_iter_ws(WsArgs wa)
     const float sxc = __fmul_rn(xcl < 5 ? (xcl < 2 ? 0.14f : 0.4472f) : 1.f,
                                 xcl >= w - 5 ? (w - xcl - 1 < 2 ? 0.14f : 0.4472f) : 1.f);
 
-    const float* R0 = wa.R + (int64_t)wa.map0.slot(b) * wa.R_stride;
-    const float* R1 = wa.R + (int64_t)wa.map1.slot(b) * wa.R_stride;
+    const float* R0 = wa.R + wa.map0.offset(b, wa.R_stride);
+    const float* R1 = wa.R + wa.map1.offset(b, wa.R_stride);
     const float4* R0a = reinterpret_cast<const float4*>(R0);
     const float* R0b = R0 + (int64_t)4 * h * w;
     const float4* R1a = reinterpret_cast<const float4*>(R1);
@@ -1249,8 +1249,8 @@ k_flow_gauss_iter(GaussIterArgs a)
     const int xcl = min(max(xcol, 0), w - 1);
     const bool core = t < a.CW && x0 + t < w;
 
-    const float* R0 = a.R + (int64_t)a.map0.slot(b) * a.R_stride;
-    const float* R1 = a.R + (int64_t)a.map1.slot(b) * a.R_stride;
+    const float* R0 = a.R + a.map0.offset(b, a.R_stride);
+    const float* R1 = a.R + a.map1.offset(b, a.R_stride);
     const float4* R0a = reinterpret_cast<const float4*>(R0);
     const float4* R1a = reinterpret_cast<const float4*>(R1);
     const float* R0b = R0 + (int64_t)4 * h * w;

@@ -94,12 +94,16 @@ static bool taps_benign(const double* k, int n)
 // ------------------------------------------------------------------------------------------------
 template <typename T, bool EXACT>
 __global__ void __launch_bounds__(256)
-k_gauss_axis(const T* __restrict__ in, T* __restrict__ out, fdn_view v, Taps64 t64, Taps32 t32)
+k_gauss_axis(const T* __restrict__ in, T* __restrict__ out, fdn_view v, Taps64 t64, Taps32 t32, int64_t in_bs,
+             int64_t out_bs)
 {
     const int x = blockIdx.x * 256 + threadIdx.x;
     const int y = blockIdx.y;
-    const int s = blockIdx.z;
+    const int g = blockIdx.z / v.n_out;   // volume of a batch (blockIdx.z = volume * n_out + slice)
+    const int s = blockIdx.z - g * v.n_out;
     if (x >= v.W) return;
+    in += g * in_bs;
+    out += g * out_bs;
     const int klen = EXACT ? t64.klen : t32.klen;
     const int r = klen >> 1;
     const int64_t off = (int64_t)y * v.in_row_stride + x;
@@ -165,7 +169,8 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 
 template <int KLEN, bool EXACT, int VEC>
 __global__ void __launch_bounds__(128)
-k_gauss_axis_ring(const float* __restrict__ in, float* __restrict__ out, fdn_view v, TapsW<KLEN> taps, int int_rounding)
+k_gauss_axis_ring(const float* __restrict__ in, float* __restrict__ out, fdn_view v, TapsW<KLEN> taps, int int_rounding,
+                  int nseg, int64_t in_bs, int64_t out_bs)
 {
     constexpr int R = KLEN / 2;
     typedef typename std::conditional<EXACT, double, float>::type W_t;   // window element
@@ -174,8 +179,11 @@ k_gauss_axis_ring(const float* __restrict__ in, float* __restrict__ out, fdn_vie
     const int t = threadIdx.x;
     const int x = (blockIdx.x * 128 + t) * VEC;
     const int y = blockIdx.y;
-    const int s0 = blockIdx.z * GA_SEG;
+    const int g = blockIdx.z / nseg;   // volume of a batch (blockIdx.z = volume * nseg + segment)
+    const int s0 = (blockIdx.z - g * nseg) * GA_SEG;
     if (x >= v.W) return;       // (no block-level synchronisation below)
+    in += g * in_bs;
+    out += g * out_bs;
     const int s_end = min(s0 + GA_SEG, v.n_out);
     const int n_in_seg = s_end - s0 + 2 * R;          // input slices this thread consumes: s0 - R .. s_end - 1 + R
     const float* src = in + (int64_t)y * v.in_row_stride + x;
@@ -276,7 +284,7 @@ k_gauss_axis_ring(const float* __restrict__ in, float* __restrict__ out, fdn_vie
 
 template <int KLEN>
 static int launch_gauss_axis_ring(const float* in, float* out, const fdn_view& v, const double* k, int exact,
-                                  cudaStream_t st)
+                                  cudaStream_t st, int batch, int64_t in_bs, int64_t out_bs)
 {
     TapsW<KLEN> taps;
     for (int i = 0; i < KLEN; i++) { taps.k64[i] = k[i]; taps.k32[i] = (float)k[i]; }
@@ -290,45 +298,57 @@ static int launch_gauss_axis_ring(const float* in, float* out, const fdn_view& v
     if (aligned(2)) vec = 2;
     if (!exact && KLEN <= 17 && aligned(4)) vec = 4;
     const int ir = taps_benign(k, KLEN) ? 1 : 0;
-    dim3 grid((unsigned)cdiv(v.W, 128 * vec), (unsigned)v.H, (unsigned)cdiv(v.n_out, GA_SEG));
-    ProfScope ps(K_GAUSS_AXIS, 8.0 * v.n_out * v.H * v.W, st);
-    if (exact) {
-        if (vec == 2) k_gauss_axis_ring<KLEN, true, 2><<<grid, 128, 0, st>>>(in, out, v, taps, ir);
-        else k_gauss_axis_ring<KLEN, true, 1><<<grid, 128, 0, st>>>(in, out, v, taps, ir);
-    } else {
-        if (vec == 4) k_gauss_axis_ring<KLEN, false, 4><<<grid, 128, 0, st>>>(in, out, v, taps, ir);
-        else if (vec == 2) k_gauss_axis_ring<KLEN, false, 2><<<grid, 128, 0, st>>>(in, out, v, taps, ir);
-        else k_gauss_axis_ring<KLEN, false, 1><<<grid, 128, 0, st>>>(in, out, v, taps, ir);
+    while (batch > 1 && vec > 1 && (in_bs % vec != 0 || out_bs % vec != 0)) vec /= 2;   // every volume stays aligned
+    const int nseg = (int)cdiv(v.n_out, GA_SEG);
+    const int per_launch = 65535 / nseg;   // volumes per launch: batch x segments in blockIdx.z
+    for (int g0 = 0; g0 < batch; g0 += per_launch) {
+        const int nb = batch - g0 < per_launch ? batch - g0 : per_launch;
+        const float* i_ = in + g0 * in_bs;
+        float* o_ = out + g0 * out_bs;
+        dim3 grid((unsigned)cdiv(v.W, 128 * vec), (unsigned)v.H, (unsigned)(nb * nseg));
+        ProfScope ps(K_GAUSS_AXIS, 8.0 * nb * v.n_out * v.H * v.W, st);
+        if (exact) {
+            if (vec == 2) k_gauss_axis_ring<KLEN, true, 2><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
+            else k_gauss_axis_ring<KLEN, true, 1><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
+        } else {
+            if (vec == 4) k_gauss_axis_ring<KLEN, false, 4><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
+            else if (vec == 2) k_gauss_axis_ring<KLEN, false, 2><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
+            else k_gauss_axis_ring<KLEN, false, 1><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
+        }
+        FDN_LAUNCHED("k_gauss_axis_ring");
     }
-    FDN_LAUNCHED("k_gauss_axis_ring");
     return FDN_OK;
 }
 
 int launch_gauss_axis(const float* in, float* out, const fdn_view& v, const double* k, int klen, int exact,
-                      cudaStream_t st)
+                      cudaStream_t st, int batch, int64_t in_bs, int64_t out_bs)
 {
     FDN_CHECK_ARG(klen >= 1 && klen <= FDN_MAX_KLEN && (klen & 1), "kernel length %d unsupported (odd, <= %d)", klen,
                   FDN_MAX_KLEN);
     FDN_CHECK_ARG(v.H <= 65535 && v.n_out <= 65535, "view too large for one launch");
     switch (klen) {  // sigma = 0.5, 1, 1.5, 2, 2.5, 3, 4 (radius int(4 sigma + 0.5))
-        case 5: return launch_gauss_axis_ring<5>(in, out, v, k, exact, st);
-        case 9: return launch_gauss_axis_ring<9>(in, out, v, k, exact, st);
-        case 13: return launch_gauss_axis_ring<13>(in, out, v, k, exact, st);
-        case 17: return launch_gauss_axis_ring<17>(in, out, v, k, exact, st);
-        case 21: return launch_gauss_axis_ring<21>(in, out, v, k, exact, st);
-        case 25: return launch_gauss_axis_ring<25>(in, out, v, k, exact, st);
-        case 33: return launch_gauss_axis_ring<33>(in, out, v, k, exact, st);
+        case 5: return launch_gauss_axis_ring<5>(in, out, v, k, exact, st, batch, in_bs, out_bs);
+        case 9: return launch_gauss_axis_ring<9>(in, out, v, k, exact, st, batch, in_bs, out_bs);
+        case 13: return launch_gauss_axis_ring<13>(in, out, v, k, exact, st, batch, in_bs, out_bs);
+        case 17: return launch_gauss_axis_ring<17>(in, out, v, k, exact, st, batch, in_bs, out_bs);
+        case 21: return launch_gauss_axis_ring<21>(in, out, v, k, exact, st, batch, in_bs, out_bs);
+        case 25: return launch_gauss_axis_ring<25>(in, out, v, k, exact, st, batch, in_bs, out_bs);
+        case 33: return launch_gauss_axis_ring<33>(in, out, v, k, exact, st, batch, in_bs, out_bs);
         default: break;
     }
     Taps64 t64;
     Taps32 t32;
     t64.klen = t32.klen = klen;
     for (int i = 0; i < klen; i++) { t64.k[i] = k[i]; t32.k[i] = (float)k[i]; }
-    dim3 grid((unsigned)cdiv(v.W, 256), (unsigned)v.H, (unsigned)v.n_out);
-    ProfScope ps(K_GAUSS_AXIS, 8.0 * v.n_out * v.H * v.W, st);
-    if (exact) k_gauss_axis<float, true><<<grid, 256, 0, st>>>(in, out, v, t64, t32);
-    else k_gauss_axis<float, false><<<grid, 256, 0, st>>>(in, out, v, t64, t32);
-    FDN_LAUNCHED("k_gauss_axis");
+    const int per_launch = 65535 / v.n_out;   // volumes per launch: batch x slices in blockIdx.z
+    for (int g0 = 0; g0 < batch; g0 += per_launch) {
+        const int nb = batch - g0 < per_launch ? batch - g0 : per_launch;
+        dim3 grid((unsigned)cdiv(v.W, 256), (unsigned)v.H, (unsigned)(nb * v.n_out));
+        ProfScope ps(K_GAUSS_AXIS, 8.0 * nb * v.n_out * v.H * v.W, st);
+        if (exact) k_gauss_axis<float, true><<<grid, 256, 0, st>>>(in + g0 * in_bs, out + g0 * out_bs, v, t64, t32, in_bs, out_bs);
+        else k_gauss_axis<float, false><<<grid, 256, 0, st>>>(in + g0 * in_bs, out + g0 * out_bs, v, t64, t32, in_bs, out_bs);
+        FDN_LAUNCHED("k_gauss_axis");
+    }
     return FDN_OK;
 }
 
@@ -493,7 +513,7 @@ int launch_gauss_axis_typed(const T* in, T* out, const fdn_view& v, const double
     for (int i = 0; i < klen; i++) { t64.k[i] = k[i]; t32.k[i] = (float)k[i]; }
     dim3 grid((unsigned)cdiv(v.W, 256), (unsigned)v.H, (unsigned)v.n_out);
     ProfScope ps(K_GAUSS_AXIS, 2.0 * sizeof(T) * v.n_out * v.H * v.W, st);
-    k_gauss_axis<T, true><<<grid, 256, 0, st>>>(in, out, v, t64, t32);
+    k_gauss_axis<T, true><<<grid, 256, 0, st>>>(in, out, v, t64, t32, 0, 0);
     FDN_LAUNCHED("k_gauss_axis");
     return FDN_OK;
 }

@@ -134,7 +134,7 @@ k_blur_rows(const T* __restrict__ in_, int64_t in_ss, int64_t in_rs, SlotMap in_
     const int y = blockIdx.y;
     const int b = blockIdx.z;
     if (x >= W) return;
-    const T* s_ = in_ + (int64_t)in_map.slot(b) * in_ss + (int64_t)y * in_rs;
+    const T* s_ = in_ + in_map.offset(b, in_ss) + (int64_t)y * in_rs;
     auto s = [&](int i) { return (float)s_[i]; };
     const int ksz = bt.ksz, r = ksz >> 1;
     float acc;
@@ -195,7 +195,7 @@ k_blur_rows4(const T* __restrict__ in, int64_t in_ss, int64_t in_rs, SlotMap in_
     const int y = blockIdx.y;
     const int b = blockIdx.z;
     if (x0 >= W) return;
-    const T* s = in + (int64_t)in_map.slot(b) * in_ss + (int64_t)y * in_rs;
+    const T* s = in + in_map.offset(b, in_ss) + (int64_t)y * in_rs;
     float v[4 + 2 * R];
     if (x0 >= R && x0 + 3 + R < W) {
 #pragma unroll
@@ -265,7 +265,7 @@ int launch_blur_rows(const T* in, int64_t in_ss, int64_t in_rs, SlotMap in_map, 
     for (int b0 = 0; b0 < n; b0 += 65535) {
         int nb = n - b0 < 65535 ? n - b0 : 65535;
         SlotMap m = in_map;
-        m.base += b0;
+        m.b0 += b0;
         ProfScope ps(K_BLUR_ROWS, (4.0 + sizeof(T)) * nb * H * W, st);
         if (win4) {
             dim3 grid((unsigned)cdiv(W, 512), (unsigned)H, (unsigned)nb);
@@ -427,7 +427,7 @@ k_polyexp(const float* __restrict__ img, int64_t img_stride, float* __restrict__
             b6 = __dadd_rn(b6, (double)__fmul_rn(__fsub_rn(r1[k], r1[-k]), pc.xg[k]));
             b5 = __dadd_rn(b5, (double)__fmul_rn(__fadd_rn(r2[k], r2[-k]), g0));
         }
-        float* dst = R + (int64_t)R_map.slot(b) * R_stride;
+        float* dst = R + R_map.offset(b, R_stride);
         float4 o;
         o.x = (float)__dmul_rn(b3, pc.ig11);
         o.y = (float)__dmul_rn(b2, pc.ig11);
@@ -492,7 +492,7 @@ k_polyexp_tma(const __grid_constant__ CUtensorMap tmap, float* __restrict__ R, i
     const uint32_t dst0 = smem_u32(&s_in[0][0]), dst1 = smem_u32(&s_in[1][0]);
     if (threadIdx.x == 0) tma_load_box(tmap_addr, dst0, bar0, box_bytes, -PL, y0 - n, b);
 
-    float* dstR = R + (int64_t)R_map.slot(b) * R_stride;
+    float* dstR = R + R_map.offset(b, R_stride);
     for (int tile = 0; tile < ntiles; tile++) {
         const int buf = tile & 1;
         if (threadIdx.x == 0 && tile + 1 < ntiles)   // prefetch the next tile into the other buffer
@@ -630,7 +630,7 @@ int launch_polyexp(const float* img, int64_t img_stride, float* R, int64_t R_str
     for (int b0 = 0; b0 < n; b0 += 65535) {
         int nb = n - b0 < 65535 ? n - b0 : 65535;
         SlotMap m = R_map;
-        m.base += b0;
+        m.b0 += b0;
         dim3 grid((unsigned)cdiv(w, PT), (unsigned)cdiv(h, PT), (unsigned)nb);
         ProfScope ps(K_POLYEXP, 24.0 * nb * h * w, st);
         k_polyexp<<<grid, 256, 0, st>>>(img + (int64_t)b0 * img_stride, img_stride, R, R_stride, m, h, w, pc);

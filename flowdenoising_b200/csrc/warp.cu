@@ -23,7 +23,7 @@ k_warp_acc(const float* __restrict__ neigh, int64_t n_ss, int64_t n_rs, SlotMap 
     const int y = blockIdx.y;
     const int b = blockIdx.z;
     if (x >= W) return;
-    const float* src = neigh + (int64_t)n_map.slot(b) * n_ss;
+    const float* src = neigh + n_map.offset(b, n_ss);
     float v;
     if (flow) {
         const float2 f = flow[((int64_t)b * H + y) * W + x];
@@ -105,7 +105,7 @@ k_warp_acc4(const float* __restrict__ neigh, int64_t n_ss, int64_t n_rs, SlotMap
     const int y = blockIdx.y;
     const int b = blockIdx.z;
     if (x >= W) return;
-    const float* src = neigh + (int64_t)n_map.slot(b) * n_ss;
+    const float* src = neigh + n_map.offset(b, n_ss);
     float v[4];
     if (flow) {
         const float4* fp = flow + (((int64_t)b * H + y) * W + x) / 2;   // two float2 flows per float4
@@ -142,7 +142,7 @@ int launch_warp_acc(const float* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_ma
         for (int b0 = 0; b0 < n; b0 += 65535) {
             const int nb = n - b0 < 65535 ? n - b0 : 65535;
             SlotMap m = n_map;
-            m.base += b0;
+            m.b0 += b0;
             dim3 grid((unsigned)cdiv(W, 512), (unsigned)H, (unsigned)nb);
             ProfScope ps(K_WARP_ACC, (double)nb * H * W * (4.0 + (flow ? 8.0 : 0.0) + (first ? 4.0 : 8.0)), st);
             k_warp_acc4<<<grid, 128, 0, st>>>(neigh, n_ss, n_rs, m,
@@ -155,7 +155,7 @@ int launch_warp_acc(const float* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_ma
     for (int b0 = 0; b0 < n; b0 += 65535) {
         const int nb = n - b0 < 65535 ? n - b0 : 65535;
         SlotMap m = n_map;
-        m.base += b0;
+        m.b0 += b0;
         dim3 grid((unsigned)cdiv(W, 128), (unsigned)H, (unsigned)nb);
         ProfScope ps(K_WARP_ACC, (double)nb * H * W * (4.0 + (flow ? 8.0 : 0.0) + (first ? 4.0 : 8.0)), st);
         k_warp_acc<<<grid, 128, 0, st>>>(neigh, n_ss, n_rs, m,
@@ -177,14 +177,14 @@ int launch_warp_acc(const float* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_ma
 template <typename T, int VEC>
 __global__ void __launch_bounds__(128)
 k_warp_pair(const T* __restrict__ neigh, int64_t n_ss, int64_t n_rs, SlotMap n_map, const float* __restrict__ flow,
-            double weight, float* __restrict__ acc, int64_t a_ss, int64_t a_rs, T* __restrict__ stash, int n, int b0,
-            int H, int W, int first)
+            double weight, float* __restrict__ acc, int64_t a_ss, int64_t a_rs, SlotMap a_map, T* __restrict__ stash,
+            int n, int b0, int H, int W, int first)
 {
     const int x = (blockIdx.x * 128 + threadIdx.x) * VEC;
     const int y = blockIdx.y;
     const int b = b0 + blockIdx.z;   // 0 .. 2n-1
     if (x >= W) return;
-    const T* src = neigh + (int64_t)n_map.slot(b) * n_ss;
+    const T* src = neigh + n_map.offset(b, n_ss);
     const int64_t fpx = ((int64_t)b * H + y) * W + x;
     float v[VEC];
     if (VEC == 4) {
@@ -199,7 +199,7 @@ k_warp_pair(const T* __restrict__ neigh, int64_t n_ss, int64_t n_rs, SlotMap n_m
         v[0] = remap_px(src, n_rs, f.x, f.y, x, y, H, W);
     }
     if (b < n) {
-        float* ap = acc + (int64_t)b * a_ss + (int64_t)y * a_rs + x;
+        float* ap = acc + a_map.offset(b, a_ss) + (int64_t)y * a_rs + x;
         if (VEC == 4) {
             float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
             if (!first) a = *reinterpret_cast<float4*>(ap);
@@ -221,9 +221,12 @@ k_warp_pair(const T* __restrict__ neigh, int64_t n_ss, int64_t n_rs, SlotMap n_m
 
 template <typename T>
 int launch_warp_pair(const T* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_map, const float* flow, double weight,
-                     float* acc, int64_t a_ss, int64_t a_rs, T* stash, int n, int H, int W, int first, cudaStream_t st)
+                     float* acc, int64_t a_ss, int64_t a_rs, SlotMap a_map, T* stash, int n, int H, int W, int first,
+                     cudaStream_t st)
 {
+    // (the volume strides of a batch move every image's base: they must keep the 16-byte alignment too)
     const bool vec4 = W % 4 == 0 && n_ss % 4 == 0 && n_rs % 4 == 0 && a_ss % 4 == 0 && a_rs % 4 == 0 &&
+                      n_map.vstride % 4 == 0 && a_map.vstride % 4 == 0 &&
                       (reinterpret_cast<uintptr_t>(neigh) & 15) == 0 && (reinterpret_cast<uintptr_t>(acc) & 15) == 0 &&
                       (reinterpret_cast<uintptr_t>(flow) & 15) == 0 &&
                       (reinterpret_cast<uintptr_t>(stash) & (4 * sizeof(T) - 1)) == 0;
@@ -235,12 +238,12 @@ int launch_warp_pair(const T* neigh, int64_t n_ss, int64_t n_rs, SlotMap n_map, 
         ProfScope ps(K_WARP_ACC, (double)nb * H * W * (8.0 + es + (first ? 4.0 + es : 8.0 + es) / 2), st);
         if (vec4) {
             dim3 grid((unsigned)cdiv(W, 512), (unsigned)H, (unsigned)nb);
-            k_warp_pair<T, 4><<<grid, 128, 0, st>>>(neigh, n_ss, n_rs, n_map, flow, weight, acc, a_ss, a_rs, stash, n, b0, H,
-                                                    W, first);
+            k_warp_pair<T, 4><<<grid, 128, 0, st>>>(neigh, n_ss, n_rs, n_map, flow, weight, acc, a_ss, a_rs, a_map, stash, n,
+                                                    b0, H, W, first);
         } else {
             dim3 grid((unsigned)cdiv(W, 128), (unsigned)H, (unsigned)nb);
-            k_warp_pair<T, 1><<<grid, 128, 0, st>>>(neigh, n_ss, n_rs, n_map, flow, weight, acc, a_ss, a_rs, stash, n, b0, H,
-                                                    W, first);
+            k_warp_pair<T, 1><<<grid, 128, 0, st>>>(neigh, n_ss, n_rs, n_map, flow, weight, acc, a_ss, a_rs, a_map, stash, n,
+                                                    b0, H, W, first);
         }
         FDN_LAUNCHED("k_warp_pair");
     }
@@ -257,14 +260,15 @@ template <typename T, int VEC>
 __global__ void __launch_bounds__(128)
 k_acc_finish(const T* __restrict__ centre, int64_t c_ss, int64_t c_rs, SlotMap c_map, const T* __restrict__ stash,
              int64_t stash_stride, int r, FinishTaps taps, float* __restrict__ acc, int64_t a_ss, int64_t a_rs,
-             T* __restrict__ out, int64_t o_ss, int64_t o_rs, int b0, int H, int W, int have_acc)
+             SlotMap a_map, T* __restrict__ out, int64_t o_ss, int64_t o_rs, SlotMap o_map, int b0, int H, int W,
+             int have_acc)
 {
     const int x = (blockIdx.x * 128 + threadIdx.x) * VEC;
     const int y = blockIdx.y;
     const int b = b0 + blockIdx.z;
     if (x >= W) return;
-    const T* cp = centre + (int64_t)c_map.slot(b) * c_ss + (int64_t)y * c_rs + x;
-    float* ap = acc + (int64_t)b * a_ss + (int64_t)y * a_rs + x;
+    const T* cp = centre + c_map.offset(b, c_ss) + (int64_t)y * c_rs + x;
+    float* ap = acc + a_map.offset(b, a_ss) + (int64_t)y * a_rs + x;
     const T* sp = stash + ((int64_t)b * H + y) * W + x;
     float a[VEC], v[VEC];
     auto load = [&](const T* p, float* dst) {
@@ -298,7 +302,7 @@ k_acc_finish(const T* __restrict__ centre, int64_t c_ss, int64_t c_rs, SlotMap c
         if (VEC == 4) *reinterpret_cast<float4*>(ap) = make_float4(a[0], a[1 % VEC], a[2 % VEC], a[3 % VEC]);
         else *ap = a[0];
     } else {   // filtered_vol[z] = tmp_slice (:325): truncation toward zero
-        T* op = out + (int64_t)b * o_ss + (int64_t)y * o_rs + x;
+        T* op = out + o_map.offset(b, o_ss) + (int64_t)y * o_rs + x;
         if (VEC == 4) store4(op, a[0], a[1 % VEC], a[2 % VEC], a[3 % VEC]);
         else *op = store_cast<T>(a[0]);
     }
@@ -306,8 +310,8 @@ k_acc_finish(const T* __restrict__ centre, int64_t c_ss, int64_t c_rs, SlotMap c
 
 template <typename T>
 int launch_acc_finish(const T* centre, int64_t c_ss, int64_t c_rs, SlotMap c_map, const T* stash, int r, const double* k,
-                      float* acc, int64_t a_ss, int64_t a_rs, T* out, int64_t o_ss, int64_t o_rs, int n, int H, int W,
-                      int have_acc, cudaStream_t st)
+                      float* acc, int64_t a_ss, int64_t a_rs, SlotMap a_map, T* out, int64_t o_ss, int64_t o_rs,
+                      SlotMap o_map, int n, int H, int W, int have_acc, cudaStream_t st)
 {
     FDN_CHECK_ARG(r >= 0 && r <= FDN_MAX_R, "kernel radius %d unsupported (<= %d)", r, FDN_MAX_R);
     FDN_CHECK_ARG(H <= 65535, "image too tall for one launch");
@@ -316,9 +320,11 @@ int launch_acc_finish(const T* centre, int64_t c_ss, int64_t c_rs, SlotMap c_map
     FinishTaps taps;
     for (int i = 0; i <= r; i++) taps.k[i] = k[i];
     bool vec4 = W % 4 == 0 && c_ss % 4 == 0 && c_rs % 4 == 0 && a_ss % 4 == 0 && a_rs % 4 == 0 &&
+                c_map.vstride % 4 == 0 && a_map.vstride % 4 == 0 &&
                 (reinterpret_cast<uintptr_t>(centre) & al) == 0 && (reinterpret_cast<uintptr_t>(acc) & 15) == 0 &&
                 (reinterpret_cast<uintptr_t>(stash) & al) == 0;
-    if (typed) vec4 = vec4 && o_ss % 4 == 0 && o_rs % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & al) == 0;
+    if (typed)
+        vec4 = vec4 && o_ss % 4 == 0 && o_rs % 4 == 0 && o_map.vstride % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & al) == 0;
     const int64_t stash_stride = (int64_t)n * H * W;
     const double es = (double)sizeof(T);
     for (int b0 = 0; b0 < n; b0 += 65535) {
@@ -328,11 +334,11 @@ int launch_acc_finish(const T* centre, int64_t c_ss, int64_t c_rs, SlotMap c_map
         if (vec4) {
             dim3 grid((unsigned)cdiv(W, 512), (unsigned)H, (unsigned)nb);
             k_acc_finish<T, 4><<<grid, 128, 0, st>>>(centre, c_ss, c_rs, c_map, stash, stash_stride, r, taps, acc, a_ss, a_rs,
-                                                     out, o_ss, o_rs, b0, H, W, have_acc);
+                                                     a_map, out, o_ss, o_rs, o_map, b0, H, W, have_acc);
         } else {
             dim3 grid((unsigned)cdiv(W, 128), (unsigned)H, (unsigned)nb);
             k_acc_finish<T, 1><<<grid, 128, 0, st>>>(centre, c_ss, c_rs, c_map, stash, stash_stride, r, taps, acc, a_ss, a_rs,
-                                                     out, o_ss, o_rs, b0, H, W, have_acc);
+                                                     a_map, out, o_ss, o_rs, o_map, b0, H, W, have_acc);
         }
         FDN_LAUNCHED("k_acc_finish");
     }
@@ -488,9 +494,9 @@ int launch_copy3d(const T* in, int64_t in_sa, int64_t in_sb, int b0, int bw, int
 
 #define FDN_INST_WARP(T)                                                                                              \
     template int launch_warp_pair<T>(const T*, int64_t, int64_t, SlotMap, const float*, double, float*, int64_t, int64_t, \
-                                     T*, int, int, int, int, cudaStream_t);                                               \
+                                     SlotMap, T*, int, int, int, int, cudaStream_t);                                      \
     template int launch_acc_finish<T>(const T*, int64_t, int64_t, SlotMap, const T*, int, const double*, float*, int64_t, \
-                                      int64_t, T*, int64_t, int64_t, int, int, int, int, cudaStream_t);
+                                      int64_t, SlotMap, T*, int64_t, int64_t, SlotMap, int, int, int, int, cudaStream_t);
 FDN_INST_WARP(float)
 FDN_INST_WARP(uint8_t)
 FDN_INST_WARP(uint16_t)

@@ -100,6 +100,7 @@ class DeviceEngine:
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.workspace_limit_bytes = workspace_limit_bytes
         self._ws = None
+        self.sub_batch = None   # volumes per device call of the last filter_batch (0: one at a time, chunked)
 
     # ---- workspace ----
     def _workspace(self, nbytes: int):
@@ -336,6 +337,104 @@ class DeviceEngine:
         self.filter_view(vt, ot, v, kernels[2], flow, chunk, exact)
         out = self.transpose_yx(ot, a.view(Z, Y, X))
         return b, out
+
+    # ---- a batch of same-shape volumes [B, Z, Y, X] (subtomograms, montage tiles) ----
+    @staticmethod
+    def _batch_views(Z: int, Y: int, X: int):
+        """Views of the Z, Y and X pass of one volume; the X pass runs on the [Z, X, Y] transpose."""
+        return (View(Z, Z, 0, 1, Y, X, Y * X, X, Y * X, X), View(Y, Y, 0, 1, Z, X, X, Y * X, X, Y * X),
+                View(X, X, 0, 1, Z, Y, Y, X * Y, Y, X * Y))
+
+    def _pick_batch(self, views, klens, ofp: OfParams, B: int) -> int:
+        """Most volumes per device call whose workspace fits the limit (the rule of _pick_chunk: 85 % of free HBM,
+        or workspace_limit_bytes); 0 when not even one whole volume fits."""
+        need = lambda b: max(self.lib.fdn_workspace_bytes_batch(C.byref(v), b, k, C.byref(ofp))
+                             for v, k in zip(views, klens))
+        full = need(B)
+        if full == 0:
+            _lib.check(1)
+        limit = self.workspace_limit_bytes
+        if limit is None:
+            have = self._ws.numel() if self._ws is not None else 0
+            if full <= have:
+                return B    # the workspace this engine holds is enough: no driver query
+            free, _total = self.torch.cuda.mem_get_info(self.device)
+            limit = int((free + have) * 0.85)
+        if full <= limit:
+            return B
+        if need(1) > limit:
+            return 0
+        lo, hi = 1, B
+        while lo < hi:
+            mid = (lo + hi + 1) // 2
+            if need(mid) <= limit:
+                lo = mid
+            else:
+                hi = mid - 1
+        return lo
+
+    def filter_batch(self, vols, kernels: Sequence, flow: Optional[FlowParams], exact: bool = True):
+        """DeviceEngine.filter for each volume of a contiguous float32 batch [B, Z, Y, X], many volumes per device
+        call. Returns (zy, zyx) [B, Z, Y, X] with filter's buffer roles; volume g of each equals filter(vols[g]) bit
+        for bit. The batch runs in sub-batches whose workspace fits (sub_batch holds the size last used); a volume
+        too large to go whole through the batched pass runs through filter (chunked)."""
+        torch = self.torch
+        if not (vols.is_cuda and vols.dim() == 4 and vols.is_contiguous() and vols.dtype == torch.float32):
+            raise ValueError("expected a contiguous float32 CUDA tensor [B, Z, Y, X]")
+        B, Z, Y, X = (int(s) for s in vols.shape)
+        ks = [_taps(k) for k in kernels]
+        vs = Z * Y * X
+        zy = torch.empty_like(vols)
+        a = torch.empty_like(vols)
+        if flow is None:
+            self.sub_batch = B
+            out = torch.empty_like(vols)
+            vz = self._batch_views(Z, Y, X)[0]
+            with torch.cuda.device(self.device):
+                st = _stream_ptr(torch)
+                _lib.check(self.lib.fdn_gauss_axis_batch(vols.data_ptr(), a.data_ptr(), C.byref(vz), B, vs, vs,
+                                                         ks[0][1], ks[0][0].size, int(bool(exact)), st))
+                # the Y pass of [B, Z, Y, X] is the Y pass of a [B*Z, Y, X] volume (at most 65535 rows per launch)
+                per = max(1, 65535 // Z)
+                for g0 in range(0, B, per):
+                    nb = min(per, B - g0)
+                    vy = View(Y, Y, 0, 1, nb * Z, X, X, Y * X, X, Y * X)
+                    _lib.check(self.lib.fdn_gauss_axis(a[g0].data_ptr(), zy[g0].data_ptr(), C.byref(vy), ks[1][1],
+                                                       ks[1][0].size, int(bool(exact)), st))
+                # and the X pass the rows of B*Z*Y
+                _lib.check(self.lib.fdn_gauss_rows(zy.data_ptr(), out.data_ptr(), B * Z * Y, X, ks[2][1],
+                                                   ks[2][0].size, int(bool(exact)), st))
+            return zy, out
+        views = self._batch_views(Z, Y, X)
+        ofp = flow.c_struct()
+        with torch.cuda.device(self.device):
+            sb = self._pick_batch(views, [k.size for k, _ in ks], ofp, B)
+            self.sub_batch = sb
+            if sb == 0:     # one volume does not fit whole: the chunked single-volume path
+                for g in range(B):
+                    z1, o1 = self.filter(vols[g], kernels, flow, exact=exact)
+                    zy[g].copy_(z1)
+                    a[g].copy_(o1)
+                    del z1, o1
+                return zy, a
+            ot = torch.empty((B, Z, X, Y), dtype=torch.float32, device=vols.device)   # (not needed by the fallback)
+            nbytes = max(self.lib.fdn_workspace_bytes_batch(C.byref(v), sb, k.size, C.byref(ofp))
+                         for v, (k, _) in zip(views, ks))
+            ws = self._workspace(nbytes)
+            st = _stream_ptr(torch)
+            for g0 in range(0, B, sb):
+                nb = min(sb, B - g0)
+                run = lambda src, dst, v, k: _lib.check(self.lib.fdn_filter_axis_batch(
+                    src.data_ptr(), dst.data_ptr(), C.byref(v), nb, vs, vs, k[1], k[0].size, C.byref(ofp),
+                    ws.data_ptr(), ws.numel(), st))
+                run(vols[g0], a[g0], views[0], ks[0])
+                run(a[g0], zy[g0], views[1], ks[1])                                  # zy = Z+Y
+                # X pass on the [Z, X, Y] transposes: `a` (the Z result) is dead now and holds first the transposed
+                # input, then the final result
+                vt = self.transpose_yx(zy[g0:g0 + nb].view(nb * Z, Y, X), a[g0:g0 + nb].view(nb * Z, X, Y))
+                run(vt, ot[g0], views[2], ks[2])
+                self.transpose_yx(ot[g0:g0 + nb].view(nb * Z, X, Y), a[g0:g0 + nb].view(nb * Z, Y, X))
+        return zy, a
 
     # ---- building blocks exposed for the module-level functions and the parity tests ----
     def farneback(self, prev, nxt, flow_init, params: FlowParams):

@@ -825,6 +825,64 @@ class FlowDenoising(GaussianDenoising):
                                        bool(gaussian_window))
 
 
+class _Stack:
+    """A sequence of same-shape 3-D host arrays seen as one [n, Z, Y, X] array by the staging upload (slices along the
+    first axis are stacked when the staging copy asks for them: no host copy of the whole batch)."""
+
+    def __init__(self, items):
+        self.items = items
+        self.shape = (len(items),) + tuple(int(s) for s in items[0].shape)
+
+    def __getitem__(self, sl):
+        return np.stack([np.asarray(v, dtype=np.float32) for v in self.items[sl]])
+
+    def __array__(self, dtype=None, copy=None):
+        return self[0:len(self.items)] if dtype is None else self[0:len(self.items)].astype(dtype)
+
+
+def filter_volumes(vols, kernels, l=OF_LEVELS, w=OF_WINDOW_SIZE, get_flow=get_flow_with_prev_flow, no_OF=False,
+                   iterations=OF_ITERS, poly_n=OF_POLY_N, poly_sigma=OF_POLY_SIGMA, gaussian_window=False, exact=True):
+    '''Z+Y+X results of many volumes (subtomograms, montage tiles): a 4-D host array [n, Z, Y, X] or a sequence of 3-D
+    host arrays, any dtype NumPy casts (filtered as float32, like FlowDenoising(...).filter). Volumes of one shape are
+    filtered together, many per device call (DeviceEngine.filter_batch); each result equals
+    FlowDenoising(1, vol, ...).filter(kernels) (GaussianDenoising with no_OF) on that volume alone, bit for bit.
+    Returns a list of float32 arrays in input order. Not part of the reference's surface.'''
+    items = list(vols)
+    for v in items:
+        if np.ndim(v) != 3:
+            raise ValueError("every volume must be a 3-D array (Z, Y, X)")
+    ks = [np.asarray(k, np.float64) for k in kernels]
+    for k in ks:
+        assert k.size % 2 != 0  # kernel.size must be odd (src/flowdenoising.py:309)
+    flow = None if no_OF else FlowParams(int(l), int(w), int(iterations), int(poly_n), float(poly_sigma),
+                                         get_flow is not get_flow_without_prev_flow, bool(gaussian_window))
+    groups = {}
+    for i, v in enumerate(items):
+        groups.setdefault(tuple(int(s) for s in np.shape(v)), []).append(i)
+    results = [None] * len(items)
+    if not items:
+        return results
+    eng = _get_engine()
+    torch = eng.torch
+    for shape, idx in groups.items():
+        # host sub-batches: the batch, its Z result / Z+Y / transposed buffers take 16 bytes per voxel of the device;
+        # up to a quarter of the free memory goes to them, the rest to the workspace (filter_batch splits further)
+        free, _total = torch.cuda.mem_get_info(eng.device)
+        per_vol = 16 * int(np.prod(shape))
+        n = max(1, min(len(idx), int(0.25 * free) // per_vol))
+        for j0 in range(0, len(idx), n):
+            part = idx[j0:j0 + n]
+            d = _upload_volume(_Stack([items[i] for i in part]), torch, eng.device)
+            _zy, zyx = eng.filter_batch(d, ks, flow, exact=exact)
+            res = np.empty((len(part),) + shape, np.float32)
+            dl = _Download(zyx, res, torch)
+            dl.wait()
+            del d, _zy, zyx
+            for j, i in enumerate(part):
+                results[i] = res[j]
+    return results
+
+
 def int_or_str(text):
     '''Helper function for argument parsing.'''
     try:
@@ -888,6 +946,12 @@ def build_parser():
     parser.add_argument("--compat_zy_output", action="store_true",
                         help="Write the Z+Y intermediate like the reference CLI does (flowdenoising.py:520) "
                              "instead of the full Z+Y+X result")
+    parser.add_argument("--inputs", nargs="+", default=None, metavar="FILE",
+                        help="Filter many MRC / TIFF volumes (subtomograms, montage tiles); volumes of one shape run "
+                             "together, many per device call. Each result is written as --output_dir/<basename> "
+                             "(float32). Instead of -i / -o")
+    parser.add_argument("--output_dir", default=None, metavar="DIR",
+                        help="Directory of the --inputs results (created if missing)")
     return parser
 
 
@@ -933,6 +997,8 @@ def main(argv=None):
     if len(sigma) != 3:
         parser.error("--sigma takes one or three values (Z, Y, X)")
     logging.info(f"sigma={tuple(sigma)}")
+    if args.inputs is not None or args.output_dir is not None:
+        return _main_batch(args, argv, sigma, get_flow)
 
     logging.info(f"reading \"{args.input}\"")
     time_0 = time.perf_counter()
@@ -996,6 +1062,46 @@ def main(argv=None):
     else:
         volume_io.write_volume(args.output, np.asarray(filtered_vol, dtype=np.float32))
     logging.info(f"written \"{args.output}\" in {time.perf_counter() - time_0} seconds")
+    return 0
+
+
+def _main_batch(args, argv, sigma, get_flow):
+    """--inputs / --output_dir: every input filtered with filter_volumes, written as output_dir/<basename>."""
+    from . import volume_io
+    if args.inputs is None:
+        parser.error("--output_dir needs --inputs")
+    if args.output_dir is None:
+        parser.error("--inputs needs --output_dir")
+    probe = build_parser()
+    probe.set_defaults(input=argparse.SUPPRESS, output=argparse.SUPPRESS)
+    explicit = probe.parse_args(argv)
+    if explicit.input != argparse.SUPPRESS or explicit.output != argparse.SUPPRESS:
+        parser.error("--inputs replaces -i / -o (results go to --output_dir)")
+    for flag, bad in (("-m", args.memory_map), ("--gpus > 1", args.gpus > 1), ("--border mean", args.border != "wrap"),
+                      ("--slab_slices", args.slab_slices is not None), ("--keep_dtype", args.keep_dtype),
+                      ("--compat_zy_output", args.compat_zy_output)):
+        if bad:
+            parser.error(f"--inputs does not support {flag} (in-core float32 volumes on one GPU)")
+    names = [os.path.basename(p) for p in args.inputs]
+    if len(set(names)) != len(names):
+        dup = sorted({n for n in names if names.count(n) > 1})
+        parser.error(f"--inputs: several inputs share a basename ({', '.join(dup)}); their results would collide")
+    vols = []
+    for p in args.inputs:
+        logging.info(f"reading \"{p}\"")
+        vols.append(np.ascontiguousarray(volume_io.read_volume(p), dtype=np.float32))
+    kernels = [get_gaussian_kernel(s) for s in sigma]
+    logging.info(f"Filtering {len(vols)} volumes ...")
+    time_0 = time.perf_counter()
+    results = filter_volumes(vols, kernels, args.levels, args.winsize, get_flow, no_OF=args.no_OF,
+                             iterations=args.iterations, poly_n=args.poly_n, poly_sigma=args.poly_sigma,
+                             gaussian_window=args.gaussian_window)
+    logging.info(f"{len(vols)} volumes filtered in {time.perf_counter() - time_0} seconds")
+    os.makedirs(args.output_dir, exist_ok=True)
+    for name, res in zip(names, results):
+        out = os.path.join(args.output_dir, name)
+        logging.info(f"writing \"{out}\"")
+        volume_io.write_volume(out, np.asarray(res, dtype=np.float32))
     return 0
 
 

@@ -81,6 +81,8 @@ typedef struct fdn_view {
 } fdn_view;
 
 /* ---- library / error handling ---- */
+/* 101. The batch entry points (fdn_workspace_bytes_batch, fdn_filter_axis_batch, fdn_gauss_axis_batch) were added
+ * without a version change: a caller that needs them looks them up with dlsym. */
 int fdn_version(void);
 const char* fdn_last_error(void);
 /* Number of this library's kernel launches since the last reset (bench.py "gpu_launches"). */
@@ -145,6 +147,22 @@ int fdn_gauss_rows(const float* d_in, float* d_out, int64_t n_rows, int W, const
                    int exact, void* stream);
 /* Batched 2-D transpose of the last two axes: in [n][A][B] -> out [n][B][A]. */
 int fdn_transpose_yx(const float* d_in, float* d_out, int n, int A, int B, void* stream);
+
+/* ---- batches of same-shape volumes (subtomograms, montage tiles): the loop of the reference's
+ * GaussianDenoising.filter_along_{Z,Y,X} (src/flowdenoising.py:175-283) run for many volumes in one device pass ----
+ * A batch of `batch` volumes of one shape. Volume g's view (whole periodic axis: periodic = 1, halo = 0,
+ * n_out = n_in) starts at d_in + g*in_batch_stride and d_out + g*out_batch_stride (elements). Volume g's result
+ * equals fdn_filter_axis / fdn_gauss_axis on that volume alone, bit for bit. Every launch carries the image pairs of
+ * all volumes, so the launch count of a pass does not grow with the batch. Rejected with FDN_ERR_INVALID before
+ * anything is launched: batch < 1, a view that is not a whole periodic axis, a kernel longer than FDN_MAX_KLEN, bad
+ * optical-flow parameters (as fdn_filter_axis), more than 2^31 - 1 image pairs (2 * batch * n_in) in one launch.
+ * fdn_workspace_bytes_batch returns 0 for any of these. Progress counts batch * n_out slices per pass. */
+size_t fdn_workspace_bytes_batch(const fdn_view* view, int batch, int klen, const fdn_of_params* of);
+int fdn_filter_axis_batch(const float* d_in, float* d_out, const fdn_view* view, int batch, int64_t in_batch_stride,
+                          int64_t out_batch_stride, const double* kernel, int klen, const fdn_of_params* of,
+                          void* d_workspace, size_t workspace_bytes, void* stream);
+int fdn_gauss_axis_batch(const float* d_in, float* d_out, const fdn_view* view, int batch, int64_t in_batch_stride,
+                         int64_t out_batch_stride, const double* kernel, int klen, int exact, void* stream);
 
 /* ---- typed volumes: the reference's integer semantics (SURVEY App. B Q3) ----
  * An integer volume keeps its dtype through a pass in the reference: cv2.remap of an integer neighbour returns an
