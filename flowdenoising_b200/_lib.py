@@ -27,6 +27,9 @@ FARNEBACK_GAUSSIAN = 256   # FDN_OF_FARNEBACK_GAUSSIAN (= cv2.OPTFLOW_FARNEBACK_
 # FDN_DTYPE_*: element types of typed volumes (the reference's integer semantics, opt-in)
 DTYPE_F32, DTYPE_U8, DTYPE_I8, DTYPE_U16, DTYPE_I16 = 0, 1, 2, 3, 4
 
+# FDN_BORDER_*: the border along a pass's axis (fdn_view.periodic, fdn_gauss_rows_border)
+BORDER_WRAP, BORDER_REFLECT, BORDER_MIRROR, BORDER_NEAREST = 1, 2, 3, 4
+
 
 class View(C.Structure):
     """struct fdn_view."""
@@ -102,6 +105,8 @@ SIGNATURES = {
                                        C.c_int, C.c_void_p]),
     "fdn_gauss_rows_typed": (C.c_int, [c_f32p, c_f32p, C.c_int, c_i64, C.c_int, C.POINTER(C.c_double), C.c_int,
                                        C.c_int, C.c_void_p]),
+    "fdn_gauss_rows_border": (C.c_int, [c_f32p, c_f32p, C.c_int, c_i64, C.c_int, C.POINTER(C.c_double), C.c_int,
+                                        C.c_int, C.c_int, C.c_void_p]),
     "fdn_transpose_yx_typed": (C.c_int, [c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "fdn_remap_typed": (C.c_int, [c_f32p, c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "fdn_transpose_strided_typed": (C.c_int, [c_f32p, C.c_int, c_i64, c_i64, c_f32p, c_i64, c_i64, C.c_int, C.c_int,

@@ -127,6 +127,14 @@ static int make_geometry(int H, int W, int levels, Geometry* g)
     return FDN_OK;
 }
 
+// the border arithmetic (border_index: periods up to 2 n) stays inside int
+static int check_border_extent(int periodic, int64_t n)
+{
+    FDN_CHECK_ARG(view_border(periodic) == FDN_BORDER_WRAP || n <= (1 << 30),
+                  "border %d needs an axis of at most 2^30 slices (%lld)", periodic, (long long)n);
+    return FDN_OK;
+}
+
 static int check_of(const fdn_of_params* of)
 {
     FDN_CHECK_ARG(of->winsize >= 1 && of->winsize <= 31, "winsize %d unsupported (1..31)", of->winsize);
@@ -261,6 +269,7 @@ static int make_plan(const fdn_view& v, int klen, const fdn_of_params& of, int c
                       "non-periodic view needs >= r halo slices on both sides (r=%d, halo=%d, n_in=%d, n_out=%d)",
                       p->r, v.halo, v.n_in, v.n_out);
     }
+    if ((rc = check_border_extent(v.periodic, v.n_in))) return rc;
     if ((rc = check_of(&of))) return rc;
     if ((rc = make_geometry(v.H, v.W, of.levels, &p->g))) return rc;
     FDN_CHECK_ARG(batch >= 1, "batch must be >= 1");
@@ -323,6 +332,7 @@ static int filter_axis_of(const T* d_in, T* d_out, const fdn_view& v, const doub
     PolyConsts pc;
     prepare_poly_consts(of.poly_n, of.poly_sigma, &pc);
     const int wrap_in = v.periodic ? v.n_in : 0;
+    const int border = view_border(v.periodic);   // of every map below that wraps (input slices, full_wrap R slots)
     const int64_t R_vs = (int64_t)p.slots * p.g.R_slot;   // R-cache floats per volume
     bool cache_full = false;
 
@@ -339,6 +349,7 @@ static int filter_axis_of(const T* d_in, T* d_out, const fdn_view& v, const doub
             for (int sb = 0; sb < batch * need; sb += batch * p.chunk) {
                 const int nb = batch * need - sb < batch * p.chunk ? batch * need - sb : batch * p.chunk;
                 SlotMap in_map{p.full_wrap ? sb : ubase + sb, wrap_in};
+                in_map.border = border;
                 in_map.per = need;
                 in_map.vstride = in_bs;
                 SlotMap R_map{sb, 0};
@@ -356,6 +367,7 @@ static int filter_axis_of(const T* d_in, T* d_out, const fdn_view& v, const doub
         // every map below resolves image j of a chain to volume j / C, slice j % C (one volume: always volume 0)
         auto vmap = [&](int b1, int wrap, int split, int b2, int64_t vstride) {
             SlotMap m{b1, wrap, split, b2};
+            m.border = border;
             m.per = C;
             m.vstride = vstride;
             return m;
@@ -610,6 +622,8 @@ int fdn_gauss_axis_batch(const float* d_in, float* d_out, const fdn_view* view, 
     FDN_CHECK_ARG(v.n_in >= 1 && v.H >= 1 && v.W >= 1, "empty view");
     FDN_CHECK_ARG(v.periodic && v.halo == 0 && v.n_out == v.n_in,
                   "a batch member must be a whole periodic axis (periodic = 1, halo = 0, n_out = n_in)");
+    int rc0;
+    if ((rc0 = check_border_extent(v.periodic, v.n_in))) return rc0;
     const cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int rc = launch_gauss_axis(d_in, d_out, v, kernel, klen, exact, st, batch, in_batch_stride, out_batch_stride);
     if (rc == FDN_OK) progress_add(st, 1000ll * batch * v.n_out);
@@ -666,6 +680,7 @@ int fdn_gauss_axis_typed(const void* d_in, void* d_out, int dtype, const fdn_vie
     if (v.periodic) FDN_CHECK_ARG(v.halo >= 0 && v.halo < v.n_in && v.n_out <= v.n_in,
                                   "periodic views need 0 <= halo < n_in and n_out <= n_in");
     else FDN_CHECK_ARG(v.halo >= klen / 2 && v.n_in >= v.n_out + v.halo + klen / 2, "halo too small");
+    if ((rc = check_border_extent(v.periodic, v.n_in))) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     switch (dtype) {
         case FDN_DTYPE_U8:
@@ -689,27 +704,38 @@ int fdn_gauss_axis_typed(const void* d_in, void* d_out, int dtype, const fdn_vie
 int fdn_gauss_rows_typed(const void* d_in, void* d_out, int dtype, int64_t n_rows, int W, const double* kernel, int klen,
                          int exact, void* stream)
 {
+    return fdn_gauss_rows_border(d_in, d_out, dtype, n_rows, W, kernel, klen, exact, FDN_BORDER_WRAP, stream);
+}
+
+int fdn_gauss_rows_border(const void* d_in, void* d_out, int dtype, int64_t n_rows, int W, const double* kernel,
+                          int klen, int exact, int border, void* stream)
+{
     int rc;
+    FDN_CHECK_ARG(border >= FDN_BORDER_WRAP && border <= FDN_BORDER_NEAREST,
+                  "unknown border %d (FDN_BORDER_WRAP, _REFLECT, _MIRROR or _NEAREST)", border);
+    if ((rc = check_border_extent(border, W))) return rc;
     if ((rc = check_dtype(dtype, false))) return rc;
-    if (dtype == FDN_DTYPE_F32)
-        return fdn_gauss_rows(static_cast<const float*>(d_in), static_cast<float*>(d_out), n_rows, W, kernel, klen, exact,
-                              stream);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (dtype == FDN_DTYPE_F32) {
+        FDN_CHECK_ARG(d_in && d_out && kernel && n_rows >= 1 && W >= 1, "bad argument");
+        return launch_gauss_rows(static_cast<const float*>(d_in), static_cast<float*>(d_out), n_rows, W, kernel, klen,
+                                 exact, st, border);
+    }
     FDN_CHECK_ARG(exact, "typed volumes run the exact no-OF arithmetic only (the fast mode moves truncation boundaries)");
     FDN_CHECK_ARG(d_in && d_out && kernel && n_rows >= 1 && W >= 1, "bad argument");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
     switch (dtype) {
         case FDN_DTYPE_U8:
             return launch_gauss_rows_typed(static_cast<const uint8_t*>(d_in), static_cast<uint8_t*>(d_out), n_rows, W, kernel,
-                                           klen, st);
+                                           klen, st, border);
         case FDN_DTYPE_I8:
             return launch_gauss_rows_typed(static_cast<const int8_t*>(d_in), static_cast<int8_t*>(d_out), n_rows, W, kernel,
-                                           klen, st);
+                                           klen, st, border);
         case FDN_DTYPE_U16:
             return launch_gauss_rows_typed(static_cast<const uint16_t*>(d_in), static_cast<uint16_t*>(d_out), n_rows, W,
-                                           kernel, klen, st);
+                                           kernel, klen, st, border);
         default:
             return launch_gauss_rows_typed(static_cast<const int16_t*>(d_in), static_cast<int16_t*>(d_out), n_rows, W, kernel,
-                                           klen, st);
+                                           klen, st, border);
     }
 }
 
@@ -757,7 +783,9 @@ int fdn_gauss_axis(const float* d_in, float* d_out, const fdn_view* view, const 
     if (v.periodic) FDN_CHECK_ARG(v.halo >= 0 && v.halo < v.n_in && v.n_out <= v.n_in,
                                   "periodic views need 0 <= halo < n_in and n_out <= n_in");
     else FDN_CHECK_ARG(v.halo >= klen / 2 && v.n_in >= v.n_out + v.halo + klen / 2, "halo too small");
-    int rc = launch_gauss_axis(d_in, d_out, v, kernel, klen, exact, static_cast<cudaStream_t>(stream));
+    int rc;
+    if ((rc = check_border_extent(v.periodic, v.n_in))) return rc;
+    rc = launch_gauss_axis(d_in, d_out, v, kernel, klen, exact, static_cast<cudaStream_t>(stream));
     if (rc == FDN_OK) progress_add(static_cast<cudaStream_t>(stream), 1000ll * v.n_out);
     return rc;
 }

@@ -84,9 +84,34 @@ struct BlurTaps {
 };
 int prepare_blur_taps(int ksz, double sigma, BlurTaps* bt);
 
+// ---- borders along a pass's axis (FDN_BORDER_*, include/fdn_b200.h) ----
+// fdn_view.periodic -> the border its periodic indices take (every nonzero value but the three named modes wraps)
+static inline int view_border(int periodic)
+{
+    return (periodic == FDN_BORDER_REFLECT || periodic == FDN_BORDER_MIRROR || periodic == FDN_BORDER_NEAREST)
+               ? periodic : FDN_BORDER_WRAP;
+}
+// slice of an axis of n (1 <= n <= 2^30) that index i maps to under `border`; an index inside [0, n) maps to itself
+__host__ __device__ __forceinline__ int border_index(int i, int n, int border)
+{
+    if ((unsigned)i < (unsigned)n) return i;
+    if (border == FDN_BORDER_NEAREST) return i < 0 ? 0 : n - 1;
+    if (border == FDN_BORDER_REFLECT || border == FDN_BORDER_MIRROR) {
+        if (n == 1) return 0;
+        const int p = border == FDN_BORDER_REFLECT ? 2 * n : 2 * n - 2;
+        int j = i % p;
+        if (j < 0) j += p;
+        return j < n ? j : (border == FDN_BORDER_REFLECT ? p - 1 - j : p - j);
+    }
+    int j = i % n;
+    if (j < 0) j += n;
+    return j;
+}
+
 // Batch addressing of cached per-slice data: image b of a launch lives in slot
-//   s = base + b            (wrap == 0)
-//   s = (base + b) mod wrap (wrap  > 0)
+//   s = base + b                          (wrap == 0)
+//   s = (base + b) mod wrap               (wrap  > 0, border == FDN_BORDER_WRAP)
+//   s = border_index(base + b, wrap, border) (wrap > 0, another border)
 // A batch may be the concatenation of two runs (the backward and the forward chain of a pass advance together):
 // images b >= split continue at base2 + (b - split).
 // A run may span several volumes of a batch (fdn_filter_axis_batch): image j of a run belongs to volume j / per, and
@@ -98,6 +123,7 @@ struct SlotMap {
     int per = 0x7fffffff;
     int64_t vstride = 0;
     int b0 = 0;
+    int border = FDN_BORDER_WRAP;
     // element (or float) offset of image b's data: slot * stride + volume * vstride
     __host__ __device__ inline int64_t offset(int b, int64_t stride) const
     {
@@ -108,8 +134,12 @@ struct SlotMap {
         j -= g * per;
         int s = (first ? base : base2) + j;
         if (wrap > 0) {
-            s %= wrap;
-            if (s < 0) s += wrap;
+            if (border == FDN_BORDER_WRAP) {
+                s %= wrap;
+                if (s < 0) s += wrap;
+            } else {
+                s = border_index(s, wrap, border);
+            }
         }
         return (int64_t)s * stride + (int64_t)g * vstride;
     }
@@ -182,16 +212,18 @@ int launch_acc_finish(const T* centre, int64_t c_ss, int64_t c_rs, SlotMap c_map
 template <typename T>
 int launch_remap(const T* src, const float* flow, T* dst, int n, int H, int W, cudaStream_t st);
 // no-OF
-// batch volumes of view v, volume g at in + g * in_bs / out + g * out_bs (elements)
+// batch volumes of view v, volume g at in + g * in_bs / out + g * out_bs (elements); v.periodic selects the border
 int launch_gauss_axis(const float* in, float* out, const fdn_view& v, const double* k, int klen, int exact,
                       cudaStream_t st, int batch = 1, int64_t in_bs = 0, int64_t out_bs = 0);
+// border: FDN_BORDER_* at both ends of every row
 int launch_gauss_rows(const float* in, float* out, int64_t rows, int W, const double* k, int klen, int exact,
-                      cudaStream_t st);
+                      cudaStream_t st, int border = FDN_BORDER_WRAP);
 // typed no-OF passes: T in, T out, exact arithmetic only, truncated store
 template <typename T>
 int launch_gauss_axis_typed(const T* in, T* out, const fdn_view& v, const double* k, int klen, cudaStream_t st);
 template <typename T>
-int launch_gauss_rows_typed(const T* in, T* out, int64_t rows, int W, const double* k, int klen, cudaStream_t st);
+int launch_gauss_rows_typed(const T* in, T* out, int64_t rows, int W, const double* k, int klen, cudaStream_t st,
+                            int border);
 template <typename T>
 int launch_transpose(const T* in, T* out, int n, int A, int B, cudaStream_t st);
 template <typename T>

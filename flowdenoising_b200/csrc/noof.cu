@@ -92,7 +92,9 @@ static bool taps_benign(const double* k, int n)
 // the typed volumes (T = uint8 / int8 / uint16 / int16, exact mode only): every input is converted to float32 as
 // NumPy does for `int_slice * kernel[i]`, the float32 sum is truncated toward zero into T once, at the store.
 // ------------------------------------------------------------------------------------------------
-template <typename T, bool EXACT>
+// BORDERED: the view's indices take the border v.periodic (FDN_BORDER_REFLECT, _MIRROR or _NEAREST) instead of the wrap
+// (the wrap instantiations are the kernels of the periodic pass, unchanged)
+template <typename T, bool EXACT, bool BORDERED>
 __global__ void __launch_bounds__(256)
 k_gauss_axis(const T* __restrict__ in, T* __restrict__ out, fdn_view v, Taps64 t64, Taps32 t32, int64_t in_bs,
              int64_t out_bs)
@@ -110,7 +112,9 @@ k_gauss_axis(const T* __restrict__ in, T* __restrict__ out, fdn_view v, Taps64 t
     float acc = 0.f;
     for (int i = 0; i < klen; i++) {
         int j = s + v.halo + i - r;
-        if (v.periodic) {
+        if (BORDERED) {
+            j = border_index(j, v.n_in, v.periodic);
+        } else if (v.periodic) {
             j %= v.n_in;
             if (j < 0) j += v.n_in;
         }
@@ -122,9 +126,10 @@ k_gauss_axis(const T* __restrict__ in, T* __restrict__ out, fdn_view v, Taps64 t
 }
 
 #define GR_TILE 512
-template <typename T, bool EXACT>
+// BORDERED: both row ends take `border` (FDN_BORDER_REFLECT, _MIRROR or _NEAREST) instead of the wrap
+template <typename T, bool EXACT, bool BORDERED>
 __global__ void __launch_bounds__(256)
-k_gauss_rows(const T* __restrict__ in, T* __restrict__ out, int W, Taps64 t64, Taps32 t32)
+k_gauss_rows(const T* __restrict__ in, T* __restrict__ out, int W, Taps64 t64, Taps32 t32, int border)
 {
     extern __shared__ float s_seg[];  // GR_TILE + klen - 1
     const int klen = EXACT ? t64.klen : t32.klen;
@@ -134,8 +139,13 @@ k_gauss_rows(const T* __restrict__ in, T* __restrict__ out, int W, Taps64 t64, T
     const T* src = in + row * W;
     const int nload = min(GR_TILE, W - x0) + 2 * r;
     for (int i = threadIdx.x; i < nload; i += 256) {
-        int j = (x0 - r + i) % W;
-        if (j < 0) j += W;
+        int j;
+        if (BORDERED) {
+            j = border_index(x0 - r + i, W, border);
+        } else {
+            j = (x0 - r + i) % W;
+            if (j < 0) j += W;
+        }
         s_seg[i] = (float)src[j];
     }
     __syncthreads();
@@ -167,7 +177,7 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" :: "n"(N) : "memory"); }
 
-template <int KLEN, bool EXACT, int VEC>
+template <int KLEN, bool EXACT, int VEC, bool BORDERED>
 __global__ void __launch_bounds__(128)
 k_gauss_axis_ring(const float* __restrict__ in, float* __restrict__ out, fdn_view v, TapsW<KLEN> taps, int int_rounding,
                   int nseg, int64_t in_bs, int64_t out_bs)
@@ -191,18 +201,24 @@ k_gauss_axis_ring(const float* __restrict__ in, float* __restrict__ out, fdn_vie
 
     // q-th input of the segment (q = 0 .. n_in_seg - 1) <-> view slice s0 - R + q (+ halo, periodic wrap). The copies
     // are issued in order of q: the next slice index and its address advance incrementally (no division per copy).
+    // BORDERED (v.periodic: FDN_BORDER_REFLECT, _MIRROR or _NEAREST): each copy maps its index, which costs a compare
+    // inside the axis and a division only for the r slices beyond either end.
     int jn = s0 - R + v.halo;
-    if (v.periodic) {
+    if (!BORDERED && v.periodic) {
         jn %= v.n_in;
         if (jn < 0) jn += v.n_in;
     }
+    const int u0 = jn;
     const float* pn = src + (int64_t)jn * v.in_slice_stride;
     int qn = 0;
     auto issue = [&]() {
         if (qn < n_in_seg) {
+            if (BORDERED) pn = src + (int64_t)border_index(u0 + qn, v.n_in, v.periodic) * v.in_slice_stride;
             cp_async_thread<4 * VEC>(&ring[qn % GA_DEPTH][t], pn);
-            pn += v.in_slice_stride;
-            if (++jn == v.n_in && v.periodic) { jn = 0; pn = src; }
+            if (!BORDERED) {
+                pn += v.in_slice_stride;
+                if (++jn == v.n_in && v.periodic) { jn = 0; pn = src; }
+            }
         }
         ++qn;
         cp_async_commit();      // one group per q, empty past the end: wait_group counts stay uniform
@@ -282,7 +298,7 @@ k_gauss_axis_ring(const float* __restrict__ in, float* __restrict__ out, fdn_vie
     cp_async_wait<0>();
 }
 
-template <int KLEN>
+template <int KLEN, bool BD>
 static int launch_gauss_axis_ring(const float* in, float* out, const fdn_view& v, const double* k, int exact,
                                   cudaStream_t st, int batch, int64_t in_bs, int64_t out_bs)
 {
@@ -308,32 +324,30 @@ static int launch_gauss_axis_ring(const float* in, float* out, const fdn_view& v
         dim3 grid((unsigned)cdiv(v.W, 128 * vec), (unsigned)v.H, (unsigned)(nb * nseg));
         ProfScope ps(K_GAUSS_AXIS, 8.0 * nb * v.n_out * v.H * v.W, st);
         if (exact) {
-            if (vec == 2) k_gauss_axis_ring<KLEN, true, 2><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
-            else k_gauss_axis_ring<KLEN, true, 1><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
+            if (vec == 2) k_gauss_axis_ring<KLEN, true, 2, BD><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
+            else k_gauss_axis_ring<KLEN, true, 1, BD><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
         } else {
-            if (vec == 4) k_gauss_axis_ring<KLEN, false, 4><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
-            else if (vec == 2) k_gauss_axis_ring<KLEN, false, 2><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
-            else k_gauss_axis_ring<KLEN, false, 1><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
+            if (vec == 4) k_gauss_axis_ring<KLEN, false, 4, BD><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
+            else if (vec == 2) k_gauss_axis_ring<KLEN, false, 2, BD><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
+            else k_gauss_axis_ring<KLEN, false, 1, BD><<<grid, 128, 0, st>>>(i_, o_, v, taps, ir, nseg, in_bs, out_bs);
         }
         FDN_LAUNCHED("k_gauss_axis_ring");
     }
     return FDN_OK;
 }
 
-int launch_gauss_axis(const float* in, float* out, const fdn_view& v, const double* k, int klen, int exact,
-                      cudaStream_t st, int batch, int64_t in_bs, int64_t out_bs)
+template <bool BD>
+static int launch_gauss_axis_border(const float* in, float* out, const fdn_view& v, const double* k, int klen,
+                                    int exact, cudaStream_t st, int batch, int64_t in_bs, int64_t out_bs)
 {
-    FDN_CHECK_ARG(klen >= 1 && klen <= FDN_MAX_KLEN && (klen & 1), "kernel length %d unsupported (odd, <= %d)", klen,
-                  FDN_MAX_KLEN);
-    FDN_CHECK_ARG(v.H <= 65535 && v.n_out <= 65535, "view too large for one launch");
     switch (klen) {  // sigma = 0.5, 1, 1.5, 2, 2.5, 3, 4 (radius int(4 sigma + 0.5))
-        case 5: return launch_gauss_axis_ring<5>(in, out, v, k, exact, st, batch, in_bs, out_bs);
-        case 9: return launch_gauss_axis_ring<9>(in, out, v, k, exact, st, batch, in_bs, out_bs);
-        case 13: return launch_gauss_axis_ring<13>(in, out, v, k, exact, st, batch, in_bs, out_bs);
-        case 17: return launch_gauss_axis_ring<17>(in, out, v, k, exact, st, batch, in_bs, out_bs);
-        case 21: return launch_gauss_axis_ring<21>(in, out, v, k, exact, st, batch, in_bs, out_bs);
-        case 25: return launch_gauss_axis_ring<25>(in, out, v, k, exact, st, batch, in_bs, out_bs);
-        case 33: return launch_gauss_axis_ring<33>(in, out, v, k, exact, st, batch, in_bs, out_bs);
+        case 5: return launch_gauss_axis_ring<5, BD>(in, out, v, k, exact, st, batch, in_bs, out_bs);
+        case 9: return launch_gauss_axis_ring<9, BD>(in, out, v, k, exact, st, batch, in_bs, out_bs);
+        case 13: return launch_gauss_axis_ring<13, BD>(in, out, v, k, exact, st, batch, in_bs, out_bs);
+        case 17: return launch_gauss_axis_ring<17, BD>(in, out, v, k, exact, st, batch, in_bs, out_bs);
+        case 21: return launch_gauss_axis_ring<21, BD>(in, out, v, k, exact, st, batch, in_bs, out_bs);
+        case 25: return launch_gauss_axis_ring<25, BD>(in, out, v, k, exact, st, batch, in_bs, out_bs);
+        case 33: return launch_gauss_axis_ring<33, BD>(in, out, v, k, exact, st, batch, in_bs, out_bs);
         default: break;
     }
     Taps64 t64;
@@ -345,11 +359,22 @@ int launch_gauss_axis(const float* in, float* out, const fdn_view& v, const doub
         const int nb = batch - g0 < per_launch ? batch - g0 : per_launch;
         dim3 grid((unsigned)cdiv(v.W, 256), (unsigned)v.H, (unsigned)(nb * v.n_out));
         ProfScope ps(K_GAUSS_AXIS, 8.0 * nb * v.n_out * v.H * v.W, st);
-        if (exact) k_gauss_axis<float, true><<<grid, 256, 0, st>>>(in + g0 * in_bs, out + g0 * out_bs, v, t64, t32, in_bs, out_bs);
-        else k_gauss_axis<float, false><<<grid, 256, 0, st>>>(in + g0 * in_bs, out + g0 * out_bs, v, t64, t32, in_bs, out_bs);
+        if (exact) k_gauss_axis<float, true, BD><<<grid, 256, 0, st>>>(in + g0 * in_bs, out + g0 * out_bs, v, t64, t32, in_bs, out_bs);
+        else k_gauss_axis<float, false, BD><<<grid, 256, 0, st>>>(in + g0 * in_bs, out + g0 * out_bs, v, t64, t32, in_bs, out_bs);
         FDN_LAUNCHED("k_gauss_axis");
     }
     return FDN_OK;
+}
+
+int launch_gauss_axis(const float* in, float* out, const fdn_view& v, const double* k, int klen, int exact,
+                      cudaStream_t st, int batch, int64_t in_bs, int64_t out_bs)
+{
+    FDN_CHECK_ARG(klen >= 1 && klen <= FDN_MAX_KLEN && (klen & 1), "kernel length %d unsupported (odd, <= %d)", klen,
+                  FDN_MAX_KLEN);
+    FDN_CHECK_ARG(v.H <= 65535 && v.n_out <= 65535, "view too large for one launch");
+    if (v.periodic && view_border(v.periodic) != FDN_BORDER_WRAP)
+        return launch_gauss_axis_border<true>(in, out, v, k, klen, exact, st, batch, in_bs, out_bs);
+    return launch_gauss_axis_border<false>(in, out, v, k, klen, exact, st, batch, in_bs, out_bs);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -358,10 +383,12 @@ int launch_gauss_axis(const float* in, float* out, const fdn_view& v, const doub
 // Four consecutive outputs x0 .. x0 + 3 of a row need inputs x0 - R .. x0 + 3 + R: the NV aligned 16-byte groups
 // starting at x0 - PAD (PAD = R rounded up to a multiple of 4), each wrapped periodically as a whole (W % 4 == 0).
 // All NV loads of a thread are independent and issued back to back; the groups a thread shares with its neighbours
-// come from L1.
-template <int KLEN>
+// come from L1. BORDERED (`border`: FDN_BORDER_REFLECT, _MIRROR or _NEAREST): a group lies wholly inside or wholly
+// outside the row (W % 4 == 0); one outside is reversed or repeated by the border, so it maps element by element.
+template <int KLEN, bool BORDERED>
 __global__ void __launch_bounds__(128)
-k_gauss_rows_direct(const float* __restrict__ in, float* __restrict__ out, int W, int64_t rows, TapsW<KLEN> taps)
+k_gauss_rows_direct(const float* __restrict__ in, float* __restrict__ out, int W, int64_t rows, TapsW<KLEN> taps,
+                    int border)
 {
     constexpr int R = KLEN / 2;
     constexpr int PAD = (R + 3) / 4 * 4;
@@ -374,6 +401,11 @@ k_gauss_rows_direct(const float* __restrict__ in, float* __restrict__ out, int W
 #pragma unroll
     for (int g = 0; g < NV; g++) {
         int j = x0 - PAD + 4 * g;
+        if (BORDERED && (unsigned)j >= (unsigned)W) {
+#pragma unroll
+            for (int e = 0; e < 4; e++) win[4 * g + e] = __ldg(src + border_index(j + e, W, border));
+            continue;
+        }
         j %= W;
         if (j < 0) j += W;
         const float4 qv = __ldg(reinterpret_cast<const float4*>(src + j));
@@ -393,10 +425,10 @@ k_gauss_rows_direct(const float* __restrict__ in, float* __restrict__ out, int W
 // Exact mode along rows: a block stages 512 outputs' inputs (+ wrapped halo) of one row in shared memory, every value
 // loaded and range-checked ONCE (the check decides, for the whole block, whether the fast rounding forms are allowed),
 // then each thread computes four consecutive outputs from a float64 register window.
-template <int KLEN>
+template <int KLEN, bool BORDERED>
 __global__ void __launch_bounds__(128)
 k_gauss_rows_tile(const float* __restrict__ in, float* __restrict__ out, int W, int64_t rows, TapsW<KLEN> taps,
-                  int int_rounding)
+                  int int_rounding, int border)
 {
     constexpr int R = KLEN / 2;
     constexpr int PAD = (R + 3) / 4 * 4;
@@ -411,9 +443,15 @@ k_gauss_rows_tile(const float* __restrict__ in, float* __restrict__ out, int W, 
     unsigned bad = int_rounding ? 0u : 1u;
     for (int g = t; g < NG; g += 128) {
         int j = xb - PAD + 4 * g;               // beyond the row's end (last, partial tile): wrapped, harmless
-        j %= W;
-        if (j < 0) j += W;
-        const float4 qv = __ldg(reinterpret_cast<const float4*>(src + j));
+        float4 qv;
+        if (BORDERED && (unsigned)j >= (unsigned)W) {     // (outside the row as a whole group, as in the direct kernel)
+            qv = make_float4(__ldg(src + border_index(j, W, border)), __ldg(src + border_index(j + 1, W, border)),
+                             __ldg(src + border_index(j + 2, W, border)), __ldg(src + border_index(j + 3, W, border)));
+        } else {
+            j %= W;
+            if (j < 0) j += W;
+            qv = __ldg(reinterpret_cast<const float4*>(src + j));
+        }
         bad |= not_benign_f32(qv.x) | not_benign_f32(qv.y) | not_benign_f32(qv.z) | not_benign_f32(qv.w);
         *reinterpret_cast<float4*>(tile + 4 * g) = qv;
     }
@@ -445,9 +483,9 @@ k_gauss_rows_tile(const float* __restrict__ in, float* __restrict__ out, int W, 
         make_float4((float)acc[0], (float)acc[1], (float)acc[2], (float)acc[3]);
 }
 
-template <int KLEN>
+template <int KLEN, bool BD>
 static int launch_gauss_rows_direct(const float* in, float* out, int64_t rows, int W, const double* k, int exact,
-                                    cudaStream_t st)
+                                    int border, cudaStream_t st)
 {
     TapsW<KLEN> taps;
     for (int i = 0; i < KLEN; i++) { taps.k64[i] = k[i]; taps.k32[i] = (float)k[i]; }
@@ -456,29 +494,28 @@ static int launch_gauss_rows_direct(const float* in, float* out, int64_t rows, i
     dim3 grid((unsigned)cdiv(W, 512), (unsigned)ny, (unsigned)cdiv(rows, 65535));
     ProfScope ps(K_GAUSS_ROWS, 8.0 * rows * W, st);
     if (exact) {
-        k_gauss_rows_tile<KLEN><<<grid, 128, 0, st>>>(in, out, W, rows, taps, ir);
+        k_gauss_rows_tile<KLEN, BD><<<grid, 128, 0, st>>>(in, out, W, rows, taps, ir, border);
         FDN_LAUNCHED("k_gauss_rows_tile");
     } else {
-        k_gauss_rows_direct<KLEN><<<grid, 128, 0, st>>>(in, out, W, rows, taps);
+        k_gauss_rows_direct<KLEN, BD><<<grid, 128, 0, st>>>(in, out, W, rows, taps, border);
         FDN_LAUNCHED("k_gauss_rows_direct");
     }
     return FDN_OK;
 }
 
-int launch_gauss_rows(const float* in, float* out, int64_t rows, int W, const double* k, int klen, int exact,
-                      cudaStream_t st)
+template <bool BD>
+static int launch_gauss_rows_border(const float* in, float* out, int64_t rows, int W, const double* k, int klen,
+                                    int exact, int border, cudaStream_t st)
 {
-    FDN_CHECK_ARG(klen >= 1 && klen <= FDN_MAX_KLEN && (klen & 1), "kernel length %d unsupported (odd, <= %d)", klen,
-                  FDN_MAX_KLEN);
     if (W % 4 == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0) {
         switch (klen) {
-            case 5: return launch_gauss_rows_direct<5>(in, out, rows, W, k, exact, st);
-            case 9: return launch_gauss_rows_direct<9>(in, out, rows, W, k, exact, st);
-            case 13: return launch_gauss_rows_direct<13>(in, out, rows, W, k, exact, st);
-            case 17: return launch_gauss_rows_direct<17>(in, out, rows, W, k, exact, st);
-            case 21: return launch_gauss_rows_direct<21>(in, out, rows, W, k, exact, st);
-            case 25: return launch_gauss_rows_direct<25>(in, out, rows, W, k, exact, st);
-            case 33: return launch_gauss_rows_direct<33>(in, out, rows, W, k, exact, st);
+            case 5: return launch_gauss_rows_direct<5, BD>(in, out, rows, W, k, exact, border, st);
+            case 9: return launch_gauss_rows_direct<9, BD>(in, out, rows, W, k, exact, border, st);
+            case 13: return launch_gauss_rows_direct<13, BD>(in, out, rows, W, k, exact, border, st);
+            case 17: return launch_gauss_rows_direct<17, BD>(in, out, rows, W, k, exact, border, st);
+            case 21: return launch_gauss_rows_direct<21, BD>(in, out, rows, W, k, exact, border, st);
+            case 25: return launch_gauss_rows_direct<25, BD>(in, out, rows, W, k, exact, border, st);
+            case 33: return launch_gauss_rows_direct<33, BD>(in, out, rows, W, k, exact, border, st);
             default: break;
         }
     }
@@ -491,11 +528,20 @@ int launch_gauss_rows(const float* in, float* out, int64_t rows, int W, const do
         const int64_t nr = rows - r0 < 65535 ? rows - r0 : 65535;
         dim3 grid((unsigned)cdiv(W, GR_TILE), (unsigned)nr);
         ProfScope ps(K_GAUSS_ROWS, 8.0 * nr * W, st);
-        if (exact) k_gauss_rows<float, true><<<grid, 256, smem, st>>>(in + r0 * W, out + r0 * W, W, t64, t32);
-        else k_gauss_rows<float, false><<<grid, 256, smem, st>>>(in + r0 * W, out + r0 * W, W, t64, t32);
+        if (exact) k_gauss_rows<float, true, BD><<<grid, 256, smem, st>>>(in + r0 * W, out + r0 * W, W, t64, t32, border);
+        else k_gauss_rows<float, false, BD><<<grid, 256, smem, st>>>(in + r0 * W, out + r0 * W, W, t64, t32, border);
         FDN_LAUNCHED("k_gauss_rows");
     }
     return FDN_OK;
+}
+
+int launch_gauss_rows(const float* in, float* out, int64_t rows, int W, const double* k, int klen, int exact,
+                      cudaStream_t st, int border)
+{
+    FDN_CHECK_ARG(klen >= 1 && klen <= FDN_MAX_KLEN && (klen & 1), "kernel length %d unsupported (odd, <= %d)", klen,
+                  FDN_MAX_KLEN);
+    if (border != FDN_BORDER_WRAP) return launch_gauss_rows_border<true>(in, out, rows, W, k, klen, exact, border, st);
+    return launch_gauss_rows_border<false>(in, out, rows, W, k, klen, exact, border, st);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -513,13 +559,17 @@ int launch_gauss_axis_typed(const T* in, T* out, const fdn_view& v, const double
     for (int i = 0; i < klen; i++) { t64.k[i] = k[i]; t32.k[i] = (float)k[i]; }
     dim3 grid((unsigned)cdiv(v.W, 256), (unsigned)v.H, (unsigned)v.n_out);
     ProfScope ps(K_GAUSS_AXIS, 2.0 * sizeof(T) * v.n_out * v.H * v.W, st);
-    k_gauss_axis<T, true><<<grid, 256, 0, st>>>(in, out, v, t64, t32, 0, 0);
+    if (v.periodic && view_border(v.periodic) != FDN_BORDER_WRAP)
+        k_gauss_axis<T, true, true><<<grid, 256, 0, st>>>(in, out, v, t64, t32, 0, 0);
+    else
+        k_gauss_axis<T, true, false><<<grid, 256, 0, st>>>(in, out, v, t64, t32, 0, 0);
     FDN_LAUNCHED("k_gauss_axis");
     return FDN_OK;
 }
 
 template <typename T>
-int launch_gauss_rows_typed(const T* in, T* out, int64_t rows, int W, const double* k, int klen, cudaStream_t st)
+int launch_gauss_rows_typed(const T* in, T* out, int64_t rows, int W, const double* k, int klen, cudaStream_t st,
+                            int border)
 {
     FDN_CHECK_ARG(klen >= 1 && klen <= FDN_MAX_KLEN && (klen & 1), "kernel length %d unsupported (odd, <= %d)", klen,
                   FDN_MAX_KLEN);
@@ -532,7 +582,10 @@ int launch_gauss_rows_typed(const T* in, T* out, int64_t rows, int W, const doub
         const int64_t nr = rows - r0 < 65535 ? rows - r0 : 65535;
         dim3 grid((unsigned)cdiv(W, GR_TILE), (unsigned)nr);
         ProfScope ps(K_GAUSS_ROWS, 2.0 * sizeof(T) * nr * W, st);
-        k_gauss_rows<T, true><<<grid, 256, smem, st>>>(in + r0 * W, out + r0 * W, W, t64, t32);
+        if (border != FDN_BORDER_WRAP)
+            k_gauss_rows<T, true, true><<<grid, 256, smem, st>>>(in + r0 * W, out + r0 * W, W, t64, t32, border);
+        else
+            k_gauss_rows<T, true, false><<<grid, 256, smem, st>>>(in + r0 * W, out + r0 * W, W, t64, t32, border);
         FDN_LAUNCHED("k_gauss_rows");
     }
     return FDN_OK;
@@ -540,7 +593,7 @@ int launch_gauss_rows_typed(const T* in, T* out, int64_t rows, int W, const doub
 
 #define FDN_INST_NOOF(T)                                                                                              \
     template int launch_gauss_axis_typed<T>(const T*, T*, const fdn_view&, const double*, int, cudaStream_t);         \
-    template int launch_gauss_rows_typed<T>(const T*, T*, int64_t, int, const double*, int, cudaStream_t);
+    template int launch_gauss_rows_typed<T>(const T*, T*, int64_t, int, const double*, int, cudaStream_t, int);
 FDN_INST_NOOF(uint8_t)
 FDN_INST_NOOF(int8_t)
 FDN_INST_NOOF(uint16_t)

@@ -80,6 +80,34 @@ def _stream_ptr(torch):
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
+# border along the filtered axis -> FDN_BORDER_* (include/fdn_b200.h); "wrap" is the reference's periodic pass
+BORDERS = {"wrap": _lib.BORDER_WRAP, "reflect": _lib.BORDER_REFLECT, "mirror": _lib.BORDER_MIRROR,
+           "nearest": _lib.BORDER_NEAREST}
+
+
+def border_code(border: str) -> int:
+    """FDN_BORDER_* of a border name (ValueError for any other, "mean" included: it has no device route)."""
+    if border not in BORDERS:
+        raise ValueError(f"border must be one of {', '.join(BORDERS)} (got {border!r})")
+    return BORDERS[border]
+
+
+def border_indices(idx, n: int, border: str) -> np.ndarray:
+    """Slices of an axis of n that the (any integer) indices idx take under `border`: the index maps of
+    include/fdn_b200.h, np.pad's symmetric / reflect / edge modes. "wrap" and "mean" (whose padding is not a slice)
+    wrap periodically."""
+    i = np.asarray(idx, dtype=np.int64)
+    if border == "nearest":
+        return np.clip(i, 0, n - 1)
+    if border in ("reflect", "mirror"):
+        if n == 1:
+            return np.zeros_like(i)
+        p = 2 * n if border == "reflect" else 2 * n - 2
+        j = i % p
+        return np.where(j < n, j, p - 1 - j if border == "reflect" else p - j)
+    return i % n
+
+
 def dtype_code(t) -> int:
     """FDN_DTYPE_* of a tensor's dtype (ValueError for any other dtype)."""
     import torch
@@ -162,11 +190,16 @@ class DeviceEngine:
 
     # ---- one pass over an explicit view ----
     def filter_view(self, d_in, d_out, view: View, kernel, flow: Optional[FlowParams], chunk: Optional[int] = None,
-                    exact: bool = True):
+                    exact: bool = True, border: str = "wrap"):
         """out[s] = sum_i k[i] * warp(in[s+halo+i-r]) for the slices of `view` (see fdn_view). Integer tensors run the
-        typed pass (exact arithmetic only)."""
+        typed pass (exact arithmetic only). A periodic view (periodic != 0) maps its indices with `border` ("wrap":
+        the view's own periodic value); a view with an explicit halo (periodic == 0) ignores it."""
         torch = self.torch
         k, kp = _taps(kernel)
+        code = border_code(border)
+        if view.periodic and code != _lib.BORDER_WRAP:
+            view = View.from_buffer_copy(view)
+            view.periodic = code
         if d_in.dtype != torch.float32:
             return self._filter_view_typed(d_in, d_out, view, k, kp, flow, chunk, exact)
         with torch.cuda.device(self.device):
@@ -279,9 +312,11 @@ class DeviceEngine:
                                                                 int(out_sb), int(n), int(A), int(B), _stream_ptr(torch)))
 
     def filter_along_axis(self, vol, out, axis: int, kernel, flow: Optional[FlowParams], chunk: Optional[int] = None,
-                          exact: bool = True, scratch=None):
-        """One pass of the reference's filter_along_{Z,Y,X} (src/flowdenoising.py:175-283) on the device."""
+                          exact: bool = True, scratch=None, border: str = "wrap"):
+        """One pass of the reference's filter_along_{Z,Y,X} (src/flowdenoising.py:175-283) on the device. `border`: how
+        the axis continues beyond its ends ("wrap", the reference; "reflect", "mirror", "nearest": SciPy's modes)."""
         torch = self.torch
+        code = border_code(border)
         self._check_vol(vol); self._check_vol(out)
         if vol.data_ptr() == out.data_ptr():
             raise ValueError("in-place passes are not supported")
@@ -289,16 +324,20 @@ class DeviceEngine:
             raise ValueError("a pass writes the dtype it reads")
         Z, Y, X = vol.shape
         if axis == 0:
-            v = View(Z, Z, 0, 1, Y, X, Y * X, X, Y * X, X)
+            v = View(Z, Z, 0, code, Y, X, Y * X, X, Y * X, X)
             self.filter_view(vol, out, v, kernel, flow, chunk, exact)
         elif axis == 1:
-            v = View(Y, Y, 0, 1, Z, X, X, Y * X, X, Y * X)
+            v = View(Y, Y, 0, code, Z, X, X, Y * X, X, Y * X)
             self.filter_view(vol, out, v, kernel, flow, chunk, exact)
         elif axis == 2:
             if flow is None:
                 k, kp = _taps(kernel)
                 with torch.cuda.device(self.device):
-                    if vol.dtype == torch.float32:
+                    if code != _lib.BORDER_WRAP:
+                        _lib.check(self.lib.fdn_gauss_rows_border(vol.data_ptr(), out.data_ptr(), dtype_code(vol),
+                                                                  Z * Y, X, kp, k.size, int(bool(exact)), code,
+                                                                  _stream_ptr(torch)))
+                    elif vol.dtype == torch.float32:
                         _lib.check(self.lib.fdn_gauss_rows(vol.data_ptr(), out.data_ptr(), Z * Y, X, kp, k.size,
                                                            int(bool(exact)), _stream_ptr(torch)))
                     else:
@@ -308,42 +347,44 @@ class DeviceEngine:
             # slices vol[:, :, x] are (Z, Y) images with element-strided columns: run on the [Z, X, Y] transpose
             vt = self.transpose_yx(vol, scratch[0] if scratch else None)
             ot = scratch[1] if scratch else torch.empty_like(vt)
-            v = View(X, X, 0, 1, Z, Y, Y, X * Y, Y, X * Y)
+            v = View(X, X, 0, code, Z, Y, Y, X * Y, Y, X * Y)
             self.filter_view(vt, ot, v, kernel, flow, chunk, exact)
             self.transpose_yx(ot.view(Z, X, Y), out)
         else:
             raise ValueError("axis must be 0, 1 or 2")
 
     def filter(self, vol, kernels: Sequence, flow: Optional[FlowParams], chunk: Optional[int] = None,
-               exact: bool = True):
-        """Z, Y, X passes (src/flowdenoising.py:285-290). Returns (zy, zyx): the reference leaves the Z+Y
-        intermediate in `vol` and the final result in `filtered_vol`; `vol` itself is not modified here."""
+               exact: bool = True, border: str = "wrap"):
+        """Z, Y, X passes (src/flowdenoising.py:285-290), each with `border` along its axis. Returns (zy, zyx): the
+        reference leaves the Z+Y intermediate in `vol` and the final result in `filtered_vol`; `vol` itself is not
+        modified here."""
         torch = self.torch
+        code = border_code(border)
         self._check_vol(vol)
         Z, Y, X = vol.shape
         # every volume-sized buffer exists before the first pass sizes its workspace from the free memory
         a = torch.empty_like(vol)
         b = torch.empty_like(vol)
         ot = torch.empty((Z, X, Y), dtype=vol.dtype, device=vol.device) if flow is not None else torch.empty_like(vol)
-        self.filter_along_axis(vol, a, 0, kernels[0], flow, chunk, exact)
-        self.filter_along_axis(a, b, 1, kernels[1], flow, chunk, exact)      # b = ZY
+        self.filter_along_axis(vol, a, 0, kernels[0], flow, chunk, exact, border=border)
+        self.filter_along_axis(a, b, 1, kernels[1], flow, chunk, exact, border=border)      # b = ZY
         if flow is None:
-            self.filter_along_axis(b, ot, 2, kernels[2], flow, chunk, exact)
+            self.filter_along_axis(b, ot, 2, kernels[2], flow, chunk, exact, border=border)
             return b, ot
         # X pass on the [Z, X, Y] transpose: `a` (the Z result) is dead now and holds first the transposed input,
         # then -- once the pass has written `ot` -- the final result
         vt = self.transpose_yx(b, a.view(Z, X, Y))
-        v = View(X, X, 0, 1, Z, Y, Y, X * Y, Y, X * Y)
+        v = View(X, X, 0, code, Z, Y, Y, X * Y, Y, X * Y)
         self.filter_view(vt, ot, v, kernels[2], flow, chunk, exact)
         out = self.transpose_yx(ot, a.view(Z, Y, X))
         return b, out
 
     # ---- a batch of same-shape volumes [B, Z, Y, X] (subtomograms, montage tiles) ----
     @staticmethod
-    def _batch_views(Z: int, Y: int, X: int):
-        """Views of the Z, Y and X pass of one volume; the X pass runs on the [Z, X, Y] transpose."""
-        return (View(Z, Z, 0, 1, Y, X, Y * X, X, Y * X, X), View(Y, Y, 0, 1, Z, X, X, Y * X, X, Y * X),
-                View(X, X, 0, 1, Z, Y, Y, X * Y, Y, X * Y))
+    def _batch_views(Z: int, Y: int, X: int, code: int = _lib.BORDER_WRAP):
+        """Views of the Z, Y and X pass of one volume with border `code`; the X pass runs on the [Z, X, Y] transpose."""
+        return (View(Z, Z, 0, code, Y, X, Y * X, X, Y * X, X), View(Y, Y, 0, code, Z, X, X, Y * X, X, Y * X),
+                View(X, X, 0, code, Z, Y, Y, X * Y, Y, X * Y))
 
     def _pick_batch(self, views, klens, ofp: OfParams, B: int) -> int:
         """Most volumes per device call whose workspace fits the limit (the rule of _pick_chunk: 85 % of free HBM,
@@ -373,12 +414,14 @@ class DeviceEngine:
                 hi = mid - 1
         return lo
 
-    def filter_batch(self, vols, kernels: Sequence, flow: Optional[FlowParams], exact: bool = True):
+    def filter_batch(self, vols, kernels: Sequence, flow: Optional[FlowParams], exact: bool = True,
+                     border: str = "wrap"):
         """DeviceEngine.filter for each volume of a contiguous float32 batch [B, Z, Y, X], many volumes per device
-        call. Returns (zy, zyx) [B, Z, Y, X] with filter's buffer roles; volume g of each equals filter(vols[g]) bit
-        for bit. The batch runs in sub-batches whose workspace fits (sub_batch holds the size last used); a volume
-        too large to go whole through the batched pass runs through filter (chunked)."""
+        call. Returns (zy, zyx) [B, Z, Y, X] with filter's buffer roles; volume g of each equals filter(vols[g],
+        border=border) bit for bit. The batch runs in sub-batches whose workspace fits (sub_batch holds the size last
+        used); a volume too large to go whole through the batched pass runs through filter (chunked)."""
         torch = self.torch
+        code = border_code(border)
         if not (vols.is_cuda and vols.dim() == 4 and vols.is_contiguous() and vols.dtype == torch.float32):
             raise ValueError("expected a contiguous float32 CUDA tensor [B, Z, Y, X]")
         B, Z, Y, X = (int(s) for s in vols.shape)
@@ -389,7 +432,7 @@ class DeviceEngine:
         if flow is None:
             self.sub_batch = B
             out = torch.empty_like(vols)
-            vz = self._batch_views(Z, Y, X)[0]
+            vz = self._batch_views(Z, Y, X, code)[0]
             with torch.cuda.device(self.device):
                 st = _stream_ptr(torch)
                 _lib.check(self.lib.fdn_gauss_axis_batch(vols.data_ptr(), a.data_ptr(), C.byref(vz), B, vs, vs,
@@ -398,21 +441,25 @@ class DeviceEngine:
                 per = max(1, 65535 // Z)
                 for g0 in range(0, B, per):
                     nb = min(per, B - g0)
-                    vy = View(Y, Y, 0, 1, nb * Z, X, X, Y * X, X, Y * X)
+                    vy = View(Y, Y, 0, code, nb * Z, X, X, Y * X, X, Y * X)
                     _lib.check(self.lib.fdn_gauss_axis(a[g0].data_ptr(), zy[g0].data_ptr(), C.byref(vy), ks[1][1],
                                                        ks[1][0].size, int(bool(exact)), st))
                 # and the X pass the rows of B*Z*Y
-                _lib.check(self.lib.fdn_gauss_rows(zy.data_ptr(), out.data_ptr(), B * Z * Y, X, ks[2][1],
-                                                   ks[2][0].size, int(bool(exact)), st))
+                if code == _lib.BORDER_WRAP:
+                    _lib.check(self.lib.fdn_gauss_rows(zy.data_ptr(), out.data_ptr(), B * Z * Y, X, ks[2][1],
+                                                       ks[2][0].size, int(bool(exact)), st))
+                else:
+                    _lib.check(self.lib.fdn_gauss_rows_border(zy.data_ptr(), out.data_ptr(), _lib.DTYPE_F32, B * Z * Y,
+                                                              X, ks[2][1], ks[2][0].size, int(bool(exact)), code, st))
             return zy, out
-        views = self._batch_views(Z, Y, X)
+        views = self._batch_views(Z, Y, X, code)
         ofp = flow.c_struct()
         with torch.cuda.device(self.device):
             sb = self._pick_batch(views, [k.size for k, _ in ks], ofp, B)
             self.sub_batch = sb
             if sb == 0:     # one volume does not fit whole: the chunked single-volume path
                 for g in range(B):
-                    z1, o1 = self.filter(vols[g], kernels, flow, exact=exact)
+                    z1, o1 = self.filter(vols[g], kernels, flow, exact=exact, border=border)
                     zy[g].copy_(z1)
                     a[g].copy_(o1)
                     del z1, o1

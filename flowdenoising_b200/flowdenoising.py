@@ -453,7 +453,9 @@ class GaussianDenoising():
         self._flow_params = None  # no OF
         self.exact = True         # no-OF arithmetic: bit-exact NumPy emulation (False: float32 FMA)
         # beyond the reference's surface (set after construction; the CLI maps --border / --gpus / --slab_slices):
-        self.border = "wrap"      # "mean": the sequential variant's padding (src/flowdenoising_sequential.py:88-89)
+        # "wrap": the reference's periodic axis; "reflect", "mirror", "nearest": SciPy's modes, in core or streamed;
+        # "mean": the sequential variant's padding (src/flowdenoising_sequential.py:88-89), streamed, float32 only
+        self.border = "wrap"
         self.devices = None       # CUDA devices to spread slabs over (None: the current one)
         self.slab_slices = None   # output slices per streamed slab (None: sized from the free device memory)
         self.streaming = None     # None: stream slab by slab only when needed (memory map, > device memory, ...)
@@ -496,7 +498,7 @@ class GaussianDenoising():
         if dt == np.int8 and self._flow() is not None:
             raise ValueError("keep_dtype: int8 volumes are supported without optical flow only (cv2.remap, which the "
                              "reference calls, rejects int8 images)")
-        if self.border != "wrap":
+        if self.border == "mean":
             raise ValueError("keep_dtype: streaming with --border mean is not supported for integer volumes (the "
                              "reference defines no integer mean padding)")
         return True
@@ -504,7 +506,7 @@ class GaussianDenoising():
     def _streaming_needed(self):
         if self.streaming is not None:
             return bool(self.streaming)
-        if isinstance(self.vol, np.memmap) or self.border != "wrap" or (self.devices and len(self.devices) > 1):
+        if isinstance(self.vol, np.memmap) or self.border == "mean" or (self.devices and len(self.devices) > 1):
             return True
         eng = _get_engine()
         free, _total = eng.torch.cuda.mem_get_info(eng.device)
@@ -533,7 +535,7 @@ class GaussianDenoising():
             d_in = torch.from_numpy(np.ascontiguousarray(self.vol)).to(eng.device)
             d_out = torch.empty_like(d_in)
             self._begin_device_call()
-            eng.filter_along_axis(d_in, d_out, axis, kernel, self._flow(), exact=self.exact)
+            eng.filter_along_axis(d_in, d_out, axis, kernel, self._flow(), exact=self.exact, border=self.border)
             self.filtered_vol[...] = d_out.cpu().numpy()
             self._end_device_call(self.vol.shape[axis])
             return
@@ -552,7 +554,7 @@ class GaussianDenoising():
         d_in = _upload_volume(self.vol, torch, eng.device)
         d_out = torch.empty_like(d_in)
         self._begin_device_call()
-        eng.filter_along_axis(d_in, d_out, axis, kernel, self._flow(), exact=self.exact)
+        eng.filter_along_axis(d_in, d_out, axis, kernel, self._flow(), exact=self.exact, border=self.border)
         dl = _Download(d_out, self.filtered_vol, torch)
         dl.wait()
         self._end_device_call(self.vol.shape[axis])
@@ -570,7 +572,8 @@ class GaussianDenoising():
         self._pass(2, kernel)
 
     # The reference's per-slice / per-chunk entry points (:133-173). A slice is not a useful unit of GPU work,
-    # but they are kept so that code driving the reference slice by slice still runs.
+    # but they are kept so that code driving the reference slice by slice still runs. The neighbours of a slice are
+    # the slices the border maps to (the reference's `% n` for wrap and, as before, for mean).
     def _slice(self, axis, idx, kernel):
         eng = _get_engine()
         torch = eng.torch
@@ -578,7 +581,7 @@ class GaussianDenoising():
         assert kernel.size % 2 != 0
         r = kernel.size // 2
         n = self.vol.shape[axis]
-        idxs = [(idx + d) % n for d in range(-r, r + 1)]
+        idxs = _engine.border_indices(np.arange(idx - r, idx + r + 1), n, self.border)
         typed = self._typed()
         slab = np.ascontiguousarray(np.moveaxis(np.take(self.vol, idxs, axis=axis), axis, 0),
                                     dtype=self.vol.dtype if typed else np.float32)
@@ -602,7 +605,7 @@ class GaussianDenoising():
 
     def _chunk(self, axis, start, count, kernel):
         '''The reference's unit of parallel work (:160-173) as ONE device call: the chunk's slices plus an r-slice
-        periodic halo go up as a slab, one non-periodic view filters them, the result comes back. Same bits as
+        halo (the slices the border maps to) go up as a slab, one non-periodic view filters them, the result comes back. Same bits as
         slice-by-slice calls (every output slice sees the same inputs).'''
         if count <= 0:
             return
@@ -612,7 +615,7 @@ class GaussianDenoising():
         assert kernel.size % 2 != 0
         r = kernel.size // 2
         n = self.vol.shape[axis]
-        idxs = [(start + d) % n for d in range(-r, count + r)]
+        idxs = _engine.border_indices(np.arange(start - r, start + count + r), n, self.border)
         typed = self._typed()
         slab = np.ascontiguousarray(np.moveaxis(np.take(self.vol, idxs, axis=axis), axis, 0),
                                     dtype=self.vol.dtype if typed else np.float32)
@@ -659,7 +662,7 @@ class GaussianDenoising():
             # the plain sequence: upload in the dtype, three typed passes, the ZY intermediate and the result home
             d_in = torch.from_numpy(np.ascontiguousarray(self.vol)).to(eng.device)
             self._begin_device_call()
-            zy, zyx = eng.filter(d_in, ks, self._flow(), exact=self.exact)
+            zy, zyx = eng.filter(d_in, ks, self._flow(), exact=self.exact, border=self.border)
             self.vol[...] = zy.cpu().numpy()
             self.filtered_vol[...] = zyx.cpu().numpy()
             self._end_device_call(Z + Y + X)
@@ -703,15 +706,16 @@ class GaussianDenoising():
         b = torch.empty_like(d_in)
         ot = torch.empty((Z, X, Y), dtype=torch.float32, device=d_in.device) if flow is not None else torch.empty_like(d_in)
         self._begin_device_call()
-        eng.filter_along_axis(d_in, a, 0, ks[0], flow, exact=self.exact)
-        eng.filter_along_axis(a, b, 1, ks[1], flow, exact=self.exact)          # b = Z+Y
+        bd = self.border
+        eng.filter_along_axis(d_in, a, 0, ks[0], flow, exact=self.exact, border=bd)
+        eng.filter_along_axis(a, b, 1, ks[1], flow, exact=self.exact, border=bd)          # b = Z+Y
         dl_zy = _Download(b, self.vol, torch)                                   # ... goes home while X runs
         if flow is None:
-            eng.filter_along_axis(b, ot, 2, ks[2], None, exact=self.exact)
+            eng.filter_along_axis(b, ot, 2, ks[2], None, exact=self.exact, border=bd)
             out = ot
         else:
             vt = eng.transpose_yx(b, a.view(Z, X, Y))
-            v = _engine.View(X, X, 0, 1, Z, Y, Y, X * Y, Y, X * Y)
+            v = _engine.View(X, X, 0, _engine.border_code(bd), Z, Y, Y, X * Y, Y, X * Y)
             eng.filter_view(vt, ot, v, ks[2], flow, exact=self.exact)
             out = eng.transpose_yx(ot, a.view(Z, Y, X))
         dl = _Download(out, self.filtered_vol, torch)
@@ -744,9 +748,11 @@ class GaussianDenoising():
         View = _engine.View
         Z, Y, X = (int(v) for v in self.vol.shape)
         rz = ks[0].size // 2
+        pc = _engine.border_code(self.border)    # fdn_view.periodic of every whole-axis view and window below
         if head <= 0 or head + 2 * rz >= Z:      # (head 0: tools/overlap_lab3.py measures the download split alone)
             ranges, head_key, head = [(0, Z)], 0, 0
-        else:   # what the head needs first: its periodic neighbours at the far end, then slices 0 .. head + r
+        else:   # what the head needs first: its periodic neighbours at the far end (the other borders map the head's
+            # neighbours below 0 into slices 0 .. r), then slices 0 .. head + r
             ranges, head_key = [(Z - rz, Z), (0, head + rz), (head + rz, Z - rz)], 1
         up = _Upload(self.vol, torch, eng.device, ranges)
         d_in = up.d
@@ -754,9 +760,9 @@ class GaussianDenoising():
         b = torch.empty_like(d_in)
         ot = torch.empty((Z, X, Y), dtype=torch.float32, device=d_in.device)
         # one workspace for all three passes, sized after every volume-sized buffer exists
-        for v, k in ((View(Z, Z, 0, 1, Y, X, Y * X, X, Y * X, X), ks[0]),
-                     (View(Y, Y, 0, 1, Z, X, X, Y * X, X, Y * X), ks[1]),
-                     (View(X, X, 0, 1, Z, Y, Y, X * Y, Y, X * Y), ks[2])):
+        for v, k in ((View(Z, Z, 0, pc, Y, X, Y * X, X, Y * X, X), ks[0]),
+                     (View(Y, Y, 0, pc, Z, X, X, Y * X, X, Y * X), ks[1]),
+                     (View(X, X, 0, pc, Z, Y, Y, X * Y, Y, X * Y), ks[2])):
             eng.reserve_workspace(v, k.size, flow)
         # a pageable result array is usually untouched memory: map its pages while the passes run
         pre = None if _is_pinned_f32(self.filtered_vol, torch) else _prefault(self.filtered_vol)
@@ -767,28 +773,28 @@ class GaussianDenoising():
             up.ready(head_key)
             _mark(torch, "head uploaded")
             if head > 0:
-                eng.filter_view(d_in, a, View(Z, head, 0, 1, Y, X, Y * X, X, Y * X, X), ks[0], flow, exact=self.exact)
+                eng.filter_view(d_in, a, View(Z, head, 0, pc, Y, X, Y * X, X, Y * X, X), ks[0], flow, exact=self.exact)
             _mark(torch, "Z head")
             up.ready(len(ranges) - 1)
             _mark(torch, "all uploaded")
-            eng.filter_view(d_in, a[head:], View(Z, Z - head, head, 1, Y, X, Y * X, X, Y * X, X), ks[0], flow,
+            eng.filter_view(d_in, a[head:], View(Z, Z - head, head, pc, Y, X, Y * X, X, Y * X, X), ks[0], flow,
                             exact=self.exact)
         finally:
             up.close()
         _mark(torch, "Z tail")
-        eng.filter_along_axis(a, b, 1, ks[1], flow, exact=self.exact)          # b = Z+Y
+        eng.filter_view(a, b, View(Y, Y, 0, pc, Z, X, X, Y * X, X, Y * X), ks[1], flow, exact=self.exact)   # b = Z+Y
         _mark(torch, "Y")
         dl_zy = _Download(b, self.vol, torch)                                   # ... goes home while X runs
         vt = eng.transpose_yx(b, a.view(Z, X, Y))
         out = d_in                                                              # dead since the Z pass
         Xb = X - tail
-        eng.filter_view(vt, ot, View(X, Xb, 0, 1, Z, Y, Y, X * Y, Y, X * Y), ks[2], flow, exact=self.exact)
+        eng.filter_view(vt, ot, View(X, Xb, 0, pc, Z, Y, Y, X * Y, Y, X * Y), ks[2], flow, exact=self.exact)
         eng.transpose_strided(ot, 0, X * Y, Y, out, 0, Y * X, X, Z, Xb, Y)
         _mark(torch, "X body")
         if pre is not None:
             pre.join()
         dl_body = _DownloadCols(out, self.filtered_vol, 0, Xb, torch)
-        eng.filter_view(vt, ot.view(-1)[Xb * Y:], View(X, tail, Xb, 1, Z, Y, Y, X * Y, Y, X * Y), ks[2], flow,
+        eng.filter_view(vt, ot.view(-1)[Xb * Y:], View(X, tail, Xb, pc, Z, Y, Y, X * Y, Y, X * Y), ks[2], flow,
                         exact=self.exact)
         eng.transpose_strided(ot, Xb * Y, X * Y, Y, out, Xb, Y * X, X, Z, tail, Y)
         _mark(torch, "X tail")
@@ -841,12 +847,18 @@ class _Stack:
 
 
 def filter_volumes(vols, kernels, l=OF_LEVELS, w=OF_WINDOW_SIZE, get_flow=get_flow_with_prev_flow, no_OF=False,
-                   iterations=OF_ITERS, poly_n=OF_POLY_N, poly_sigma=OF_POLY_SIGMA, gaussian_window=False, exact=True):
+                   iterations=OF_ITERS, poly_n=OF_POLY_N, poly_sigma=OF_POLY_SIGMA, gaussian_window=False, exact=True,
+                   border="wrap"):
     '''Z+Y+X results of many volumes (subtomograms, montage tiles): a 4-D host array [n, Z, Y, X] or a sequence of 3-D
     host arrays, any dtype NumPy casts (filtered as float32, like FlowDenoising(...).filter). Volumes of one shape are
     filtered together, many per device call (DeviceEngine.filter_batch); each result equals
-    FlowDenoising(1, vol, ...).filter(kernels) (GaussianDenoising with no_OF) on that volume alone, bit for bit.
+    FlowDenoising(1, vol, ...).filter(kernels) (GaussianDenoising with no_OF) on that volume alone, bit for bit, with
+    the same `border` ("wrap", "reflect", "mirror" or "nearest"; "mean" raises ValueError).
     Returns a list of float32 arrays in input order. Not part of the reference's surface.'''
+    if border == "mean":
+        raise ValueError("filter_volumes: border 'mean' is not supported (it streams volume by volume; use "
+                         "wrap, reflect, mirror or nearest)")
+    _engine.border_code(border)
     items = list(vols)
     for v in items:
         if np.ndim(v) != 3:
@@ -873,7 +885,9 @@ def filter_volumes(vols, kernels, l=OF_LEVELS, w=OF_WINDOW_SIZE, get_flow=get_fl
         for j0 in range(0, len(idx), n):
             part = idx[j0:j0 + n]
             d = _upload_volume(_Stack([items[i] for i in part]), torch, eng.device)
-            _zy, zyx = eng.filter_batch(d, ks, flow, exact=exact)
+            # (wrap goes without the keyword: an engine that predates the borders still serves it)
+            bkw = {} if border == "wrap" else {"border": border}
+            _zy, zyx = eng.filter_batch(d, ks, flow, exact=exact, **bkw)
             res = np.empty((len(part),) + shape, np.float32)
             dl = _Download(zyx, res, torch)
             dl.wait()
@@ -920,9 +934,13 @@ def build_parser():
                         default=number_of_PUs)
     parser.add_argument("--gpus", type=int, default=1,
                         help="Number of GPUs of this node to spread each pass over (slabs of slices with an r-slice halo)")
-    parser.add_argument("--border", choices=["wrap", "mean"], default="wrap",
-                        help="Border along the filtered axis: periodic like flowdenoising.py, or padded with the "
-                             "volume's mean like flowdenoising_sequential.py")
+    parser.add_argument("--border", choices=["wrap", "reflect", "mirror", "nearest", "mean"], default="wrap",
+                        help="Border along the filtered axis. wrap: periodic, the far end of the volume continues it, "
+                             "like flowdenoising.py (the reference); reflect: the volume mirrored about its end face, "
+                             "edge slice repeated (d c b a | a b c d, SciPy's reflect); mirror: mirrored about the edge "
+                             "slice (d c b | a b c d, SciPy's mirror, OpenCV's BORDER_REFLECT_101); nearest: the edge "
+                             "slice repeated (a a a | a b c d); mean: padded with the volume's mean like "
+                             "flowdenoising_sequential.py (float32, always streamed slab by slab)")
     parser.add_argument("--slab_slices", type=int, default=None,
                         help="Output slices per streamed slab when the volume does not stay on the device "
                              "(default: sized from the free device memory)")
@@ -1077,7 +1095,7 @@ def _main_batch(args, argv, sigma, get_flow):
     explicit = probe.parse_args(argv)
     if explicit.input != argparse.SUPPRESS or explicit.output != argparse.SUPPRESS:
         parser.error("--inputs replaces -i / -o (results go to --output_dir)")
-    for flag, bad in (("-m", args.memory_map), ("--gpus > 1", args.gpus > 1), ("--border mean", args.border != "wrap"),
+    for flag, bad in (("-m", args.memory_map), ("--gpus > 1", args.gpus > 1), ("--border mean", args.border == "mean"),
                       ("--slab_slices", args.slab_slices is not None), ("--keep_dtype", args.keep_dtype),
                       ("--compat_zy_output", args.compat_zy_output)):
         if bad:
@@ -1095,7 +1113,7 @@ def _main_batch(args, argv, sigma, get_flow):
     time_0 = time.perf_counter()
     results = filter_volumes(vols, kernels, args.levels, args.winsize, get_flow, no_OF=args.no_OF,
                              iterations=args.iterations, poly_n=args.poly_n, poly_sigma=args.poly_sigma,
-                             gaussian_window=args.gaussian_window)
+                             gaussian_window=args.gaussian_window, border=args.border)
     logging.info(f"{len(vols)} volumes filtered in {time.perf_counter() - time_0} seconds")
     os.makedirs(args.output_dir, exist_ok=True)
     for name, res in zip(names, results):

@@ -2,12 +2,13 @@
 one or several GPUs slab by slab.
 
 Covers what the reference offers for volumes that do not fit the device: `-m/--memory_map`
-(/root/reference/src/flowdenoising.py:407-409, live in src/flowdenoising_sequential.py:510-512) and, as an option, the
-sequential variant's mean-padding border (src/flowdenoising_sequential.py:88-89) instead of the periodic one
-(src/flowdenoising.py:312).
+(/root/reference/src/flowdenoising.py:407-409, live in src/flowdenoising_sequential.py:510-512) and, as options, the
+sequential variant's mean-padding border (src/flowdenoising_sequential.py:88-89) and SciPy's reflect, mirror and
+nearest borders instead of the periodic one (src/flowdenoising.py:312).
 
 Within a pass every output slice depends only on its 2r neighbour slices, so a pass is cut into slabs along the
-FILTERED axis, each uploaded with an r-slice halo (periodic wrap or the volume's mean), filtered on a non-periodic
+FILTERED axis, each uploaded with an r-slice halo (the slices the border maps to -- periodic wrap, reversed runs for
+reflect and mirror, the edge slice repeated for nearest -- or the volume's mean), filtered on a non-periodic
 view (the same `fdn_view` the multi-GPU path uses) and downloaded:
 
     Z pass   slab = vol[z0-r : z1+r]            device [zl+2r][Y][X]            slices = planes
@@ -36,7 +37,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import View
-from .engine import DeviceEngine, FlowParams
+from .engine import BORDERS, DeviceEngine, FlowParams, border_indices
 
 
 _TYPED = tuple(np.dtype(t) for t in (np.uint8, np.int8, np.uint16, np.int16))
@@ -52,15 +53,28 @@ def _lib_dtype(dt):
             np.dtype(np.int16): _lib.DTYPE_I16}[np.dtype(dt)]
 
 
-def _runs(lo: int, hi: int, n: int):
-    """[lo, hi) as (dst offset, src start, length, inside) runs: indices outside [0, n) wrap periodically."""
+def _runs(lo: int, hi: int, n: int, border: str = "wrap"):
+    """[lo, hi) as (dst offset, src start, length, step, inside) runs: dst[offset + t] = src[start + t * step] for
+    t < length, step 1, -1 (reflect, mirror) or 0 (nearest: the edge slice repeated). Indices outside [0, n) take the
+    border's slice (border_indices; "wrap" and "mean" wrap periodically, "mean" then fills the runs not inside)."""
     out = []
-    i = lo
-    while i < hi:
-        j = i % n
-        length = min(hi - i, n - j)
-        out.append((i - lo, j, length, 0 <= i < n))
-        i += length
+    if border not in ("reflect", "mirror", "nearest"):
+        i = lo
+        while i < hi:
+            j = i % n
+            length = min(hi - i, n - j)
+            out.append((i - lo, j, length, 1, 0 <= i < n))
+            i += length
+        return out
+    idx = border_indices(np.arange(lo, hi), n, border)
+    t = 0
+    while t < hi - lo:
+        step = int(idx[t + 1] - idx[t]) if t + 1 < hi - lo else 1
+        length = 1
+        while t + length < hi - lo and idx[t + length] - idx[t + length - 1] == step:
+            length += 1
+        out.append((t, int(idx[t]), length, step, 0 <= lo + t and lo + t + length <= n))
+        t += length
     return out
 
 
@@ -110,7 +124,8 @@ class _DeviceLane:
 class StreamingDenoiser:
     """Three-pass filter of a host-resident volume (see the module docstring).
 
-    border: "wrap" (the reference, src/flowdenoising.py:312) or "mean" (the sequential variant's padding).
+    border: "wrap" (the reference, src/flowdenoising.py:312), "reflect", "mirror", "nearest" (SciPy's modes, the device
+    passes' FDN_BORDER_*) or "mean" (the sequential variant's padding).
     slab_slices: output slices per slab (None: sized from `device_budget_bytes` / the free device memory).
     devices: CUDA device indices to spread the slabs over (default: the current device).
     keep_dtype: an integer volume runs the typed passes in its own dtype (see the module docstring); otherwise every
@@ -120,8 +135,8 @@ class StreamingDenoiser:
                  slab_slices: Optional[int] = None, devices: Optional[Sequence[int]] = None,
                  device_budget_bytes: Optional[int] = None, progress: Optional[Callable[[float], None]] = None,
                  keep_dtype: bool = False):
-        if border not in ("wrap", "mean"):
-            raise ValueError("border must be 'wrap' or 'mean'")
+        if border not in BORDERS and border != "mean":
+            raise ValueError(f"border must be one of {', '.join(BORDERS)} or 'mean'")
         self.keep_dtype = bool(keep_dtype)
         torch = _lib.require_cuda()
         self.torch = torch
@@ -139,7 +154,7 @@ class StreamingDenoiser:
         dt = np.dtype(src.dtype)
         if not self.keep_dtype or dt not in _TYPED:
             return np.dtype(np.float32)
-        if self.border != "wrap":
+        if self.border == "mean":
             raise ValueError("keep_dtype: streaming with --border mean is not supported for integer volumes (the "
                              "reference defines no integer mean padding)")
         return dt
@@ -197,14 +212,19 @@ class StreamingDenoiser:
 
     # ---------------------------------------------------------------------------------------------- host <-> staging
     def _gather(self, src, axis, lo, hi, dst, mean):
-        """dst[...] = src[lo:hi along axis] with indices outside [0, n) wrapped or replaced by the mean."""
+        """dst[...] = src[lo:hi along axis] with indices outside [0, n) mapped by the border or replaced by the mean."""
         n = src.shape[axis]
-        for off, start, length, inside in _runs(lo, hi, n):
+        for off, start, length, step, inside in _runs(lo, hi, n, self.border):
             sl_d = [slice(None)] * 3
             sl_s = [slice(None)] * 3
             sl_d[axis] = slice(off, off + length)
-            sl_s[axis] = slice(start, start + length)
-            if inside or self.border == "wrap":
+            if step == 1:
+                sl_s[axis] = slice(start, start + length)
+            elif step == -1:
+                sl_s[axis] = slice(start, start - length if start >= length else None, -1)
+            else:
+                sl_s[axis] = slice(start, start + 1)        # broadcast over the run
+            if inside or self.border != "mean":
                 np.copyto(dst[tuple(sl_d)], src[tuple(sl_s)], casting="unsafe")
             else:
                 dst[tuple(sl_d)] = mean

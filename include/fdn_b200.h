@@ -66,13 +66,29 @@ typedef struct fdn_of_params {
     int flags;           /* 0 (box window) or FDN_OF_FARNEBACK_GAUSSIAN; any other bit is rejected */
 } fdn_of_params;
 
+/* Border of a pass along its axis (fdn_view.periodic, fdn_gauss_rows_border): how an input index i outside [0, n)
+ * of an axis of n slices maps to a slice. Each equals the periodic pass on the axis padded by r slices with NumPy's
+ * np.pad mode in brackets, cropped back to n (SciPy's ndimage name first):
+ *   FDN_BORDER_WRAP     i mod n, the reference (`% self.vol.shape[0]`, src/flowdenoising.py:312)      [wrap]
+ *   FDN_BORDER_REFLECT  d c b a | a b c d: p = 2n, j = i mod p, j < n ? j : p - 1 - j                 [symmetric]
+ *   FDN_BORDER_MIRROR   d c b | a b c d: n = 1 -> 0, else p = 2n - 2, j = i mod p, j < n ? j : p - j  [reflect]
+ *   FDN_BORDER_NEAREST  a a a | a b c d: clamp(i, 0, n - 1)                                            [edge]
+ * The mapped neighbours are slices of the volume, so the modes need no padded copy and run the same launches as the
+ * wrap. Views of more than 2^30 slices (rows of more than 2^30 elements) take the wrap only. */
+#define FDN_BORDER_WRAP 1
+#define FDN_BORDER_REFLECT 2
+#define FDN_BORDER_MIRROR 3
+#define FDN_BORDER_NEAREST 4
+
 /* Geometry of one volume view of a pass. The view holds n_in slices of (H, W). Output slice s (0..n_out-1)
  * is centred on input slice s+halo; its neighbours are input slices s+halo+d, d in [-r, r]. If periodic != 0
- * every input index wraps modulo n_in exactly like `% self.vol.shape[0]` in src/flowdenoising.py:312 (whole axis
- * resident: halo = 0, n_out = n_in; a WINDOW of the axis: halo = first output slice, n_out <= n_in, d_out pointing at
- * that slice -- the plugin runs the first / last slices of a pass as their own call so that the upload / download
- * of the rest overlaps them); otherwise the caller guarantees halo >= r slices on both sides (multi-GPU slabs carry
- * the periodic halo explicitly). */
+ * every input index is mapped to [0, n_in) by the border periodic names: FDN_BORDER_REFLECT, _MIRROR or _NEAREST, and
+ * any other nonzero value (FDN_BORDER_WRAP = 1 among them) wraps modulo n_in exactly like `% self.vol.shape[0]` in
+ * src/flowdenoising.py:312 (whole axis resident: halo = 0, n_out = n_in; a WINDOW of the axis: halo = first output
+ * slice, n_out <= n_in, d_out pointing at that slice, indices mapped as absolute indices of the axis -- the plugin runs
+ * the first / last slices of a pass as their own call so that the upload / download of the rest overlaps them);
+ * periodic == 0: the caller guarantees halo >= r slices on both sides (multi-GPU slabs carry the periodic halo
+ * explicitly, streamed slabs the halo of their border). */
 typedef struct fdn_view {
     int n_in, n_out, halo, periodic;
     int H, W;
@@ -81,8 +97,9 @@ typedef struct fdn_view {
 } fdn_view;
 
 /* ---- library / error handling ---- */
-/* 101. The batch entry points (fdn_workspace_bytes_batch, fdn_filter_axis_batch, fdn_gauss_axis_batch) were added
- * without a version change: a caller that needs them looks them up with dlsym. */
+/* 101. The batch entry points (fdn_workspace_bytes_batch, fdn_filter_axis_batch, fdn_gauss_axis_batch), the borders
+ * FDN_BORDER_REFLECT / _MIRROR / _NEAREST and fdn_gauss_rows_border were added without a version change: a caller
+ * that needs them looks them up with dlsym. */
 int fdn_version(void);
 const char* fdn_last_error(void);
 /* Number of this library's kernel launches since the last reset (bench.py "gpu_launches"). */
@@ -145,12 +162,17 @@ int fdn_gauss_axis(const float* d_in, float* d_out, const fdn_view* view, const 
  * periodic wrap. */
 int fdn_gauss_rows(const float* d_in, float* d_out, int64_t n_rows, int W, const double* kernel, int klen,
                    int exact, void* stream);
+/* fdn_gauss_rows / fdn_gauss_rows_typed (dtype: FDN_DTYPE_*) with the border `border` (FDN_BORDER_WRAP ..
+ * FDN_BORDER_NEAREST) at both ends of every row. FDN_BORDER_WRAP runs exactly fdn_gauss_rows(_typed). Any other
+ * border value is rejected with FDN_ERR_INVALID before anything is launched. */
+int fdn_gauss_rows_border(const void* d_in, void* d_out, int dtype, int64_t n_rows, int W, const double* kernel,
+                          int klen, int exact, int border, void* stream);
 /* Batched 2-D transpose of the last two axes: in [n][A][B] -> out [n][B][A]. */
 int fdn_transpose_yx(const float* d_in, float* d_out, int n, int A, int B, void* stream);
 
 /* ---- batches of same-shape volumes (subtomograms, montage tiles): the loop of the reference's
  * GaussianDenoising.filter_along_{Z,Y,X} (src/flowdenoising.py:175-283) run for many volumes in one device pass ----
- * A batch of `batch` volumes of one shape. Volume g's view (whole periodic axis: periodic = 1, halo = 0,
+ * A batch of `batch` volumes of one shape. Volume g's view (whole axis with a border: periodic != 0, halo = 0,
  * n_out = n_in) starts at d_in + g*in_batch_stride and d_out + g*out_batch_stride (elements). Volume g's result
  * equals fdn_filter_axis / fdn_gauss_axis on that volume alone, bit for bit. Every launch carries the image pairs of
  * all volumes, so the launch count of a pass does not grow with the batch. Rejected with FDN_ERR_INVALID before
